@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU algorithm (numpy oracle port)
+    python bench.py ... --dump-outputs DIR                   # also save what the last timed step computed, as .npy
 
 A "step" is ONE CAVI iteration (reference `_update_CAVI`, model.py:623-660) over the whole synthetic network, with the
 ELBO evaluated on the reference's cadence (iteration 1, every 10th, the last; model.py:1036) inside the timed region.
@@ -56,7 +57,7 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--no-c5", action="store_true", help="skip the config-5 workload (configs.c5)")
-    ap.add_argument("--c5-steps", type=int, default=20)
+    ap.add_argument("--c5-steps", type=int, default=None, help="timed steps of the config-5 workload (default: --steps)")
     ap.add_argument("--c5-nodes", type=int, default=0)
     ap.add_argument("--tile-h", type=int, default=128)
     ap.add_argument("--trace", action="store_true", help="print per-batch device times (rank 0, stderr)")
@@ -66,6 +67,10 @@ def parse():
     ap.add_argument("--config", default="c3", choices=["c3", "c4", "c5", "c5s"],
                     help="headline workload: c3 (default, BASELINE's metric); builder runs: c4 = dense reporting N=8k "
                          "M=64 L=2 K=2, c5 = config 5 weak-scaled, c5s = config 5 at N=16k")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy: posterior "
+                         "parameters, ELBO and a fixed sample of the rho slab (rank 0's rows); the config-5 "
+                         "workload's as DIR/c5_<name>.npy")
     return ap.parse_args()
 
 
@@ -470,7 +475,28 @@ def hbm_peak():
         return 6650.0, "fallback of B200_PROFILING.md (of fallback)"
 
 
-def run_workload(args, config, N, L, K, steps, warmup, dist, world, rank, dev, do_e2e, clock_index):
+def dump_outputs(eng, row0, out_dir, prefix, n_sample=1 << 18):
+    """What the timed iterations hand their caller: posterior parameters and ELBO (float64) and the dense rho slab
+    (float32), the slab as a fixed sample of at most `n_sample` ties with their global flat ids (l*N + i)*N + j."""
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    p = eng.params()
+    rho = eng.rho_slab()
+    L, nloc, N, K = rho.shape
+    total = L * nloc * N
+    idx = np.unique(np.random.RandomState(0).randint(0, total, size=min(n_sample, total), dtype=np.int64))
+    sample = rho.view(-1, K)[torch.from_numpy(idx).to(rho.device)].cpu().numpy()
+    l, rest = np.divmod(idx, nloc * N)
+    i, j = np.divmod(rest, N)
+    out = {k: p[k] for k in ("gamma_shp", "gamma_rte", "phi_shp", "phi_rte", "nu_shp", "nu_rte")}
+    out.update(elbo=np.float64(eng.elbo()), rho_sample=sample,
+               rho_sample_tie=((l * N + row0 + i) * N + j).astype(np.float64))
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, prefix + name + ".npy"), np.asarray(a))
+
+
+def run_workload(args, config, N, L, K, steps, warmup, dist, world, rank, dev, do_e2e, clock_index, dump_prefix=""):
     """Generate this rank's shard, pack it, run warm-up + `steps` timed iterations, the dense kernel in isolation, and
     (optionally) the end-to-end fit from pinned host buffers.  Returns the result dict (rank 0 uses it)."""
     import torch
@@ -566,6 +592,8 @@ def run_workload(args, config, N, L, K, steps, warmup, dist, world, rank, dev, d
     launches = eng.n_launch - n0
     value = steps * T / (ms * 1e-3)
     elbo_final = eng.elbo()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(eng, sh.row0, args.dump_outputs, dump_prefix)
 
     # ---- dominant kernel in isolation: the per-tie dense kernel (writes 4*K bytes per owned tie)
     reps = 20
@@ -707,9 +735,10 @@ def run_ours(args):
     c5 = None
     if not args.no_c5 and args.config == "c3":
         _, L5, K5, N5 = config_dims("c5", world, args.c5_nodes)
-        r5 = run_workload(args, "c5", N5, L5, K5, args.c5_steps, min(args.warmup, 5), dist, world, rank, dev,
-                          do_e2e=False, clock_index=None)
-        c5 = {"workload": workload_name("c5", N5, L5, K5, world), "n_gpus": world, "steps": args.c5_steps,
+        c5_steps = args.steps if args.c5_steps is None else args.c5_steps
+        r5 = run_workload(args, "c5", N5, L5, K5, c5_steps, min(args.warmup, 5), dist, world, rank, dev,
+                          do_e2e=False, clock_index=None, dump_prefix="c5_")
+        c5 = {"workload": workload_name("c5", N5, L5, K5, world), "n_gpus": world, "steps": c5_steps,
               "ms_per_step": r5["ms"] / r5["steps"], "value": r5["value"], "unit": "ties/s",
               "iter_per_s": r5["steps"] / (r5["ms"] * 1e-3), "ties": r5["ties"], "nnz_X": r5["nnz_X"],
               "special_ties": r5["special_ties"], "slab_gb_per_gpu": r5["slab_gb_per_gpu"],

@@ -120,6 +120,36 @@ def save_fixture(name, X, R, L, N, M, K, model_kwargs, fit_kwargs, rec, extra=No
     print("wrote", path, os.path.getsize(path) // 1024, "KiB", "iters", len(its), "elbo[-1]", its[-1]["elbo"])
 
 
+def reference_prior(seed, L, N, K, ties):
+    """The reference's random prior of `ties` ((n, 3) l,i,j): `1 + 0.01 * RandomState(seed).rand(L, N, N, K)` normalised
+    per tie (model.py:470-472, bias0 = 0), the first draw of the fit's stream."""
+    d = np.random.RandomState(int(seed)).rand(L, N, N, K)
+    pr = 1.0 + 0.01 * d[ties[:, 0], ties[:, 1], ties[:, 2]]
+    return pr / pr.sum(axis=-1)[:, None]
+
+
+def shrink_fixture(name, rho_fraction=0.5, check_rows=64):
+    """Keep a fixture under 1 MB: the random prior is replaced by its seed (redrawn by tests/golden_util.py and checked
+    against its first `check_rows` rows, which stay stored), and the final rho is kept on a seeded sample of
+    `rho_fraction` of the ties (the column/row sums and the argmax sum still cover all of them)."""
+    path = os.path.join(GOLDEN_DIR, name + ".npz")
+    z = np.load(path)
+    out = {k: z[k] for k in z.files}
+    L, N, M, K = (int(v) for v in z["dims"])
+    seed = json.loads(str(z["meta_json"]))["fit_kwargs"]["seed"]
+    pr = reference_prior(seed, L, N, K, z["init_pr_ties"].astype(np.int64))
+    assert np.array_equal(pr, z["init_pr_vals"]), "the stored prior is not the seed's first draw"
+    del out["init_pr_vals"]
+    out["init_pr_seed"] = np.array(seed, dtype=np.int64)
+    out["init_pr_vals_head"] = z["init_pr_vals"][:check_rows]
+    n = len(z["rho_final_ties"])
+    keep = np.sort(np.random.RandomState(0).choice(n, int(rho_fraction * n), replace=False))
+    out["rho_final_ties"] = z["rho_final_ties"][keep]
+    out["rho_final_vals"] = z["rho_final_vals"][keep]
+    np.savez_compressed(path, **out)
+    print("shrunk", path, os.path.getsize(path) // 1024, "KiB")
+
+
 def scenario_f1(vm, exaggeration):
     """`test_model.py:117-188` (over) / `:263-334` (under): the reference's only known answers."""
     from sklearn.metrics import f1_score
@@ -280,6 +310,7 @@ def scenario_gm_n640_l2_k3(vm):
     model_kwargs = dict(mutuality=True, convergence_tol=0.0)
     rec = run_reference_trace(gt.X, fit_kwargs, model_kwargs)
     save_fixture("gm_n640_l2_k3", gt.X, gt.R, 2, 640, 640, 3, model_kwargs, fit_kwargs, rec, keep_rho="summary")
+    shrink_fixture("gm_n640_l2_k3")
 
 
 SCENARIOS = {

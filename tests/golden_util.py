@@ -56,8 +56,21 @@ class Golden:
         return dict(
             gamma_shp=z["init_gamma_shp"], gamma_rte=z["init_gamma_rte"], phi_shp=z["init_phi_shp"],
             phi_rte=z["init_phi_rte"], nu_shp=float(z["init_nu_shp"]),
-            pr_ties=z["init_pr_ties"].astype(np.int64), pr_vals=z["init_pr_vals"],
+            pr_ties=z["init_pr_ties"].astype(np.int64), pr_vals=self.init_pr_vals(),
         )
+
+    def init_pr_vals(self):
+        """Prior of the ties `init_pr_ties`.  Large fixtures store the reference's seed instead of the values
+        (oracle/gen_golden.py, shrink_fixture): the draw is redone and checked against the rows kept."""
+        from oracle.gen_golden import reference_prior
+
+        z = self.z
+        if "init_pr_vals" in z.files:
+            return z["init_pr_vals"]
+        pr = reference_prior(int(z["init_pr_seed"]), self.L, self.N, self.K, z["init_pr_ties"].astype(np.int64))
+        head = z["init_pr_vals_head"]
+        assert np.array_equal(pr[: len(head)], head), "redrawn prior differs from the stored rows"
+        return pr
 
     def R_coo(self):
         """Explicit COO (subs (4,nnz), vals) of the mask -- for feeding the public API."""
