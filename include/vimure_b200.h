@@ -122,9 +122,9 @@ typedef struct vm_ctx {
                   ln rho_k/rho_0 = ln2 lo_k - S (E[lambda_k]-E[lambda_0])
                                    + x [ (f_k-f_0) E[log theta_m] + f_k E[log lambda_k] - f_0 E[log lambda_0] ],
                every term O(1..30).
-     On iterations that store the slab and do not evaluate the ELBO a light fp32 kernel (k_shortcut: one thread per tie,
-     coalesced per-tie constants + one 16-byte per-node table gather, no entry list, no fp64 transcendental) evaluates
-     these ties -- posterior into rho_u32, (posterior - closed form) into the fixed-point per-reporter corrections, the
+     On iterations that store the slab and do not evaluate the ELBO the dense kernel itself (k_dense_sc: in fp32, from
+     one 16/32-byte record per tie (u_rec) and the per-node table, no entry list, no fp64 transcendental) evaluates
+     these ties -- posterior into the slab and rho_u32, (posterior - closed form) into the fixed-point per-reporter corrections, the
      SINGLE ties' part of the nu statistic (x z2 sum_k rho_k/(z1_k+z2), model.py:822-825) -- and the fp64 special-tie
      kernel only visits the others (`cx_idx`, `cx_*`); every other iteration runs the special-tie kernel over all special
      ties in fp64, as does any layer for which k_phi_finish cannot rule out a completely underflowed tie or an fp32 range

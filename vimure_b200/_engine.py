@@ -168,7 +168,7 @@ class CaviEngine:
         if elbo:
             n += 1 + (1 if self.mutuality else 0)
         elif self.simple_mode and fast:
-            n += 2  # the special-tie kernel is launched twice (layers that take the shortcut / that cannot) + k_shortcut
+            n += 2  # the special-tie kernel is launched twice (layers that take the shortcut / that cannot) + k_patch_rest
         elif self.all32_mode:
             n += 1  # k_all32 + the fp64 special-tie kernel for the layers whose guard fails
         return n

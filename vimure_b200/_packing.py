@@ -228,7 +228,7 @@ def pack_torch(X_subs, X_vals, L, N, M, K, mask, device, row0=0, nloc=None, tile
     P.t["u_x0sum"] = x0sum.to(torch.float32).contiguous()
     # ---- shortcut ties (include/vimure_b200.h, vm_ctx.simple_mode): off the diagonal, in a full column tile, and either
     # SIMPLE (no entry with a reciprocal report) or SINGLE (exactly one entry, with a reciprocal report, reported by the row
-    # or the column node).  On iterations without ELBO the shortcut kernel (k_shortcut) evaluates them and the special-tie kernel walks
+    # or the column node).  On iterations without ELBO the dense kernel (k_dense_sc) evaluates them and the special-tie kernel walks
     # `cx_idx`, the others, through compacted copies of their per-tie arrays.
     P.simple_ok = bool(simple and mask.kind == "ego" and K <= 4 and (N * K) % 4 == 0 and N >= TILE_W and P.tile_h <= 128
                        and (split_e0 or not mutuality) and U > 0 and N < (1 << 24))

@@ -225,7 +225,7 @@ __device__ __forceinline__ void vm_alloc(bool mut, double x, double xT, double G
 #define VM_LC_LP0(K) (2 * (K) + 1)     // log(1+EPS)
 #define VM_LC_LPK(K) (2 * (K) + 2)     // log(EPS)
 #define VM_LC_DEAD(K) (2 * (K) + 3)    // != 0: some closed-form row of this layer may underflow completely
-#define VM_LC_SIMPLE(K) (2 * (K) + 4)  // != 0: the fp32 kernels (k_shortcut / k_all32) evaluate the special ties of this layer
+#define VM_LC_SIMPLE(K) (2 * (K) + 4)  // != 0: the fp32 kernels (k_dense_sc / k_all32) evaluate the special ties of this layer
 #define VM_LC_G(K, k) (2 * (K) + 5 + (k))  // (E[log lambda_k] - E[log lambda_0]) log2e
 // fixed-point scale of fixP (sums of rho_k X over the simple ties of a layer: up to ~1e7)
 #define VM_FIXP_SCALE 1073741824.0

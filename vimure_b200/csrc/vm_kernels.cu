@@ -5,9 +5,11 @@
 //   phase phi   : k_gamma_finish -> k_phi_partial -> k_phi_reduce         (red2)
 //   phase rho   : k_phi_finish -> k_tables
 //                 -> special ties: k_special<K> (fp64; every special tie on ELBO iterations, the non-shortcut ones otherwise)
-//                                  + k_shortcut<K> (ego mask, fp32) | k_all32<K> (all-reporter mask, fp32, entry-parallel)
-//                 -> every tie:    k_dense_tma<K> (TMA bulk stores; the HBM-bound kernel) + k_dense<K> (partial tiles,
-//                                  general masks, dead rows) on the aux stream, k_sums_stage1 / k_elbo_b next to them
+//                                  | k_all32<K> (all-reporter mask, fp32, entry-parallel)
+//                 -> every tie:    k_dense_tma<K> (TMA bulk stores; the HBM-bound kernel), or k_dense_sc<K> (the same, also
+//                                  evaluating the shortcut ties in fp32; ego mask, no ELBO), + k_dense<K> (partial tiles,
+//                                  general masks, dead rows) on the aux stream, k_sums_stage1 / k_elbo_b next to them (and
+//                                  next to k_dense_sc, the list-mode k_special) -> [k_patch_rest]
 //                 -> k_col_reduce -> k_stats_* -> k_sums_reduce   (red3)
 //   phase finish: [k_elbo_partial] -> k_finish
 // All reductions are two-pass (block partials, then a fixed-order second pass) or integer atomics on fixed-point values:
@@ -474,7 +476,7 @@ __device__ __forceinline__ double vm_Er(const vm_ctx& c, int l, int n) {
   return (n < (int)c.M && c.rep[(int64_t)l * c.M + n]) ? c.E_theta[(int64_t)l * c.M + n] : 0.0;
 }
 
-// per-node table of the shortcut-tie kernel (k_shortcut): q_1..q_{K-1}, G_theta, E[log theta] log2e, active flag
+// per-node table of the shortcut ties (k_dense_sc): q_1..q_{K-1}, G_theta, E[log theta] log2e, active flag
 template <int K>
 struct NodeTab {
   static constexpr int STRIDE = (K == 2) ? 4 : (K <= 6 ? 8 : K + 2);
@@ -622,7 +624,7 @@ __device__ __forceinline__ void vm_fix_accumulate(unsigned long long* fix_l, boo
 #ifndef VM_SPECIAL_MINBLK
 #define VM_SPECIAL_MINBLK 3
 #endif
-// LIST (ego mask, no ELBO), for the iterations on which k_shortcut evaluates the shortcut ties of the layers flagged
+// LIST (ego mask, no ELBO), for the iterations on which k_dense_sc evaluates the shortcut ties of the layers flagged
 // VM_LC_SIMPLE.  LIST = 1 handles those layers: it walks the special ties that take NO shortcut through their compacted
 // copies of the per-tie arrays (`cx_*`: coalesced; walking the original arrays at low density multiplied the DRAM bytes
 // read per tie, profiles/ncu_r1_simple_dense_fast_special.txt); its grid covers that list only (n_cxblk blocks per
@@ -942,14 +944,8 @@ __global__ void __launch_bounds__(256, (K <= 2 ? (ELBO ? 3 : VM_SPECIAL_MINBLK) 
 // pointers and row terms of the next row and the patch data of the current row are prefetched before the arithmetic.
 // Column partials of the 8 warps are combined through shared memory once, at the end of the CTA.
 // TW = 128*NCH depends on K so that the column accumulators (NCH*4*(K-1) registers) stay in registers.
-__device__ __forceinline__ void vm_cp_async4(void* smem, const void* g) {
-  const unsigned s = (unsigned)__cvta_generic_to_shared(smem);
-  asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(s), "l"(g));
-}
-__device__ __forceinline__ void vm_cp_async_commit() { asm volatile("cp.async.commit_group;"); }
-__device__ __forceinline__ void vm_cp_async_wait_all() { asm volatile("cp.async.wait_group 0;" ::: "memory"); }
 
-// does k_dense_fast handle this (layer, column tile)?  (everything else is k_dense's)
+// does a TMA dense kernel handle this (layer, column tile)?  (everything else is k_dense's)
 template <int K>
 __device__ __forceinline__ bool vm_fast_tile(const vm_ctx& c, int l, int ct) {
   return (((c.N * K) & 3) == 0) && ((int64_t)(ct + 1) * DenseCfg<K>::TW <= c.N) && c.r_mode != VM_R_CSR &&
@@ -1045,7 +1041,7 @@ __global__ void __launch_bounds__(VM_DENSE_THREADS) k_dense(const __grid_constan
   const int ct = blockIdx.x;
   const int l = blockIdx.y / rtn, rt = rt0 + (blockIdx.y - l * rtn);  // row tiles [rt0, rt0+rtn) of every layer
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  if (skip_fast && vm_fast_tile<K>(c, l, ct)) return;  // k_dense_fast has written this tile
+  if (skip_fast && vm_fast_tile<K>(c, l, ct)) return;  // a TMA dense kernel has written this tile
   const int jt = ct * TW;
   const int i_lo = rt * (int)c.tile_h, i_hi = min(i_lo + (int)c.tile_h, nloc);
   const bool may_dead = vm_may_dead<K>(c, l);
@@ -1191,233 +1187,29 @@ __global__ void __launch_bounds__(VM_DENSE_THREADS) k_dense(const __grid_constan
   }
 }
 
-// ---- fast variant of the dense kernel ---------------------------------------------------------------------------
+// ---- fast (TMA) dense kernels: tile limit ---------------------------------------------------------------------------
 // Same tiling and warp-autonomous structure as k_dense, for the common case: separable mask (ego / all), slab stored,
-// no ELBO, N*K % 4 == 0, column tile entirely inside the matrix, and no row of the layer can underflow completely
-// (checked on the device; k_dense handles every tile this kernel skips).  ~10 instructions per tie, branch-free
-// chunk loop.  Everything the row loop needs from global memory (column/row terms, tile pointers) is fetched once
-// per CTA, and the patch data of the warp's rows are staged with cp.async into shared memory up front, so nothing
-// in the row loop waits on a load.
+// K <= 4, N*K % 4 == 0, column tile entirely inside the matrix, and no row of the layer can underflow completely
+// (checked on the device; k_dense handles every tile they skip).  ~10 instructions per tie, branch-free chunk loop.
 #define VM_FAST_MAX_TILE_H 128
 
-#ifndef VM_FAST_CAPW
-#define VM_FAST_CAPW 320
-#endif
-template <int K>
-struct FastCfg {
-  // special ties staged per warp (all the rows of the warp); the rest are fetched directly.  A warp owns tile_h/8 = 16
-  // row segments of TW = 512 ties: ~300 special ties at the density of config 3 (3.7 %)
-  static constexpr int CAPW = VM_FAST_CAPW;
-};
-
-#ifndef VM_FAST_MINBLK2
-#define VM_FAST_MINBLK2 4
-#endif
-
-// shared memory of k_dense_fast (dynamic: K >= 3 needs more than the 48 KB a static allocation may hold)
-template <int K>
-struct FastSmem {
-  static constexpr int TW = DenseCfg<K>::TW, NW = VM_DENSE_THREADS / 32, CAPW = FastCfg<K>::CAPW, TH = VM_FAST_MAX_TILE_H;
-  float qs[K - 1][TW];      // column terms of the log2-odds
-  float colbuf[K - 1][TW];  // cross-warp column sums
-  float stage[NW][StageCfg<K>::FLOATS];
-  float pval[NW][CAPW][K];  // staged patch data of the warp's rows
-  int pcol[NW][CAPW];
-  float ps[K - 1][TH];      // row terms
-  int tp0[TH], tp1[TH];     // special-tie range of every row segment
-  double sm_red[8];
-};
-
-template <int K, bool ELBO>
-__global__ void __launch_bounds__(VM_DENSE_THREADS, (K <= 2 && !ELBO) ? VM_FAST_MINBLK2 : 2) k_dense_fast(const __grid_constant__ vm_ctx c, double* catpart, int rt0, int rtn) {
-  constexpr int NCH = DenseCfg<K>::NCH, TW = DenseCfg<K>::TW, NW = VM_DENSE_THREADS / 32, CAPW = FastCfg<K>::CAPW;
-  extern __shared__ __align__(16) unsigned char vm_fast_smem[];
-  FastSmem<K>& S = *reinterpret_cast<FastSmem<K>*>(vm_fast_smem);
-  const int N = (int)c.N, nloc = (int)c.nloc, nct = (int)c.nct, nrt = (int)c.nrt;
-  const int ct = blockIdx.x;
-  const int l = blockIdx.y / rtn, rt = rt0 + (blockIdx.y - l * rtn);  // row tiles [rt0, rt0+rtn) of every layer
-  if (!vm_fast_tile<K>(c, l, ct)) return;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int jt = ct * TW;
-  const int i_lo = rt * (int)c.tile_h;
-  const int nrows = min((int)c.tile_h, nloc - i_lo);
-  const double* lc = c.layer_consts + (int64_t)l * VM_LC_STRIDE(K);
-  const float lp0 = (float)lc[VM_LC_LP0(K)], lpk = (float)lc[VM_LC_LPK(K)], epsf = (float)c.eps;
-  double cat = 0.0;
-  const float* patch_src = c.rho_u32;
-  // ---- phase 0: everything the row loop reads from global memory, once per CTA
-  for (int idx = tid; idx < TW; idx += VM_DENSE_THREADS) {
-#pragma unroll
-    for (int k = 1; k < K; ++k) {
-      S.qs[k - 1][idx] = __ldg(&c.tab_q[((int64_t)l * N + jt + idx) * K + k]);
-      S.colbuf[k - 1][idx] = 0.f;
-    }
-  }
-  for (int r = tid; r < nrows; r += VM_DENSE_THREADS) {
-    const int64_t lrow = (int64_t)l * nloc + i_lo + r;
-#pragma unroll
-    for (int k = 1; k < K; ++k) S.ps[k - 1][r] = __ldg(&c.tab_p[lrow * K + k]);
-    S.tp0[r] = __ldg(&c.utile_ptr[lrow * nct + ct]);
-    S.tp1[r] = __ldg(&c.utile_ptr[lrow * nct + ct + 1]);
-  }
-  __syncthreads();
-  // ---- phase 1: stage the patch data of this warp's rows asynchronously
-  {
-    int off = 0;
-    for (int r = warp; r < nrows; r += NW) {
-      const int ua = S.tp0[r], n = S.tp1[r] - ua;
-      const int take = min(n, CAPW - off);
-      for (int e = lane; e < take; e += 32) {
-        vm_cp_async4(&S.pcol[warp][off + e], &c.u_col[ua + e]);
-#pragma unroll
-        for (int k = 0; k < K; ++k) vm_cp_async4(&S.pval[warp][off + e][k], &patch_src[(int64_t)(ua + e) * K + k]);
-      }
-      off += take;
-    }
-    vm_cp_async_commit();
-  }
-  // ---- phase 2: the rows (no global loads on the critical path)
-  float colacc[NCH][K - 1][4];
-#pragma unroll
-  for (int ch = 0; ch < NCH; ++ch)
-#pragma unroll
-    for (int k = 0; k < K - 1; ++k)
-#pragma unroll
-      for (int t = 0; t < 4; ++t) colacc[ch][k][t] = 0.f;
-  int off = 0;
-  bool waited = false;
-  // the shuffle reduction of a row's partial sums is software-pipelined into the NEXT row's chunk loop (one step per
-  // chunk), so that its dependent SHFL->FADD chain never stalls the warp
-  float prev[K];
-  int64_t prev_idx = -1;
-#pragma unroll
-  for (int k = 1; k < K; ++k) prev[k] = 0.f;
-  for (int r = warp; r < nrows; r += NW) {
-    const int64_t lrow = (int64_t)l * nloc + i_lo + r;
-    float p[K];
-#pragma unroll
-    for (int k = 1; k < K; ++k) p[k] = S.ps[k - 1][r];
-    float rowacc[K];
-#pragma unroll
-    for (int k = 1; k < K; ++k) rowacc[k] = 0.f;
-    float* rowdst = c.rho + lrow * N * K;
-    float* dst = rowdst + (int64_t)jt * K;
-#pragma unroll
-    for (int ch = 0; ch < NCH; ++ch) {
-      float qv[K][4];
-#pragma unroll
-      for (int k = 1; k < K; ++k) vm_load_q4<K>(&S.qs[k - 1][ch * 128], lane, qv[k]);
-      float o[4 * K];
-#pragma unroll
-      for (int t = 0; t < 4; ++t) {
-        // identical operation order to vm_formula_rho: s = ((0 + e1) + e2) + ..., inv = rcp(1 + s)
-        float e[K], s = 0.f;
-#pragma unroll
-        for (int k = 1; k < K; ++k) {
-          e[k] = vm_ex2(fminf(__fadd_rn(p[k], qv[k][t]), VM_CLAMP_LOG2));
-          s = (k == 1) ? e[k] : __fadd_rn(s, e[k]);
-        }
-        const float inv = vm_rcp(__fadd_rn(1.f, s));
-        o[t * K] = inv;
-#pragma unroll
-        for (int k = 1; k < K; ++k) {
-          const float v = __fmul_rn(e[k], inv);
-          o[t * K + k] = v;
-          colacc[ch][k - 1][t] += v;
-          rowacc[k] += v;
-        }
-        if (ELBO) cat += (double)vm_formula_cat<K>(&o[t * K], s, false, lp0, lpk, epsf);
-      }
-      vm_store_chunk<K>(dst + (int64_t)ch * 128 * K, lane, o, S.stage[warp]);
-      if (ch < 5) {  // step `ch` of the previous row's reduction (same order as warp_sum: 16, 8, 4, 2, 1)
-#pragma unroll
-        for (int k = 1; k < K; ++k) prev[k] += __shfl_down_sync(0xffffffffu, prev[k], 16 >> ch);
-      }
-    }
-#pragma unroll
-    for (int st = NCH; st < 5; ++st) {
-#pragma unroll
-      for (int k = 1; k < K; ++k) prev[k] += __shfl_down_sync(0xffffffffu, prev[k], 16 >> st);
-    }
-    // ---- row partials of the previous row; this row's become `prev`
-    if (prev_idx >= 0 && lane == 0) {
-      c.rowpart[prev_idx] = 0.f;
-#pragma unroll
-      for (int k = 1; k < K; ++k) c.rowpart[prev_idx + k] = prev[k];
-    }
-    prev_idx = (lrow * nct + ct) * K;
-#pragma unroll
-    for (int k = 1; k < K; ++k) prev[k] = rowacc[k];
-    // ---- patch the special ties of this row segment (after the row's own stores)
-    if (!waited) {
-      vm_cp_async_wait_all();
-      waited = true;
-    }
-    __syncwarp();
-    const int ua = S.tp0[r], n = S.tp1[r] - ua;
-    const int take = min(n, CAPW - off);
-    for (int e = lane; e < n; e += 32) {
-      int col;
-      float v[K];
-      if (e < take) {
-        col = S.pcol[warp][off + e];
-#pragma unroll
-        for (int k = 0; k < K; ++k) v[k] = S.pval[warp][off + e][k];
-      } else {  // more special ties than the per-warp stage holds
-        col = c.u_col[ua + e];
-#pragma unroll
-        for (int k = 0; k < K; ++k) v[k] = patch_src[(int64_t)(ua + e) * K + k];
-      }
-      float* d = rowdst + (int64_t)col * K;
-#pragma unroll
-      for (int k = 0; k < K; ++k) d[k] = v[k];
-    }
-    off += take;
-  }
-  if (prev_idx >= 0) {  // the last row of this warp
-#pragma unroll
-    for (int k = 1; k < K; ++k) prev[k] = warp_sum(prev[k]);
-    if (lane == 0) {
-      c.rowpart[prev_idx] = 0.f;
-#pragma unroll
-      for (int k = 1; k < K; ++k) c.rowpart[prev_idx + k] = prev[k];
-    }
-  }
-  // ---- column partials: combine the 8 warps in a fixed order
-  for (int w = 0; w < NW; ++w) {
-    if (warp == w) {
-#pragma unroll
-      for (int ch = 0; ch < NCH; ++ch)
-#pragma unroll
-        for (int k = 1; k < K; ++k)
-#pragma unroll
-          for (int t = 0; t < 4; ++t) S.colbuf[k - 1][ch * 128 + vm_tie_of<K>(lane, t)] += colacc[ch][k - 1][t];
-    }
-    __syncthreads();
-  }
-  for (int idx = tid; idx < TW; idx += VM_DENSE_THREADS) {
-    float* cp = c.colpart + (((int64_t)l * nrt + rt) * N + jt + idx) * K;
-    cp[0] = 0.f;
-#pragma unroll
-    for (int k = 1; k < K; ++k) cp[k] = S.colbuf[k - 1][idx];
-  }
-  if (ELBO) {
-    const double v = block_sum<VM_DENSE_THREADS>(cat, S.sm_red);
-    if (tid == 0) catpart[((int64_t)l * nrt + rt) * nct + ct] = v;
-  }
-}
-
-// ---- TMA variant of the fast dense kernel ---------------------------------------------------------------------------
-// Same tiling, arithmetic and partials as k_dense_fast.  What differs is how a row segment reaches HBM: the warp writes
-// its TW ties into a per-warp shared-memory stage in the slab's own layout (conflict-free 128-bit shared stores),
-// overwrites the special ties of the segment IN SHARED MEMORY, and one lane hands the whole segment (TW*K*4 bytes: 4 KB at
-// K = 2) to the TMA engine with ONE bulk store (cp.async.bulk.global.shared::cta).  The slab then only ever sees full,
-// contiguous writes: k_dense_fast's scattered 4-byte patch stores (two per special tie: 3e7 partial-sector L2 writes per
-// launch at config 3, +30 % write requests) cost it 0.11 ms of its 0.60 ms (measured: the same kernel without them takes
-// 0.497 ms, profiles/r2_dense_experiments.txt).  Two stages per warp: the next row is computed while the engine still reads
-// the previous one (cp.async.bulk.wait_group.read 1 before a stage is refilled).  The patch data of the NEXT row of the
-// warp are requested (one special tie per lane, registers) before the current row is swept, so their latency -- several
-// microseconds under a saturated store stream -- is covered by a whole row of work.
+// ---- TMA dense kernel ------------------------------------------------------------------------------------------------
+// A row segment reaches HBM in ONE piece: the warp writes its TW ties into a per-warp shared-memory stage in the slab's own
+// layout (conflict-free 128-bit shared stores), overwrites the special ties of the segment IN SHARED MEMORY, and one lane
+// hands the whole segment (TW*K*4 bytes: 4 KB at K = 2) to the TMA engine with ONE bulk store
+// (cp.async.bulk.global.shared::cta).  The slab then only ever sees full, contiguous writes: scattered 4-byte patch stores
+// (two per special tie: 3e7 partial-sector L2 writes per launch at config 3, +30 % write requests) cost an STG.128 version
+// of this kernel 0.11 ms of its 0.60 ms (profiles/r2_dense_experiments.txt).  Two stages per warp: the next row is computed
+// while the engine still reads the previous one (cp.async.bulk.wait_group.read 1 before a stage is refilled).  The patch
+// data of the NEXT row of the warp are requested (one special tie per lane, registers) before the current row is swept, so
+// their latency -- several microseconds under a saturated store stream -- is covered by a whole row of work.
+//
+// SC (k_dense_sc, iterations without ELBO in vm_ctx.simple_mode): the special ties of a segment that take the shortcut
+// are EVALUATED in the stage instead of patched from rho_u32 (vm_shortcut_tie), between filling the stage and the bulk
+// store; the prefetched data are their 16/32-byte records `u_rec` and the row node's node-table entry.  Every other special
+// tie of the segment (the special-tie kernel's list ties, and all special ties of a layer whose VM_LC_SIMPLE guard fails)
+// keeps its closed form here; k_patch_rest copies their rho_u32 into the slab once the special-tie kernel, which runs
+// next to this one, has written it.  The dense partials only ever count the closed form, so nothing else waits for it.
 __device__ __forceinline__ void vm_bulk_store(void* gdst, const void* ssrc, uint32_t bytes) {
   asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(gdst),
                "r"((uint32_t)__cvta_generic_to_shared(ssrc)), "r"(bytes)
@@ -1431,15 +1223,32 @@ __device__ __forceinline__ void vm_bulk_wait_read() {
 __device__ __forceinline__ void vm_bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
 __device__ __forceinline__ void vm_fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
+// A fixed-point correction fq (|fq| <= 2^42) is accumulated in shared memory as TWO 32-bit words, fq = hi * 2^22 + lo with
+// lo = the low 22 bits (unsigned) and hi = fq >> 22 (signed, |hi| <= 2^20): a node of a tile receives at most TW = 512
+// terms, so neither word can overflow (512 * 2^22 = 2^31), the two native 32-bit adds need no carry -- hence no returned
+// value to wait for: a 64-bit shared-memory atomic is a compare-and-swap spin loop (ATOMS.CAST.SPIN.64), and a carry taken
+// from the returned old value exposed the atomic's latency twice per tie and category -- and the sum is exact.
+__device__ __forceinline__ void vm_smem_add_split(unsigned int* w, long long v) {
+  atomicAdd(&w[0], (unsigned int)((unsigned long long)v & 0x3fffffull));
+  atomicAdd(&w[1], (unsigned int)(int)(v >> 22));
+}
+__device__ __forceinline__ unsigned long long vm_smem_split_value(const unsigned int* w) {
+  return (unsigned long long)((long long)(int)w[1] * 4194304ll + (long long)w[0]);
+}
+
 #define VM_TMA_NBUF 2
-template <int K>
+template <int K, bool SC = false>
 struct TmaSmem {
   static constexpr int TW = DenseCfg<K>::TW, NW = VM_DENSE_THREADS / 32, TH = VM_FAST_MAX_TILE_H;
   float rowbuf[NW][VM_TMA_NBUF][TW * K];  // row-segment stages (slab layout), 128-byte aligned (first member)
   float qs[K - 1][TW];                    // column terms of the log2-odds
-  float colbuf[K - 1][TW];                // cross-warp column sums
+  union {
+    float colbuf[K - 1][TW];                     // cross-warp column sums (after the row loop)
+    unsigned int colfix[SC ? TW : 1][K - 1][2];  // SC, row loop: corrections of the column reporters (vm_smem_add_split)
+  };
   float ps[K - 1][TH];                    // row terms
   int tp0[TH], tp1[TH];                   // special-tie range of every row segment
+  float lam[SC ? 4 * K + 1 : 1];          // SC: G_lambda_k | G_lambda_k - G_lambda_0 | E[log lambda_k] log2e | G_nu | g_k
   double sm_red[8];
 };
 
@@ -1459,14 +1268,101 @@ __device__ __forceinline__ void vm_stage_chunk(float* sb_chunk, int lane, const 
   }
 }
 
+// ---- shortcut ties: the special ties whose posterior needs no fp64 and no entry list ---------------------------------
+// (vm_ctx.simple_mode.)  A special tie u with u_px[u] > 0 takes the shortcut; its record u_rec[u] holds the column,
+// X = u_px (total count of a SIMPLE tie / the count of a SINGLE tie's one report), xt = u_pxt (0 = SIMPLE; +-x^T = SINGLE,
+// sign: reported by the row / the column node) and lo_k = u_lo = log2((pr_k+EPS)/(pr_0+EPS)).  With the per-node table
+// nodetab[l,n] = (q_1..q_{K-1}, G_theta, E[log theta] log2e, active) written by k_tables, q_k = -E[theta_n] d_k:
+//   log2 rho_k/rho_0 = q_k(i) + q_k(j) + lo_k + dat_k,
+//   SIMPLE: dat_k = X (E[log lambda_k]-E[log lambda_0]) log2e
+//   SINGLE: f_k = z1_k/(z1_k+z2), z1_k = G_theta_m G_lambda_k, z2 = G_nu x^T (model.py:686-696),
+//           dat_k = x log2e [ (f_k-f_0) E[log theta_m] + f_k E[log lambda_k] - f_0 E[log lambda_0] ]
+// every term O(1..30): fp32 does not cancel (the closed form's own p+q ~ -40 would).  The tie is accounted for exactly as
+// the special-tie kernel would: fp32 posterior rho[K] (into the slab, and into rho_u32, which the gamma/phi passes gather),
+// fq[k] = (posterior - closed form cf[k]) in fixed point for the per-reporter corrections, rho_k X of a SIMPLE tie into p0
+// (its part of the next phi-shape sums, fixP), sum_k dz2_k rho_k = x z2 sum_k rho_k/(z1_k+z2) of a SINGLE tie
+// (model.py:822-825) into nu (dev_flags[VM_FLAG_FIXNU]).  ni / nj: node-table entries of the row / column node; lam:
+// TmaSmem::lam.
+template <int K>
+__device__ __forceinline__ void vm_shortcut_tie(const float* rec, const float* ni, const float* nj, const float* lam,
+                                                const float* cf, float* rho, long long* fq, float& nu, float* p0) {
+  const float X = rec[1];
+  const float xt = rec[2];
+  const bool single = xt != 0.f, rowrep = xt > 0.f;
+  const float g = single ? (rowrep ? ni[K - 1] : nj[K - 1]) : 1.f;
+  const float el = single ? (rowrep ? ni[K] : nj[K]) : 0.f;
+  const float z2 = lam[3 * K] * fabsf(xt);
+  float f[K], iden[K];
+#pragma unroll
+  for (int k = 0; k < K; ++k) {
+    const float z1 = g * lam[k];
+    iden[k] = vm_rcp(z1 + z2);
+    f[k] = single ? z1 * iden[k] : 1.f;
+  }
+  const float t0 = z2 * g * iden[0];
+  // log2-odds against k = 0, then a softmax with the maximum subtracted: for K >= 3 the odds of two categories can
+  // both be astronomically large (a tie with a count of 20: 2^140) and only their RATIO matters -- clamping them (as
+  // the closed form may, its odds being ~2^-40) would flatten it
+  float a[K], amax = 0.f;
+#pragma unroll
+  for (int k = 1; k < K; ++k) {
+    const float dat = single ? X * ((t0 * iden[k] * lam[K + k]) * el + (f[k] * lam[2 * K + k] - f[0] * lam[2 * K]))
+                             : X * lam[3 * K + 1 + k];
+    const float qk = nj[k - 1];
+    a[k] = ni[k - 1] + qk + rec[2 + k] + dat;
+    amax = fmaxf(amax, a[k]);
+  }
+  float es[K], s = vm_ex2(-amax);
+  es[0] = s;
+#pragma unroll
+  for (int k = 1; k < K; ++k) {
+    es[k] = vm_ex2(a[k] - amax);
+    s += es[k];
+  }
+  const float inv = vm_rcp(s);
+  rho[0] = es[0] * inv;
+  float nu_t = rho[0] * iden[0];
+#pragma unroll
+  for (int k = 1; k < K; ++k) {
+    rho[k] = es[k] * inv;
+    nu_t += rho[k] * iden[k];
+    fq[k] = __double2ll_rn(((double)rho[k] - (double)cf[k]) * VM_FIX_SCALE);
+  }
+  if (single) {
+    nu += X * z2 * nu_t;
+  } else {
+#pragma unroll
+    for (int k = 0; k < K; ++k) p0[k] += rho[k] * X;
+  }
+}
+
+// floats per shortcut record u_rec: col, X, +-x^T, lo_1..lo_{K-1}, padding
+template <int K>
+struct ScRec {
+  static constexpr int RS = (K == 2) ? 4 : 8;
+};
+
+// the first K + 2 floats of a shortcut record / node-table entry (col, X, +-x^T, lo_k | q_k, G_theta, E[log theta], active)
+template <int K>
+__device__ __forceinline__ void vm_load_rec(const float* p, float* v) {
+  const float4 a = __ldg(reinterpret_cast<const float4*>(p));
+  v[0] = a.x; v[1] = a.y; v[2] = a.z; v[3] = a.w;
+  if (K == 3) v[4] = __ldg(p + 4);
+  if (K == 4) {
+    const float2 b = __ldg(reinterpret_cast<const float2*>(p + 4));
+    v[4] = b.x; v[5] = b.y;
+  }
+}
+
 #ifndef VM_TMA_PD
 #define VM_TMA_PD 2  // rows of prefetch distance of the patch entries
 #endif
-template <int K, bool ELBO, int PD = VM_TMA_PD>
-__global__ void __launch_bounds__(VM_DENSE_THREADS, (K == 2 || K == 4) ? 3 : 2) k_dense_tma(const __grid_constant__ vm_ctx c, double* catpart, int rt0, int rtn) {
+template <int K, bool ELBO, bool SC, int PD>
+__device__ __forceinline__ void dense_tma_body(const vm_ctx& c, double* catpart, int rt0, int rtn, unsigned char* smem) {
   constexpr int NCH = DenseCfg<K>::NCH, TW = DenseCfg<K>::TW, NW = VM_DENSE_THREADS / 32;
-  extern __shared__ __align__(128) unsigned char vm_tma_smem[];
-  TmaSmem<K>& S = *reinterpret_cast<TmaSmem<K>*>(vm_tma_smem);
+  constexpr int NT = NodeTab<K>::STRIDE, NV = SC ? K + 2 : K;  // floats per prefetched special tie
+  static_assert(!(SC && ELBO), "the shortcut ties are evaluated on iterations without ELBO only");
+  TmaSmem<K, SC>& S = *reinterpret_cast<TmaSmem<K, SC>*>(smem);
   const int N = (int)c.N, nloc = (int)c.nloc, nct = (int)c.nct, nrt = (int)c.nrt;
   const int ct = blockIdx.x;
   const int l = blockIdx.y / rtn, rt = rt0 + (blockIdx.y - l * rtn);  // row tiles [rt0, rt0+rtn) of every layer
@@ -1477,6 +1373,12 @@ __global__ void __launch_bounds__(VM_DENSE_THREADS, (K == 2 || K == 4) ? 3 : 2) 
   const int nrows = min((int)c.tile_h, nloc - i_lo);
   const double* lc = c.layer_consts + (int64_t)l * VM_LC_STRIDE(K);
   const float lp0 = (float)lc[VM_LC_LP0(K)], lpk = (float)lc[VM_LC_LPK(K)], epsf = (float)c.eps;
+  // SC: does this layer take the shortcut?  (if not, k_patch_rest has all its special ties)
+  const bool sc = SC && lc[VM_LC_SIMPLE(K)] != 0.0;
+  // SC: statistics of the shortcut ties (see vm_shortcut_tie): fp32 per thread (~10 ties each), fp64 per CTA
+  float nu = 0.f, p0[K];
+#pragma unroll
+  for (int k = 0; k < K; ++k) p0[k] = 0.f;
   double cat = 0.0;
   const float* patch_src = c.rho_u32;
   // ---- phase 0: tables of the tile, once per CTA
@@ -1484,7 +1386,8 @@ __global__ void __launch_bounds__(VM_DENSE_THREADS, (K == 2 || K == 4) ? 3 : 2) 
 #pragma unroll
     for (int k = 1; k < K; ++k) {
       S.qs[k - 1][idx] = __ldg(&c.tab_q[((int64_t)l * N + jt + idx) * K + k]);
-      S.colbuf[k - 1][idx] = 0.f;
+      if (SC) S.colfix[idx][k - 1][0] = S.colfix[idx][k - 1][1] = 0u;
+      else S.colbuf[k - 1][idx] = 0.f;
     }
   }
   for (int r = tid; r < nrows; r += VM_DENSE_THREADS) {
@@ -1492,7 +1395,15 @@ __global__ void __launch_bounds__(VM_DENSE_THREADS, (K == 2 || K == 4) ? 3 : 2) 
 #pragma unroll
     for (int k = 1; k < K; ++k) S.ps[k - 1][r] = __ldg(&c.tab_p[lrow * K + k]);
     S.tp0[r] = __ldg(&c.utile_ptr[lrow * nct + ct]);
-    S.tp1[r] = __ldg(&c.utile_ptr[lrow * nct + ct + 1]);
+    S.tp1[r] = (SC && !sc) ? S.tp0[r] : __ldg(&c.utile_ptr[lrow * nct + ct + 1]);
+  }
+  if (SC && tid < K) {
+    const double g0 = c.G_lambda[l * K], gkk = c.G_lambda[l * K + tid];
+    S.lam[tid] = (float)gkk;
+    S.lam[K + tid] = (float)(gkk - g0);
+    S.lam[2 * K + tid] = (float)(c.Elog_lambda[l * K + tid] * VM_LOG2E);
+    S.lam[3 * K + 1 + tid] = (float)lc[VM_LC_G(K, tid)];
+    if (tid == 0) S.lam[3 * K] = (float)c.nu[VM_NU_G];
   }
   __syncthreads();
   float colacc[NCH][K - 1][4];
@@ -1502,16 +1413,21 @@ __global__ void __launch_bounds__(VM_DENSE_THREADS, (K == 2 || K == 4) ? 3 : 2) 
     for (int k = 0; k < K - 1; ++k)
 #pragma unroll
       for (int t = 0; t < 4; ++t) colacc[ch][k][t] = 0.f;
-  // patch entries of this lane (special tie tp0[row] + lane) for the next PD rows of the warp, fetched PD rows ahead
+  // patch entries of this lane (special tie tp0[row] + lane) for the next PD rows of the warp, fetched PD rows ahead:
+  // (column, value) -- or, SC, the tie's record and the lane's float of the row node's node-table entry
   int pq_col[PD];
-  float pq_v[PD][K];
-  auto fetch = [&](int row, int& col, float* v) {
+  float pq_v[PD][NV], pq_rn[PD];
+  auto fetch = [&](int row, int& col, float* v, float& rn) {
     col = 0;
+    rn = 0.f;
 #pragma unroll
-    for (int k = 0; k < K; ++k) v[k] = 0.f;
+    for (int k = 0; k < NV; ++k) v[k] = 0.f;
     if (row < nrows) {
       const int ua = S.tp0[row], n = S.tp1[row] - ua;
-      if (lane < n) {
+      if (SC) {
+        if (n > 0) rn = __ldg(c.nodetab + ((int64_t)l * N + (int)c.row0 + i_lo + row) * NT + (lane & (NT - 1)));
+        if (lane < n) vm_load_rec<K>(c.u_rec + (int64_t)(ua + lane) * ScRec<K>::RS, v);
+      } else if (lane < n) {
         col = __ldg(&c.u_col[ua + lane]);
 #pragma unroll
         for (int k = 0; k < K; ++k) v[k] = __ldg(&patch_src[(int64_t)(ua + lane) * K + k]);
@@ -1519,7 +1435,7 @@ __global__ void __launch_bounds__(VM_DENSE_THREADS, (K == 2 || K == 4) ? 3 : 2) 
     }
   };
 #pragma unroll
-  for (int d = 0; d < PD; ++d) fetch(warp + d * NW, pq_col[d], pq_v[d]);
+  for (int d = 0; d < PD; ++d) fetch(warp + d * NW, pq_col[d], pq_v[d], pq_rn[d]);
   float prev[K];
   int64_t prev_idx = -1;
 #pragma unroll
@@ -1529,8 +1445,8 @@ __global__ void __launch_bounds__(VM_DENSE_THREADS, (K == 2 || K == 4) ? 3 : 2) 
     const int64_t lrow = (int64_t)l * nloc + i_lo + r;
     // ---- request the patch entry of the row PD rows ahead
     int pn_col;
-    float pn_v[K];
-    fetch(r + PD * NW, pn_col, pn_v);
+    float pn_v[NV], pn_rn;
+    fetch(r + PD * NW, pn_col, pn_v, pn_rn);
     float p[K];
 #pragma unroll
     for (int k = 1; k < K; ++k) p[k] = S.ps[k - 1][r];
@@ -1590,16 +1506,75 @@ __global__ void __launch_bounds__(VM_DENSE_THREADS, (K == 2 || K == 4) ? 3 : 2) 
     // ---- overwrite the special ties of this row segment in the stage, then hand the segment to the TMA engine
     __syncwarp();
     const int ua = S.tp0[r], n = S.tp1[r] - ua;
-    if (lane < n) {
-      float* d = sb + (pq_col[0] - jt) * K;
+    if constexpr (SC) {
+      if (n > 0) {  // (warp-uniform)
+        float ni[K + 2];
 #pragma unroll
-      for (int k = 0; k < K; ++k) d[k] = pq_v[0][k];
-    }
-    for (int e = 32 + lane; e < n; e += 32) {  // more than 32 special ties in the segment (rare)
-      const int col = __ldg(&c.u_col[ua + e]);
-      float* d = sb + (col - jt) * K;
+        for (int t = 0; t < K + 2; ++t) ni[t] = __shfl_sync(0xffffffffu, pq_rn[0], t);
+        long long frow[K];  // corrections of the row reporter, k >= 1
 #pragma unroll
-      for (int k = 0; k < K; ++k) d[k] = __ldg(&patch_src[(int64_t)(ua + e) * K + k]);
+        for (int k = 1; k < K; ++k) frow[k] = 0;
+        for (int e = lane; e - lane < n; e += 32) {  // more than 32 special ties in the segment: rare
+          float rec[K + 2];
+          if (e < 32) {
+#pragma unroll
+            for (int t = 0; t < K + 2; ++t) rec[t] = pq_v[0][t];
+          } else {
+#pragma unroll
+            for (int t = 0; t < K + 2; ++t) rec[t] = 0.f;
+            if (e < n) vm_load_rec<K>(c.u_rec + (int64_t)(ua + e) * ScRec<K>::RS, rec);
+          }
+          if (rec[1] > 0.f) {  // a shortcut tie (lanes past the end hold X = 0)
+            const int cj = (int)rec[0] - jt;
+            float nj[K + 2];
+            vm_load_rec<K>(c.nodetab + ((int64_t)l * N + jt + cj) * NT, nj);
+            float* d = sb + cj * K;
+            float cf[K], rho[K];
+            long long fq[K];
+#pragma unroll
+            for (int k = 1; k < K; ++k) cf[k] = d[k];  // the closed form the dense partials count for this tie
+            vm_shortcut_tie<K>(rec, ni, nj, S.lam, cf, rho, fq, nu, p0);
+            const bool act_j = nj[K + 1] != 0.f;
+#pragma unroll
+            for (int k = 1; k < K; ++k) {
+              if (act_j && fq[k] != 0) vm_smem_add_split(S.colfix[cj][k - 1], fq[k]);
+              frow[k] += fq[k];
+            }
+#pragma unroll
+            for (int k = 0; k < K; ++k) d[k] = rho[k];
+            float* ru = c.rho_u32 + (int64_t)(ua + e) * K;
+            if (K == 2) {
+              *reinterpret_cast<float2*>(ru) = make_float2(rho[0], rho[1]);
+            } else {
+#pragma unroll
+              for (int k = 0; k < K; ++k) ru[k] = rho[k];
+            }
+          }
+        }
+        if (ni[K + 1] != 0.f) {  // the row node is an active reporter: one atomic per category
+#pragma unroll
+          for (int k = 1; k < K; ++k) {
+            long long v = frow[k];
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
+            if (lane == 0 && v != 0)
+              atomicAdd(reinterpret_cast<unsigned long long*>(c.fixA) + ((int64_t)l * c.M + (int)c.row0 + i_lo + r) * K + k,
+                        (unsigned long long)v);
+          }
+        }
+      }
+    } else {
+      if (lane < n) {
+        float* d = sb + (pq_col[0] - jt) * K;
+#pragma unroll
+        for (int k = 0; k < K; ++k) d[k] = pq_v[0][k];
+      }
+      for (int e = 32 + lane; e < n; e += 32) {  // more than 32 special ties in the segment (rare)
+        const int col = __ldg(&c.u_col[ua + e]);
+        float* d = sb + (col - jt) * K;
+#pragma unroll
+        for (int k = 0; k < K; ++k) d[k] = __ldg(&patch_src[(int64_t)(ua + e) * K + k]);
+      }
     }
     vm_fence_async_smem();
     __syncwarp();
@@ -1608,12 +1583,14 @@ __global__ void __launch_bounds__(VM_DENSE_THREADS, (K == 2 || K == 4) ? 3 : 2) 
 #pragma unroll
     for (int d = 0; d + 1 < PD; ++d) {
       pq_col[d] = pq_col[d + 1];
+      pq_rn[d] = pq_rn[d + 1];
 #pragma unroll
-      for (int k = 0; k < K; ++k) pq_v[d][k] = pq_v[d + 1][k];
+      for (int k = 0; k < NV; ++k) pq_v[d][k] = pq_v[d + 1][k];
     }
     pq_col[PD - 1] = pn_col;
+    pq_rn[PD - 1] = pn_rn;
 #pragma unroll
-    for (int k = 0; k < K; ++k) pq_v[PD - 1][k] = pn_v[k];
+    for (int k = 0; k < NV; ++k) pq_v[PD - 1][k] = pn_v[k];
   }
   if (prev_idx >= 0) {  // the last row of this warp
 #pragma unroll
@@ -1623,6 +1600,22 @@ __global__ void __launch_bounds__(VM_DENSE_THREADS, (K == 2 || K == 4) ? 3 : 2) 
 #pragma unroll
       for (int k = 1; k < K; ++k) c.rowpart[prev_idx + k] = prev[k];
     }
+  }
+  if constexpr (SC) {
+    // ---- corrections of the column reporters: one global atomic per touched node and category; then colfix's space
+    // becomes colbuf
+    __syncthreads();
+    unsigned long long* fix_l = reinterpret_cast<unsigned long long*>(c.fixA) + (int64_t)l * c.M * K;
+    for (int t = tid; t < TW * (K - 1); t += VM_DENSE_THREADS) {
+      const unsigned long long v = vm_smem_split_value(&S.colfix[0][0][0] + 2 * t);
+      if (v != 0ull) atomicAdd(fix_l + (int64_t)(jt + t / (K - 1)) * K + 1 + t % (K - 1), v);
+    }
+    __syncthreads();
+    for (int idx = tid; idx < TW; idx += VM_DENSE_THREADS) {
+#pragma unroll
+      for (int k = 1; k < K; ++k) S.colbuf[k - 1][idx] = 0.f;
+    }
+    __syncthreads();
   }
   // ---- column partials: combine the 8 warps in a fixed order
   for (int w = 0; w < NW; ++w) {
@@ -1646,264 +1639,52 @@ __global__ void __launch_bounds__(VM_DENSE_THREADS, (K == 2 || K == 4) ? 3 : 2) 
     const double v = block_sum<VM_DENSE_THREADS>(cat, S.sm_red);
     if (tid == 0) catpart[((int64_t)l * nrt + rt) * nct + ct] = v;
   }
+  if (sc) {
+    // rho_k X of the SIMPLE ties (their part of the next phi-shape sums) and the nu statistic of the SINGLE ties
+    const double vn = block_sum<VM_DENSE_THREADS>((double)nu, S.sm_red);
+    if (tid == 0 && vn != 0.0)
+      atomicAdd(reinterpret_cast<unsigned long long*>(c.dev_flags) + VM_FLAG_FIXNU,
+                (unsigned long long)__double2ll_rn(vn * VM_FIXP_SCALE));
+#pragma unroll
+    for (int k = 0; k < K; ++k) {
+      const double v = block_sum<VM_DENSE_THREADS>((double)p0[k], S.sm_red);
+      if (tid == 0 && v != 0.0)
+        atomicAdd(reinterpret_cast<unsigned long long*>(c.fixP) + l * K + k,
+                  (unsigned long long)__double2ll_rn(v * VM_FIXP_SCALE));
+    }
+  }
   if (lane == 0) vm_bulk_wait_all();  // the stages must outlive the engine's reads
 }
 
-// ---- shortcut ties: the special ties whose posterior needs no fp64 and no entry list ---------------------------------
-// (vm_ctx.simple_mode.)  One thread per special tie u of the rank, in tie order (row-major): a tie with u_px[u] = 0 is
-// not a shortcut tie and is skipped (the special-tie kernel's list mode has it).  A shortcut tie's constants are
-// X = u_px (total count of a SIMPLE tie / the count of a SINGLE tie's one report), xt = u_pxt (0 = SIMPLE; +-x^T = SINGLE,
-// sign: reported by the row / the column node) and lo_k = u_lo = log2((pr_k+EPS)/(pr_0+EPS)).  With the per-node table
-// nodetab[l,n] = (q_1..q_{K-1}, G_theta, E[log theta] log2e, active) written by k_tables, q_k = -E[theta_n] d_k:
-//   log2 rho_k/rho_0 = q_k(i) + q_k(j) + lo_k + dat_k,
-//   SIMPLE: dat_k = X (E[log lambda_k]-E[log lambda_0]) log2e
-//   SINGLE: f_k = z1_k/(z1_k+z2), z1_k = G_theta_m G_lambda_k, z2 = G_nu x^T (model.py:686-696),
-//           dat_k = x log2e [ (f_k-f_0) E[log theta_m] + f_k E[log lambda_k] - f_0 E[log lambda_0] ]
-// every term O(1..30): fp32 does not cancel (the closed form's own p+q ~ -40 would).  The tie is accounted for exactly as
-// the special-tie kernel would: fp32 posterior into rho_u32 (patch source of the dense kernel, gathered by the gamma/phi
-// passes), (posterior - closed form) into the fixed-point per-reporter corrections -- the closed form recomputed with
-// the dense sweep's operations, same bits --, rho_k X of the SIMPLE ties into fixP (their part of the next phi-shape
-// sums), sum_k dz2_k rho_k = x z2 sum_k rho_k/(z1_k+z2) of the SINGLE ties (model.py:822-825) into dev_flags[VM_FLAG_FIXNU].
-// Tiled like the dense kernel -- one CTA per (layer, row tile of tile_h rows, FULL column tile of TW columns) -- because
-// what limits a tie-ordered version is not arithmetic but scattered access: a warp of 32 consecutive special ties touches
-// 32 different column nodes (table gather + one global atomic each).  Here the node tables of the tile's TW column nodes
-// and tile_h row nodes are staged in shared memory once, the per-reporter corrections are accumulated in shared memory
-// (64-bit integer atomics) and flushed with one global atomic per touched node, and the CTA's ~tile_h*19 special ties are
-// spread over all its threads (a prefix sum over the rows' segments maps a thread to its tie).
-// The kernel is latency-bound (per tie: one record load, ~150 dependent fp32 instructions, two shared-memory atomics, one
-// store), so every thread keeps VM_SC_UNR ties in flight: their records (one 16/32-byte load each: column, X, +-x^T, lo_k
-// packed per tie in `u_rec`) are requested together before any is evaluated, and the tie -> row-segment map is a byte
-// table in shared memory filled once per CTA instead of a binary search per tie.
-// A fixed-point correction fq (|fq| <= 2^42) is accumulated in shared memory as TWO 32-bit words, fq = hi * 2^22 + lo with
-// lo = the low 22 bits (unsigned) and hi = fq >> 22 (signed, |hi| <= 2^20): a node of a tile receives at most TW = 512
-// terms, so neither word can overflow (512 * 2^22 = 2^31), the two native 32-bit adds need no carry -- hence no returned
-// value to wait for: a 64-bit shared-memory atomic is a compare-and-swap spin loop (ATOMS.CAST.SPIN.64), and a carry taken
-// from the returned old value exposed the atomic's latency twice per tie and category -- and the sum is exact.
-__device__ __forceinline__ void vm_smem_add_split(unsigned int* w, long long v) {
-  atomicAdd(&w[0], (unsigned int)((unsigned long long)v & 0x3fffffull));
-  atomicAdd(&w[1], (unsigned int)(int)(v >> 22));
+template <int K, bool ELBO, int PD = VM_TMA_PD>
+__global__ void __launch_bounds__(VM_DENSE_THREADS, (K == 2 || K == 4) ? 3 : 2) k_dense_tma(const __grid_constant__ vm_ctx c, double* catpart, int rt0, int rtn) {
+  extern __shared__ __align__(128) unsigned char vm_tma_smem[];
+  dense_tma_body<K, ELBO, false, PD>(c, catpart, rt0, rtn, vm_tma_smem);
 }
-__device__ __forceinline__ unsigned long long vm_smem_split_value(const unsigned int* w) {
-  return (unsigned long long)((long long)(int)w[1] * 4194304ll + (long long)w[0]);
+// the TMA dense kernel that also evaluates the shortcut ties (iterations without ELBO, vm_ctx.simple_mode).  Prefetch
+// distance 1 row: at K = 2 the records of a second row do not fit in the 80 registers of 3 CTAs per SM.  At K = 4 its
+// column-correction table leaves room for 2 CTAs per SM only.
+template <int K, int PD = 1>
+__global__ void __launch_bounds__(VM_DENSE_THREADS, (K == 2) ? 3 : 2) k_dense_sc(const __grid_constant__ vm_ctx c, int rt0, int rtn) {
+  extern __shared__ __align__(128) unsigned char vm_tma_smem[];
+  dense_tma_body<K, false, true, PD>(c, nullptr, rt0, rtn, vm_tma_smem);
 }
 
-#define VM_SC_THREADS 256
-#define VM_SC_MAXE 6144  // ties of a tile whose row comes from the byte table (the rest falls back to a binary search)
+// Special ties k_dense_sc left at their closed form, copied from rho_u32 into the slab: the list ties of the layers
+// that take the shortcut (cx_*) and every special tie of the other layers.  (Ties of partial column tiles are rewritten
+// with the value k_dense already wrote.)
 template <int K>
-struct ScCfg {
-  static constexpr int RS = (K == 2) ? 4 : 8;   // floats per tie record: col, X, +-x^T, lo_1..lo_{K-1}, padding
-  static constexpr int UNR = (K == 2) ? 4 : 2;  // ties in flight per thread
-};
-
-template <int K>
-__global__ void __launch_bounds__(VM_SC_THREADS) k_shortcut(const __grid_constant__ vm_ctx c) {
-  const int ct = blockIdx.x, lrt = blockIdx.y;
-  constexpr int NT = NodeTab<K>::STRIDE, TW = DenseCfg<K>::TW, TH = VM_FAST_MAX_TILE_H, RS = ScCfg<K>::RS, UNR = ScCfg<K>::UNR;
-  __shared__ __align__(16) float nt_col[TW * NT];
-  __shared__ __align__(16) float nt_row[TH * NT];
-  __shared__ float s_tabp[TH][K - 1];
-  // fixed-point accumulators as (low 22 bits, rest) pairs of 32-bit words, see vm_smem_add_split
-  __shared__ unsigned int colfix[TW][K - 1][2], rowfix[TH][K - 1][2];
-  __shared__ int s_tp0[TH], s_off[TH + 1];
-  __shared__ unsigned char s_row[VM_SC_MAXE];
-  __shared__ float s_lam[3 * K + 1 + K];  // G_lambda_k | G_lambda_k - G_lambda_0 | E[log lambda_k] log2e | G_nu | g_k
-  __shared__ double sm_red[VM_SC_THREADS / 32];
-  const int N = (int)c.N, nloc = (int)c.nloc, nct = (int)c.nct, nrt = (int)c.nrt;
-  const int l = lrt / nrt, rt = lrt - l * nrt;
-  const double* lc = c.layer_consts + (int64_t)l * VM_LC_STRIDE(K);
-  if (lc[VM_LC_SIMPLE(K)] == 0.0) return;  // the special-tie kernel has this layer in full
-  const int tid = threadIdx.x;
-  const int jt = ct * TW, i_lo = rt * (int)c.tile_h;
-  const int nrows = min((int)c.tile_h, nloc - i_lo);
-  // ---- special-tie ranges of the tile's row segments, and their exclusive prefix sum
-  if (tid < TH) {
-    int a = 0, n = 0;
-    if (tid < nrows) {
-      const int64_t lrow = (int64_t)l * nloc + i_lo + tid;
-      a = __ldg(&c.utile_ptr[lrow * nct + ct]);
-      n = __ldg(&c.utile_ptr[lrow * nct + ct + 1]) - a;
-    }
-    s_tp0[tid] = a;
-    s_off[tid + 1] = n;
-  }
-  if (tid == 0) s_off[0] = 0;
-  // ---- node tables of the tile, per-layer constants, cleared accumulators (independent of the scan: issued first)
-  for (int t = tid; t < TW * NT / 4; t += VM_SC_THREADS)
-    reinterpret_cast<float4*>(nt_col)[t] = __ldg(reinterpret_cast<const float4*>(c.nodetab + ((int64_t)l * N + jt) * NT) + t);
-  for (int t = tid; t < nrows * NT / 4; t += VM_SC_THREADS)
-    reinterpret_cast<float4*>(nt_row)[t] =
-        __ldg(reinterpret_cast<const float4*>(c.nodetab + ((int64_t)l * N + (int)c.row0 + i_lo) * NT) + t);
-  for (int t = tid; t < nrows * (K - 1); t += VM_SC_THREADS) {
-    const int r = t / (K - 1), k = t - r * (K - 1) + 1;
-    s_tabp[r][k - 1] = __ldg(&c.tab_p[((int64_t)l * nloc + i_lo + r) * K + k]);
-  }
-  for (int t = tid; t < TW * (K - 1) * 2; t += VM_SC_THREADS) (&colfix[0][0][0])[t] = 0u;
-  for (int t = tid; t < TH * (K - 1) * 2; t += VM_SC_THREADS) (&rowfix[0][0][0])[t] = 0u;
-  if (tid < K) {
-    const double g0 = c.G_lambda[l * K], gkk = c.G_lambda[l * K + tid];
-    s_lam[tid] = (float)gkk;
-    s_lam[K + tid] = (float)(gkk - g0);
-    s_lam[2 * K + tid] = (float)(c.Elog_lambda[l * K + tid] * VM_LOG2E);
-    s_lam[3 * K + 1 + tid] = (float)lc[VM_LC_G(K, tid)];
-    if (tid == 0) s_lam[3 * K] = (float)c.nu[VM_NU_G];
-  }
-  __syncthreads();
-  if (tid < 32) {  // TH = 128 counts: 4 per lane, warp scan
-    int v[4], sum = 0;
+__global__ void __launch_bounds__(256) k_patch_rest(const __grid_constant__ vm_ctx c) {
+  const int l = blockIdx.y;
+  const bool sc = c.layer_consts[(int64_t)l * VM_LC_STRIDE(K) + VM_LC_SIMPLE(K)] != 0.0;
+  const int64_t lnt = (int64_t)c.nloc * c.nct;
+  const int64_t p0 = sc ? c.cx_ptr[l] : c.utile_ptr[l * lnt], p1 = sc ? c.cx_ptr[l + 1] : c.utile_ptr[(l + 1) * lnt];
+  for (int64_t p = p0 + (int64_t)blockIdx.x * blockDim.x + threadIdx.x; p < p1; p += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t u = sc ? c.cx_idx[p] : p;
+    const int lrow = sc ? c.cx_lrow[p] : c.u_lrow[u], col = sc ? c.cx_col[p] : c.u_col[u];
+    float* dst = c.rho + ((int64_t)lrow * c.N + col) * K;
 #pragma unroll
-    for (int q = 0; q < 4; ++q) {
-      v[q] = s_off[1 + 4 * tid + q];
-      sum += v[q];
-    }
-    int inc = sum;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const int t = __shfl_up_sync(0xffffffffu, inc, o);
-      if (tid >= o) inc += t;
-    }
-    int run = inc - sum;
-#pragma unroll
-    for (int q = 0; q < 4; ++q) {
-      run += v[q];
-      s_off[1 + 4 * tid + q] = run;
-    }
-  }
-  __syncthreads();
-  const int total = s_off[TH];
-  if (tid < TH) {  // tie -> row segment byte table
-    const int e1 = min(s_off[tid + 1], VM_SC_MAXE);
-    for (int e = s_off[tid]; e < e1; ++e) s_row[e] = (unsigned char)tid;
-  }
-  __syncthreads();
-  float p0[K], nu = 0.f;
-#pragma unroll
-  for (int k = 0; k < K; ++k) p0[k] = 0.f;
-  for (int e0 = tid; e0 < total; e0 += VM_SC_THREADS * UNR) {
-    int rr[UNR];
-    int64_t uu[UNR];
-    float rec[UNR][RS];
-#pragma unroll
-    for (int q = 0; q < UNR; ++q) {
-      const int e = e0 + q * VM_SC_THREADS;
-      int r = 0;
-      if (e < total) {
-        if (e < VM_SC_MAXE) {
-          r = s_row[e];
-        } else {  // the last r with s_off[r] <= e
-          int lo = 0, hi = TH;
-          while (hi - lo > 1) {
-            const int mid = (lo + hi) >> 1;
-            if (s_off[mid] <= e) lo = mid;
-            else hi = mid;
-          }
-          r = lo;
-        }
-      }
-      rr[q] = r;
-      uu[q] = (int64_t)s_tp0[r] + (e - s_off[r]);
-#pragma unroll
-      for (int v = 0; v < RS; v += 4) {
-        float4 t4 = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (e < total) t4 = __ldg(reinterpret_cast<const float4*>(c.u_rec + uu[q] * RS + v));
-        rec[q][v] = t4.x; rec[q][v + 1] = t4.y; rec[q][v + 2] = t4.z; rec[q][v + 3] = t4.w;
-      }
-    }
-#pragma unroll
-    for (int q = 0; q < UNR; ++q) {
-      const float X = rec[q][1];
-      if (!(X > 0.f)) continue;  // not a shortcut tie (or past the end)
-      const int r = rr[q];
-      const int64_t u = uu[q];
-      const int cj = (int)rec[q][0] - jt;
-      const float xt = rec[q][2];
-      const float* ni = nt_row + r * NT;
-      const float* nj = nt_col + cj * NT;
-      const bool single = xt != 0.f, rowrep = xt > 0.f;
-      const float g = single ? (rowrep ? ni[K - 1] : nj[K - 1]) : 1.f;
-      const float el = single ? (rowrep ? ni[K] : nj[K]) : 0.f;
-      const float z2 = s_lam[3 * K] * fabsf(xt);
-      float f[K], iden[K];
-#pragma unroll
-      for (int k = 0; k < K; ++k) {
-        const float z1 = g * s_lam[k];
-        iden[k] = vm_rcp(z1 + z2);
-        f[k] = single ? z1 * iden[k] : 1.f;
-      }
-      const float t0 = z2 * g * iden[0];
-      // log2-odds against k = 0, then a softmax with the maximum subtracted: for K >= 3 the odds of two categories can
-      // both be astronomically large (a tie with a count of 20: 2^140) and only their RATIO matters -- clamping them (as
-      // the closed form may, its odds being ~2^-40) would flatten it
-      float a[K], amax = 0.f, sf = 0.f, ef[K];
-#pragma unroll
-      for (int k = 1; k < K; ++k) {
-        const float dat = single ? X * ((t0 * iden[k] * s_lam[K + k]) * el + (f[k] * s_lam[2 * K + k] - f[0] * s_lam[2 * K]))
-                                 : X * s_lam[3 * K + 1 + k];
-        const float qk = nj[k - 1];
-        a[k] = ni[k - 1] + qk + rec[q][2 + k] + dat;
-        amax = fmaxf(amax, a[k]);
-        // the closed form the dense sweep counts for this tie: same operations, same bits (qk == tab_q[l,j,k])
-        ef[k] = vm_ex2(fminf(__fadd_rn(s_tabp[r][k - 1], qk), VM_CLAMP_LOG2));
-        sf = (k == 1) ? ef[k] : __fadd_rn(sf, ef[k]);
-      }
-      float es[K], s = vm_ex2(-amax);
-      es[0] = s;
-#pragma unroll
-      for (int k = 1; k < K; ++k) {
-        es[k] = vm_ex2(a[k] - amax);
-        s += es[k];
-      }
-      const float inv = vm_rcp(s), invf = vm_rcp(__fadd_rn(1.f, sf));
-      float rho[K];
-      rho[0] = es[0] * inv;
-      float nu_t = rho[0] * iden[0];
-      const bool act_i = ni[K + 1] != 0.f, act_j = nj[K + 1] != 0.f;
-#pragma unroll
-      for (int k = 1; k < K; ++k) {
-        rho[k] = es[k] * inv;
-        nu_t += rho[k] * iden[k];
-        const long long fq = __double2ll_rn(((double)rho[k] - (double)__fmul_rn(ef[k], invf)) * VM_FIX_SCALE);
-        if (fq != 0) {
-          if (act_j) vm_smem_add_split(colfix[cj][k - 1], fq);
-          if (act_i) vm_smem_add_split(rowfix[r][k - 1], fq);
-        }
-      }
-      float* ru = c.rho_u32 + u * K;
-      if (K == 2) {
-        *reinterpret_cast<float2*>(ru) = make_float2(rho[0], rho[1]);
-      } else {
-#pragma unroll
-        for (int k = 0; k < K; ++k) ru[k] = rho[k];
-      }
-      if (single) {
-        nu += X * z2 * nu_t;
-      } else {
-#pragma unroll
-        for (int k = 0; k < K; ++k) p0[k] += rho[k] * X;
-      }
-    }
-  }
-  __syncthreads();
-  // ---- flush: one global atomic per touched node and category
-  unsigned long long* fix_l = reinterpret_cast<unsigned long long*>(c.fixA) + (int64_t)l * c.M * K;
-  for (int t = tid; t < TW * (K - 1); t += VM_SC_THREADS) {
-    const unsigned long long v = vm_smem_split_value(&colfix[0][0][0] + 2 * t);
-    if (v != 0ull) atomicAdd(fix_l + (int64_t)(jt + t / (K - 1)) * K + 1 + t % (K - 1), v);
-  }
-  for (int t = tid; t < nrows * (K - 1); t += VM_SC_THREADS) {
-    const unsigned long long v = vm_smem_split_value(&rowfix[0][0][0] + 2 * t);
-    if (v != 0ull) atomicAdd(fix_l + (int64_t)((int)c.row0 + i_lo + t / (K - 1)) * K + 1 + t % (K - 1), v);
-  }
-  // rho_k X of the SIMPLE ties (their part of the next phi-shape sums) and the nu statistic of the SINGLE ties
-  const double vn = block_sum<VM_SC_THREADS>((double)nu, sm_red);
-  if (tid == 0 && vn != 0.0)
-    atomicAdd(reinterpret_cast<unsigned long long*>(c.dev_flags) + VM_FLAG_FIXNU,
-              (unsigned long long)__double2ll_rn(vn * VM_FIXP_SCALE));
-#pragma unroll
-  for (int k = 0; k < K; ++k) {
-    const double v = block_sum<VM_SC_THREADS>((double)p0[k], sm_red);
-    if (tid == 0 && v != 0.0)
-      atomicAdd(reinterpret_cast<unsigned long long*>(c.fixP) + l * K + k,
-                (unsigned long long)__double2ll_rn(v * VM_FIXP_SCALE));
+    for (int k = 0; k < K; ++k) dst[k] = c.rho_u32[u * K + k];
   }
 }
 
@@ -1917,7 +1698,7 @@ __global__ void __launch_bounds__(VM_SC_THREADS) k_shortcut(const __grid_constan
 // statistic from a shared-memory reporter table -- coalesced 12-byte entry reads, every lane busy -- and stage it in
 // shared memory; then one thread per tie sums its entries' staged values (fixed order), adds the prior and the S term,
 // normalises and accumulates the statistics.  Groups with more entries than the stage holds go through it in slices.
-// log2 rho_k/rho_0 = lo_k - S_all d_k + sum_e dat_k(e): every term O(1..30), fp32 does not cancel (see k_shortcut).
+// log2 rho_k/rho_0 = lo_k - S_all d_k + sum_e dat_k(e): every term O(1..30), fp32 does not cancel (see vm_shortcut_tie).
 #define VM_A32_CAP 128  // staged entries per slice and WARP (a warp's 32 consecutive ties have ~58 entries at config 4)
 // floats per staged entry: w_k = dz1_k (K), t_0 = dz1_0 E[log theta] and t_k = (dz1_k - dz1_0) E[log theta] (K),
 // dz2_k (K); padded to 16 bytes
@@ -2597,45 +2378,42 @@ static bool simple_iteration(const vm_ctx* c, int flags) {
   return c->simple_mode != 0 && c->r_mode == VM_R_EGO && !(flags & VM_F_ELBO) && dense_fast_eligible<K>(c, flags);
 }
 
-// dynamic shared memory of the fast dense kernel (opt-in above 48 KB; set once per process and instantiation)
-template <int K, bool ELBO>
-static cudaError_t fast_setup() {
-  static bool done = false;
-  if (done) return cudaSuccess;
-  const cudaError_t e = cudaFuncSetAttribute(k_dense_fast<K, ELBO>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                             (int)sizeof(FastSmem<K>));
-  done = (e == cudaSuccess);
-  return e;
-}
+// dynamic shared memory of the TMA dense kernels (opt-in above 48 KB)
 template <int K>
 static cudaError_t fast_setup_all() {
-  if constexpr (K <= 4) {  // the fast kernel is only instantiated (and eligible) for K <= 4
+  if constexpr (K <= 4) {  // the TMA kernels are only instantiated (and eligible) for K <= 4
     cudaError_t e;
-    if ((e = fast_setup<K, true>()) != cudaSuccess) return e;
     if ((e = cudaFuncSetAttribute(k_dense_tma<K, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                   (int)sizeof(TmaSmem<K>))) != cudaSuccess) return e;
     if ((e = cudaFuncSetAttribute(k_dense_tma<K, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                   (int)sizeof(TmaSmem<K>))) != cudaSuccess) return e;
-    return fast_setup<K, false>();
+    return cudaFuncSetAttribute(k_dense_sc<K>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(TmaSmem<K, true>));
   } else {
     return cudaSuccess;
   }
 }
 
-static bool vm_x_notma() {  // VM_X_NOTMA=1: the STG.128 fast dense kernel instead of the TMA one (A/B measurements)
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("VM_X_NOTMA");
-    v = (e && atoi(e)) ? 1 : 0;
+// the special-tie kernel in list mode, on the iterations whose shortcut ties k_dense_sc evaluates: LIST = 1 walks the list
+// of the other special ties of the layers that take the shortcut (its grid covers that list only; k_sums_stage1 reads as
+// many partial slots), LIST = 2 has every special tie of the layers that cannot
+template <int K>
+static void launch_listed(const vm_ctx* c, cudaStream_t s) {
+  if constexpr (K <= 4) {  // (simple_iteration is never true for larger K)
+    if (c->n_ublk <= 0) return;
+    const dim3 gridl((unsigned)(c->n_cxblk > 0 ? c->n_cxblk : 1), (unsigned)c->L);
+    k_special<K, false, VM_R_EGO, 1><<<gridl, 256, 0, s>>>(*c, region_u(c));
+    const dim3 grid2((unsigned)imin64(c->n_ublk, 148 * 2), (unsigned)c->L);
+    k_special<K, false, VM_R_EGO, 2><<<grid2, 256, 0, s>>>(*c, region_u(c));
   }
-  return v != 0;
 }
 
 // `sums_flags` >= 0: the scalar-sum kernels that only depend on the special-tie kernels (k_elbo_b, k_sums_stage1) also go
 // to the aux stream, under the dense kernel; *sums_done tells the caller whether they were launched here.
+// `sc` (simple_iteration): the dense kernel is k_dense_sc, and the list-mode special-tie kernels are launched here, on the
+// aux stream ahead of the sums and the partial tiles, so that they run under it; k_patch_rest follows the join.
 template <int K>
 static int launch_dense(const vm_ctx* c, int flags, cudaStream_t st, int rt0, int rtn, int sums_flags = -1,
-                        bool* sums_done = nullptr) {
+                        bool* sums_done = nullptr, bool sc = false) {
   if (sums_done) *sums_done = false;
   if (rtn <= 0) return 0;
   const dim3 grid((unsigned)c->nct, (unsigned)(c->L * rtn));
@@ -2669,20 +2447,21 @@ static int launch_dense(const vm_ctx* c, int flags, cudaStream_t st, int rt0, in
   if (side) {
     cudaEventRecord(ev_fork, st);
     cudaStreamWaitEvent(aux, ev_fork, 0);
+    if (sc) launch_listed<K>(c, aux);
     if (sums_flags >= 0) {
       if ((flags & VM_F_ELBO) && c->mutuality) k_elbo_b<K><<<VM_B_BLOCKS, 256, 0, aux>>>(*c, region_b(c));
       k_sums_stage1<<<dim3(VM_S1_BLOCKS, (unsigned)c->L), 256, 0, aux>>>(*c, sums_flags, region_u(c), region_s1(c));
       if (sums_done) *sums_done = true;
     }
+  } else if (sc) {
+    launch_listed<K>(c, st);
   }
 #define LF()                                                                                                             \
   do {                                                                                                                   \
     if constexpr (K <= 4) {                                                                                              \
-      if (!vm_x_notma()) {                                                                                               \
-        if (elbo) k_dense_tma<K, true><<<grid, VM_DENSE_THREADS, sizeof(TmaSmem<K>), st>>>(*c, cp, rt0, rtn);             \
-        else k_dense_tma<K, false><<<grid, VM_DENSE_THREADS, sizeof(TmaSmem<K>), st>>>(*c, cp, rt0, rtn);                 \
-      } else if (elbo) k_dense_fast<K, true><<<grid, VM_DENSE_THREADS, sizeof(FastSmem<K>), st>>>(*c, cp, rt0, rtn);       \
-      else k_dense_fast<K, false><<<grid, VM_DENSE_THREADS, sizeof(FastSmem<K>), st>>>(*c, cp, rt0, rtn);                  \
+      if (sc) k_dense_sc<K><<<grid, VM_DENSE_THREADS, sizeof(TmaSmem<K, true>), st>>>(*c, rt0, rtn);                      \
+      else if (elbo) k_dense_tma<K, true><<<grid, VM_DENSE_THREADS, sizeof(TmaSmem<K>), st>>>(*c, cp, rt0, rtn);          \
+      else k_dense_tma<K, false><<<grid, VM_DENSE_THREADS, sizeof(TmaSmem<K>), st>>>(*c, cp, rt0, rtn);                   \
     }                                                                                                                    \
   } while (0)
   if (fast && !side) LF();
@@ -2707,6 +2486,12 @@ static int launch_dense(const vm_ctx* c, int flags, cudaStream_t st, int rt0, in
     }
   }
 #undef LF
+  if constexpr (K <= 4) {
+    if (sc && c->n_ublk > 0) {
+      const dim3 gridp((unsigned)imin64(c->n_ublk * (VM_SPECIAL_TIES_PER_BLOCK / 256), 148 * 8), (unsigned)c->L);
+      k_patch_rest<K><<<gridp, 256, 0, st>>>(*c);
+    }
+  }
   return rc;
 }
 
@@ -2717,32 +2502,7 @@ static int launch_special(const vm_ctx* c, int flags, cudaStream_t st) {
   const dim3 grid((unsigned)gridx, (unsigned)c->L);
   const bool elbo = flags & VM_F_ELBO;
 #define LS(E, M) k_special<K, E, M><<<grid, 256, 0, st>>>(*c, region_u(c))
-  if (simple_iteration<K>(c, flags)) {
-    if constexpr (K <= 4) {  // (simple_iteration is never true for larger K)
-      // layers that take the shortcut: the special-tie kernel walks the list of the other special ties (its grid covers
-      // that list only; k_sums_stage1 reads as many partial slots) while k_shortcut evaluates the shortcut ties
-      // The list-mode launches and k_shortcut touch disjoint ties (and integer atomics): with an aux stream the former
-      // run next to the latter (-4 us per iteration at config 3)
-      cudaStream_t aux = (cudaStream_t)c->aux_stream;
-      cudaEvent_t ev_fork = (cudaEvent_t)c->ev_fork, ev_join = (cudaEvent_t)c->ev_join;
-      const bool split = aux != nullptr && aux != st && ev_fork != nullptr && ev_join != nullptr;
-      cudaStream_t sl = split ? aux : st;
-      if (split) {
-        cudaEventRecord(ev_fork, st);
-        cudaStreamWaitEvent(aux, ev_fork, 0);
-      }
-      const dim3 gridl((unsigned)(c->n_cxblk > 0 ? c->n_cxblk : 1), (unsigned)c->L);
-      k_special<K, false, VM_R_EGO, 1><<<gridl, 256, 0, sl>>>(*c, region_u(c));
-      const dim3 grid2((unsigned)imin64(gridx, 148 * 2), (unsigned)c->L);
-      k_special<K, false, VM_R_EGO, 2><<<grid2, 256, 0, sl>>>(*c, region_u(c));  // layers that cannot
-      if (c->N / DenseCfg<K>::TW > 0)
-        k_shortcut<K><<<dim3((unsigned)(c->N / DenseCfg<K>::TW), (unsigned)(c->L * c->nrt)), VM_SC_THREADS, 0, st>>>(*c);
-      if (split) {
-        cudaEventRecord(ev_join, aux);
-        cudaStreamWaitEvent(st, ev_join, 0);
-      }
-    }
-  } else if (c->r_mode == VM_R_EGO) {
+  if (c->r_mode == VM_R_EGO) {
     if (elbo) LS(true, VM_R_EGO); else LS(false, VM_R_EGO);
   } else if (c->r_mode == VM_R_ALL && c->all32_mode != 0 && !elbo) {
     // layers whose guard holds: every special tie in fp32, entry-parallel; the others: the fp64 kernel (strided grid)
@@ -2759,14 +2519,16 @@ static int launch_special(const vm_ctx* c, int flags, cudaStream_t st) {
   return 0;
 }
 
-// special-tie kernels, then the dense kernel, of one rho update.  (Running them side by side on two streams was measured
-// twice -- row chunks in round 1, a persistent shortcut kernel next to an unpatched dense kernel in round 2,
-// profiles/r2_dense_experiments.txt -- and lost both times: each wants the registers and warp slots the other holds.)
+// special-tie kernels, then the dense kernel, of one rho update.  On iterations whose shortcut ties the dense kernel
+// evaluates (simple_iteration), the list-mode special-tie kernels run next to it instead, on the aux stream (launch_dense).
+// (Running an unpatched dense kernel next to a separate shortcut kernel was measured in round 2 and lost: each wants the
+// registers and warp slots the other holds, profiles/r2_dense_experiments.txt.)
 template <int K>
 static int launch_rho_kernels(const vm_ctx* c, int flags, cudaStream_t st, bool* sums_done) {
+  const bool sc = simple_iteration<K>(c, flags);
   int rc;
-  if ((rc = launch_special<K>(c, flags, st))) return rc;
-  return launch_dense<K>(c, flags, st, 0, (int)c->nrt, flags | (simple_iteration<K>(c, flags) ? VM_F_LISTED : 0), sums_done);
+  if (!sc && (rc = launch_special<K>(c, flags, st))) return rc;
+  return launch_dense<K>(c, flags, st, 0, (int)c->nrt, flags | (sc ? VM_F_LISTED : 0), sums_done, sc);
 }
 
 template <int K>
