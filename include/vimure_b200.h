@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define VM_ABI_VERSION 15
+#define VM_ABI_VERSION 16
 
 /* reporter-mask structure (how R[l,i,j,m] is represented) */
 #define VM_R_EGO 0 /* reporter m == node m reports row m and column m (vimure synthetic.py:1184-1204, _io.py:229-242) */
@@ -40,6 +40,11 @@ extern "C" {
 #define VM_F_ELBO 1      /* also produce the ELBO (model.py:948-1019) */
 #define VM_F_NO_STORE 2  /* do not write the dense rho slab this iteration (statistics only) */
 #define VM_F_INIT 4      /* vm_phase_finish only: consume the initial statistics, do not update nu */
+#define VM_F_NO_SLAB 8   /* this rank has no slab (vm_ctx.rho == NULL): the fast dense kernels run statistics-only (no
+                            stage, no store, no patches); the tables (tab_p, tab_q, layer_consts) and rho_u32 the iteration
+                            leaves behind ARE the posterior (vm_materialize_rows evaluates it).  Not with VM_R_CSR, whose
+                            statistics gather the slab (VM_ENOTSUP).  Unlike VM_F_NO_STORE, every kernel and every number
+                            is that of a storing iteration. */
 
 /* error codes (negative) */
 #define VM_EINVAL (-1)    /* bad argument / unsupported K */
@@ -233,7 +238,8 @@ typedef struct vm_ctx {
   float* rho_u32;           /* [U*K] fp32 posterior of the special ties: patch source of the dense slab and what the gamma /
                                phi passes gather (written by the special-tie kernel and by the shortcut-tie kernel) */
   double* delta_u;          /* [U*K] rho_u - formula value */
-  float* rho;               /* [L*nloc*N*K] dense posterior slab */
+  float* rho;               /* [L*nloc*N*K] dense posterior slab, or NULL: then every iteration must pass VM_F_NO_SLAB,
+                               and the entry points that read or write the slab return VM_EINVAL */
 
   /* ---- workspaces ---- */
   double* layer_consts;     /* [L*(3*K+5)] per layer: c_k, d_k (log2 domain), S_all, log-prior consts, dead flag,
@@ -304,6 +310,12 @@ int vm_run(const vm_ctx* c, int n_iter, int flags, int last_flags, void* stream)
 
 /* Writes rho = pr_rho into the dense slab (one-hot + special ties), model.py:602. */
 int vm_materialize_prior(const vm_ctx* c, void* stream);
+
+/* The posterior the last rho update left (the implicit one of a VM_F_NO_SLAB fit, or the slab's own values), for the
+ * local rows [lrow0, lrow0+nrows), lrow = l*nloc + (i-row0), into `out` (float32 [nrows][N][K], the slab's layout):
+ * bit-identical to what a storing iteration writes into those rows of the slab.  Reads tab_p, tab_q, layer_consts,
+ * utile_ptr, u_col and rho_u32 only; VM_ENOTSUP under the general mask (VM_R_CSR). */
+int vm_materialize_rows(const vm_ctx* c, int64_t lrow0, int64_t nrows, float* out, void* stream);
 
 /* Posterior consumers on the dense slab (model.py:1148-1166, utils.py:207-217):
  * out[t] = argmax_k rho[t,k] (mode 0) or rho[t,1] >= threshold (mode 1), uint8, [L*nloc*N]. */

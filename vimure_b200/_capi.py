@@ -138,6 +138,7 @@ def open_library(path):
         "vm_iteration": (i, [P, i, vp]),
         "vm_run": (i, [P, i, i, i, vp]),
         "vm_materialize_prior": (i, [P, vp]),
+        "vm_materialize_rows": (i, [P, i64, i64, vp, vp]),
         "vm_infer": (i, [P, i, d, vp, vp]),
         "vm_sample": (i, [P, i64, ctypes.c_uint64, vp, vp]),
         "vm_infer_mean": (i, [P, vp, vp]),

@@ -1,7 +1,9 @@
 """Host-side driver of the CUDA CAVI kernels: owns the device buffers (PyTorch tensors = plumbing),
 fills the `vm_ctx` of include/vimure_b200.h and calls the extern "C" launchers.
 
-One engine = one rank's shard (node-row block) of one fit.  With `group` set, the three statistics vectors
+One engine = one rank's shard (node-row block) of one fit.  With `slab=False` it holds no dense posterior slab: every
+iteration runs with VM_F_NO_SLAB, the posterior stays implicit in the row/column tables and the special ties' rho_u32,
+and the consumers evaluate it block by block (`vm_materialize_rows`) -- bit-identical to a fit that stores the slab.  With `group` set, the three statistics vectors
 (red1: gamma-shape sums, red2: phi-shape sums, red3: A + nu + ELBO sums) are all-reduced with
 torch.distributed (NCCL over NVLink on the GPU box) between the phases -- the only exchange the path needs
 (SURVEY.md section 8e).  There is no CPU fallback: without CUDA the constructor raises.
@@ -20,8 +22,16 @@ def _packing_const():
     return SPECIAL_TIES_PER_BLOCK
 
 
+# rows of posterior the consumers of a slab-free engine materialise at a time: at most this many bytes
+IMPLICIT_BLOCK_BYTES = 256 << 20
+
+# the buffers that hold the implicit posterior of a slab-free engine (what `vm_materialize_rows` reads besides the packed
+# data)
+IMPLICIT_STATE = ("tab_p", "tab_q", "layer_consts", "rho_u32")
+
+
 class CaviEngine:
-    def __init__(self, packed, priors, mutuality=True, eps=1e-12, group=None, may_dead=False):
+    def __init__(self, packed, priors, mutuality=True, eps=1e-12, group=None, may_dead=False, slab=True):
         P = self.P = packed
         if not torch.cuda.is_available():
             raise RuntimeError("vimure_b200 needs a CUDA device: the CAVI kernels have no CPU fallback")
@@ -35,6 +45,10 @@ class CaviEngine:
         if dev.type != "cuda":
             raise RuntimeError("packed data must live on a CUDA device")
         self.mutuality = bool(mutuality)
+        self.slab = bool(slab)
+        if not self.slab and P.r_mode == 2:
+            raise ValueError("a fit without the dense slab needs an ego or all-reporter mask (the general mask's "
+                             "statistics gather the slab)")
         if self.mutuality and not getattr(P, "mutuality", True):
             raise ValueError("the data were packed for mutuality=False (no entry visits the gamma/phi passes)")
         f64 = dict(dtype=torch.float64, device=dev)
@@ -61,8 +75,9 @@ class CaviEngine:
         self.rho_u = z(max(U, 1), K)
         self.rho_u32 = torch.zeros(max(U, 1), K, **f32)
         self.delta_u = z(max(U, 1), K)
-        self.rho = torch.empty(L, nloc, N, K, **f32)
+        self.rho = torch.empty(L, nloc, N, K, **f32) if self.slab else None
         self.rho_valid = False
+        self.block_rows = max(1, IMPLICIT_BLOCK_BYTES // (N * K * 4))  # consumers of a slab-free engine
         # workspaces
         self.layer_consts = z(L * (3 * K + 5))
         self.tab_p = torch.zeros(L * nloc * K, **f32)
@@ -137,10 +152,12 @@ class CaviEngine:
             setattr(c, name, ptr(P.t[name]) if name in P.t else self._dummy.data_ptr())
         for name in ("u_logpr", "alpha_theta", "beta_theta", "alpha_lambda", "beta_lambda", "gamma_shp", "gamma_rte",
                      "phi_shp", "phi_rte", "nu", "G_theta", "E_theta", "Elog_theta", "G_lambda", "E_lambda",
-                     "Elog_lambda", "GE_theta", "rho_u", "rho_u32", "delta_u", "rho", "layer_consts", "tab_p", "tab_q",
+                     "Elog_lambda", "GE_theta", "rho_u", "rho_u32", "delta_u", "layer_consts", "tab_p", "tab_q",
                      "rowpart", "colpart", "er_node", "colsum", "dev_flags", "fixA", "fixG", "phi0", "blkpart", "red1", "red2", "red3",
                      "elbo_out", "u_rec", "nodetab", "fixP", "simple_consts", "cx_logpr", "gfpart", "u_lo"):
             setattr(c, name, ptr(getattr(self, name)))
+        c.rho = ptr(self.rho) if self.slab else None
+        self._nsl = 0 if self.slab else self.C["VM_F_NO_SLAB"]  # flag of every rho update
         c.A = self.red3.data_ptr()  # A aliases the (all-reduced) statistics vector
         c.ev_fork, c.ev_join = self._ev_fork.cuda_event, self._ev_join.cuda_event
         self._cref = ctypes.byref(c)
@@ -162,13 +179,15 @@ class CaviEngine:
         [dense_fast], dense, [col_reduce], stats, [elbo_b], sums_reduce | finish: [elbo_partial], finish."""
         P = self.P
         csr, ego = P.r_mode == 2, P.r_mode == 0
-        fast = (P.K <= 4 and store and not csr and (P.N * P.K) % 4 == 0 and P.N >= P.tile_w
+        fast = (P.K <= 4 and (store or not self.slab) and not csr and (P.N * P.K) % 4 == 0 and P.N >= P.tile_w
                 and P.tile_h <= 128)
         n = 2 + 3 + 1 + (0 if csr else 1) + 1 + (1 if fast else 0) + 1 + (1 if ego else 0) + 1 + 2 + 1
         if elbo:
             n += 1 + (1 if self.mutuality else 0)
         elif self.simple_mode and fast:
-            n += 2  # the special-tie kernel is launched twice (layers that take the shortcut / that cannot) + k_patch_rest
+            # the special-tie kernel is launched twice (layers that take the shortcut / that cannot) + k_patch_rest, which
+            # only a slab needs
+            n += 2 if self.slab else 1
         elif self.all32_mode:
             n += 1  # k_all32 + the fp64 special-tie kernel for the layers whose guard fails
         return n
@@ -236,8 +255,8 @@ class CaviEngine:
         if n <= 0:
             return
         F = self.C
-        base = 0 if store else F["VM_F_NO_STORE"]
-        last = (0 if (store or store_last) else F["VM_F_NO_STORE"]) | (F["VM_F_ELBO"] if elbo_last else 0)
+        base = (0 if store else F["VM_F_NO_STORE"]) | self._nsl
+        last = (0 if (store or store_last) else F["VM_F_NO_STORE"]) | (F["VM_F_ELBO"] if elbo_last else 0) | self._nsl
         st = self._stream()
         if self._graphs is not None:
             for it in range(n):
@@ -249,7 +268,7 @@ class CaviEngine:
                 self._sharded_iteration(last if it == n - 1 else base)
         self.n_launch += (n - 1) * self.kernels_per_iteration(False, store) + \
             self.kernels_per_iteration(elbo_last, store or store_last)
-        self.rho_valid = bool(store or store_last)
+        self.rho_valid = bool(store or store_last) and self.slab
         self.rho_is_prior = False
 
     def _sharded_iteration(self, flags):
@@ -282,7 +301,7 @@ class CaviEngine:
         synchronises the device: do it before several engines start to run side by side on their own streams)."""
         if self._graphs is not None:
             F = self.C
-            for flags in (0 if store else F["VM_F_NO_STORE"], F["VM_F_ELBO"]):
+            for flags in ((0 if store else F["VM_F_NO_STORE"]) | self._nsl, F["VM_F_ELBO"] | self._nsl):
                 self._graph(flags)
 
     def _graph(self, flags):
@@ -322,16 +341,16 @@ class CaviEngine:
         st = self._stream()
         fn = getattr(self.lib, "vm_phase_" + name)
         if name in ("rho", "finish"):
-            _capi.check(fn(self._cref, int(flags), st), "vm_phase_" + name)
+            _capi.check(fn(self._cref, int(flags) | self._nsl, st), "vm_phase_" + name)
         else:
             _capi.check(fn(self._cref, st), "vm_phase_" + name)
         if name == "rho":
-            self.rho_valid = not (flags & self.C["VM_F_NO_STORE"])
+            self.rho_valid = self.slab and not (flags & self.C["VM_F_NO_STORE"])
             self.rho_is_prior = False
 
     def dense_only(self, flags=0):
         """Launch only the per-tie dense kernel (measurement hook, see vm_dense_only)."""
-        _capi.check(self.lib.vm_dense_only(self._cref, int(flags), self._stream()), "vm_dense_only")
+        _capi.check(self.lib.vm_dense_only(self._cref, int(flags) | self._nsl, self._stream()), "vm_dense_only")
         self.n_launch += 1
 
     def elbo(self):
@@ -353,8 +372,15 @@ class CaviEngine:
             G_exp_nu=np.float64(nu[C["VM_NU_G_STALE"]]),
         )
 
-    def rho_slab(self):
-        """The dense posterior slab of this rank, float32 (L, nloc, N, K), on the device."""
+    def rho_slab(self, state=None):
+        """The dense posterior slab of this rank, float32 (L, nloc, N, K), on the device.  Without a slab it is evaluated
+        into a new tensor (from `state`, a `snapshot()`, if given)."""
+        if not self.slab:
+            old = self._use_slab(state)
+            try:
+                return self.materialize_rows(0, self.P.L * self.P.nloc).view(self.P.L, self.P.nloc, self.P.N, self.P.K)
+            finally:
+                self._restore(old)
         if not self.rho_valid:
             if getattr(self, "rho_is_prior", False):
                 _capi.check(self.lib.vm_materialize_prior(self._cref, self._stream()), "vm_materialize_prior")
@@ -364,31 +390,83 @@ class CaviEngine:
                 raise RuntimeError("the dense rho slab was not stored in the last iteration (store=False)")
         return self.rho
 
+    def materialize_rows(self, lrow0, nrows, out=None):
+        """The posterior of local rows [lrow0, lrow0+nrows) (lrow = l*nloc + i) as the slab holds it after the last rho
+        update: float32 (nrows, N, K) on the device (`vm_materialize_rows`)."""
+        P = self.P
+        if out is None:
+            out = torch.empty(nrows, P.N, P.K, dtype=torch.float32, device=self.dev)
+        _capi.check(self.lib.vm_materialize_rows(self._cref, int(lrow0), int(nrows), ctypes.c_void_p(out.data_ptr()),
+                                                 self._stream()), "vm_materialize_rows")
+        self.n_launch += 1
+        return out
+
+    def snapshot(self):
+        """Copy of the implicit posterior of a slab-free engine (row/column tables, layer constants, rho_u32: O(N + U)
+        floats) -- what a storing engine would clone its slab for.  `infer(..., slab=snapshot)` etc. read it."""
+        assert not self.slab
+        self._check_posterior()
+        return {name: getattr(self, name).clone() for name in IMPLICIT_STATE}
+
+    def _check_posterior(self):
+        if getattr(self, "rho_is_prior", True):
+            raise RuntimeError("no posterior yet: a fit without the dense slab has none before its first iteration")
+
     def _use_slab(self, slab):
-        """Point the consumers at `slab` (a copy of an earlier restart's posterior) instead of the engine's own; returns the
-        pointer to restore."""
-        old = self.ctx.rho
+        """Point the consumers at `slab` (a copy of an earlier restart's posterior: a slab tensor, or a `snapshot()` of a
+        slab-free engine) instead of the engine's own; returns what `_restore` puts back."""
+        if not self.slab:
+            if slab is None:
+                self._check_posterior()
+                return {}
+            old = {name: getattr(self.ctx, name) for name in IMPLICIT_STATE}
+            for name in IMPLICIT_STATE:
+                setattr(self.ctx, name, slab[name].data_ptr())
+            return old
+        old = {"rho": self.ctx.rho}
         if slab is None:
             self.rho_slab()
         else:
             self.ctx.rho = slab.data_ptr()
         return old
 
+    def _restore(self, old):
+        for name, v in old.items():
+            setattr(self.ctx, name, v)
+
+    def _consume(self, fn, out, what, *args):
+        """Run the slab consumer `fn(ctx, *args, out)`: on the slab, or, without one, row block by row block on a
+        materialised block, through a view of the ctx that covers the block only (L = 1, nloc = its rows; the row offset
+        l*N + row0 + i0 keeps the global tie ids (l*N+i)*N+j that key vm_sample's stream)."""
+        if self.slab:
+            _capi.check(fn(self._cref, *args, ctypes.c_void_p(out.data_ptr()), self._stream()), what)
+            self.n_launch += 1
+            return out
+        P = self.P
+        rb = min(P.nloc, self.block_rows)
+        buf = torch.empty(rb, P.N, P.K, dtype=torch.float32, device=self.dev)
+        view = _capi.ctx_class()()
+        ctypes.memmove(ctypes.byref(view), self._cref, ctypes.sizeof(view))
+        for l in range(P.L):
+            for i0 in range(0, P.nloc, rb):
+                n = min(rb, P.nloc - i0)
+                self.materialize_rows(l * P.nloc + i0, n, buf)
+                view.L, view.nloc, view.nrt = 1, n, -(-n // P.tile_h)
+                view.row0 = l * P.N + P.row0 + i0
+                view.rho = buf.data_ptr()
+                _capi.check(fn(ctypes.byref(view), *args, ctypes.c_void_p(out[l, i0].data_ptr()), self._stream()), what)
+                self.n_launch += 1
+        return out
+
     def infer(self, mode=0, threshold=0.5, slab=None):
         """argmax_k rho (mode 0) or rho[...,1] >= threshold (mode 1) on the device: uint8 (L, nloc, N)."""
         old = self._use_slab(slab)
         try:
-            return self._infer(mode, threshold)
+            P = self.P
+            out = torch.empty(P.L, P.nloc, P.N, dtype=torch.uint8, device=self.dev)
+            return self._consume(self.lib.vm_infer, out, "vm_infer", int(mode), float(threshold))
         finally:
-            self.ctx.rho = old
-
-    def _infer(self, mode, threshold):
-        P = self.P
-        out = torch.empty(P.L, P.nloc, P.N, dtype=torch.uint8, device=self.dev)
-        _capi.check(self.lib.vm_infer(self._cref, int(mode), float(threshold), ctypes.c_void_p(out.data_ptr()),
-                                      self._stream()), "vm_infer")
-        self.n_launch += 1
-        return out
+            self._restore(old)
 
     def infer_mean(self, slab=None):
         """sum_k k rho_k (reference `rho_mean`, model.py:1151-1153) on the device: float32 (L, nloc, N)."""
@@ -396,11 +474,9 @@ class CaviEngine:
         try:
             P = self.P
             out = torch.empty(P.L, P.nloc, P.N, dtype=torch.float32, device=self.dev)
-            _capi.check(self.lib.vm_infer_mean(self._cref, ctypes.c_void_p(out.data_ptr()), self._stream()), "vm_infer_mean")
-            self.n_launch += 1
-            return out
+            return self._consume(self.lib.vm_infer_mean, out, "vm_infer_mean")
         finally:
-            self.ctx.rho = old
+            self._restore(old)
 
     def sample(self, n_trials=1, seed=0, slab=None):
         """argmax of the counts of `n_trials` categorical draws per tie (reference `sample_inferred_model`,
@@ -409,9 +485,7 @@ class CaviEngine:
         try:
             P = self.P
             out = torch.empty(P.L, P.nloc, P.N, dtype=torch.uint8, device=self.dev)
-            _capi.check(self.lib.vm_sample(self._cref, int(n_trials), ctypes.c_uint64(int(seed) & (2**64 - 1)),
-                                           ctypes.c_void_p(out.data_ptr()), self._stream()), "vm_sample")
-            self.n_launch += 1
-            return out
+            return self._consume(self.lib.vm_sample, out, "vm_sample", int(n_trials),
+                                 ctypes.c_uint64(int(seed) & (2**64 - 1)))
         finally:
-            self.ctx.rho = old
+            self._restore(old)

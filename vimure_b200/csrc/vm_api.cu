@@ -34,6 +34,9 @@ extern "C" int vm_run(const vm_ctx* c, int n_iter, int flags, int last_flags, vo
 extern "C" int vm_infer(const vm_ctx* c, int mode, double threshold, uint8_t* out, void* stream) {
   VM_ROUTE(infer(c, mode, threshold, out, stream));
 }
+extern "C" int vm_materialize_rows(const vm_ctx* c, int64_t lrow0, int64_t nrows, float* out, void* stream) {
+  VM_ROUTE(materialize_rows(c, lrow0, nrows, out, stream));
+}
 
 // ---- rho_mean on the slab (model.py:1151-1153): sum_k k rho_k, 4 bytes per tie back instead of an fp64 copy of rho -----
 __global__ void __launch_bounds__(256) k_infer_mean(const float* __restrict__ rho, int64_t T, int K, float* __restrict__ out) {

@@ -28,6 +28,7 @@ struct vm_tu_api {
   int (*iteration)(const vm_ctx*, int, void*);
   int (*run)(const vm_ctx*, int, int, int, void*);
   int (*infer)(const vm_ctx*, int, double, uint8_t*, void*);
+  int (*materialize_rows)(const vm_ctx*, int64_t, int64_t, float*, void*);
 };
 
 // Column tile of the dense kernels: TW = 128*NCH columns; NCH is K-dependent so that the per-lane column accumulators

@@ -1210,6 +1210,10 @@ __global__ void __launch_bounds__(VM_DENSE_THREADS) k_dense(const __grid_constan
 // tie of the segment (the special-tie kernel's list ties, and all special ties of a layer whose VM_LC_SIMPLE guard fails)
 // keeps its closed form here; k_patch_rest copies their rho_u32 into the slab once the special-tie kernel, which runs
 // next to this one, has written it.  The dense partials only ever count the closed form, so nothing else waits for it.
+//
+// STORE = false (VM_F_NO_SLAB: the rank has no slab): statistics only -- no stage, no bulk store, no patch loads.  The
+// SC variant still evaluates the shortcut ties (rho_u32, fixA, fixP, nu); the closed form their correction subtracts is
+// recomputed with vm_formula_rho, which gives the very bits the chunk loop counted.
 __device__ __forceinline__ void vm_bulk_store(void* gdst, const void* ssrc, uint32_t bytes) {
   asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(gdst),
                "r"((uint32_t)__cvta_generic_to_shared(ssrc)), "r"(bytes)
@@ -1237,10 +1241,11 @@ __device__ __forceinline__ unsigned long long vm_smem_split_value(const unsigned
 }
 
 #define VM_TMA_NBUF 2
-template <int K, bool SC = false>
+template <int K, bool SC = false, bool STORE = true>
 struct TmaSmem {
   static constexpr int TW = DenseCfg<K>::TW, NW = VM_DENSE_THREADS / 32, TH = VM_FAST_MAX_TILE_H;
-  float rowbuf[NW][VM_TMA_NBUF][TW * K];  // row-segment stages (slab layout), 128-byte aligned (first member)
+  // row-segment stages (slab layout), 128-byte aligned (first member); a placeholder without a slab
+  float rowbuf[STORE ? NW : 1][STORE ? VM_TMA_NBUF : 1][STORE ? TW * K : 4];
   float qs[K - 1][TW];                    // column terms of the log2-odds
   union {
     float colbuf[K - 1][TW];                     // cross-warp column sums (after the row loop)
@@ -1357,12 +1362,12 @@ __device__ __forceinline__ void vm_load_rec(const float* p, float* v) {
 #ifndef VM_TMA_PD
 #define VM_TMA_PD 2  // rows of prefetch distance of the patch entries
 #endif
-template <int K, bool ELBO, bool SC, int PD>
+template <int K, bool ELBO, bool SC, int PD, bool STORE = true>
 __device__ __forceinline__ void dense_tma_body(const vm_ctx& c, double* catpart, int rt0, int rtn, unsigned char* smem) {
   constexpr int NCH = DenseCfg<K>::NCH, TW = DenseCfg<K>::TW, NW = VM_DENSE_THREADS / 32;
   constexpr int NT = NodeTab<K>::STRIDE, NV = SC ? K + 2 : K;  // floats per prefetched special tie
   static_assert(!(SC && ELBO), "the shortcut ties are evaluated on iterations without ELBO only");
-  TmaSmem<K, SC>& S = *reinterpret_cast<TmaSmem<K, SC>*>(smem);
+  TmaSmem<K, SC, STORE>& S = *reinterpret_cast<TmaSmem<K, SC, STORE>*>(smem);
   const int N = (int)c.N, nloc = (int)c.nloc, nct = (int)c.nct, nrt = (int)c.nrt;
   const int ct = blockIdx.x;
   const int l = blockIdx.y / rtn, rt = rt0 + (blockIdx.y - l * rtn);  // row tiles [rt0, rt0+rtn) of every layer
@@ -1394,8 +1399,10 @@ __device__ __forceinline__ void dense_tma_body(const vm_ctx& c, double* catpart,
     const int64_t lrow = (int64_t)l * nloc + i_lo + r;
 #pragma unroll
     for (int k = 1; k < K; ++k) S.ps[k - 1][r] = __ldg(&c.tab_p[lrow * K + k]);
-    S.tp0[r] = __ldg(&c.utile_ptr[lrow * nct + ct]);
-    S.tp1[r] = (SC && !sc) ? S.tp0[r] : __ldg(&c.utile_ptr[lrow * nct + ct + 1]);
+    if (SC || STORE) {
+      S.tp0[r] = __ldg(&c.utile_ptr[lrow * nct + ct]);
+      S.tp1[r] = (SC && !sc) ? S.tp0[r] : __ldg(&c.utile_ptr[lrow * nct + ct + 1]);
+    }
   }
   if (SC && tid < K) {
     const double g0 = c.G_lambda[l * K], gkk = c.G_lambda[l * K + tid];
@@ -1427,7 +1434,7 @@ __device__ __forceinline__ void dense_tma_body(const vm_ctx& c, double* catpart,
       if (SC) {
         if (n > 0) rn = __ldg(c.nodetab + ((int64_t)l * N + (int)c.row0 + i_lo + row) * NT + (lane & (NT - 1)));
         if (lane < n) vm_load_rec<K>(c.u_rec + (int64_t)(ua + lane) * ScRec<K>::RS, v);
-      } else if (lane < n) {
+      } else if (STORE && lane < n) {
         col = __ldg(&c.u_col[ua + lane]);
 #pragma unroll
         for (int k = 0; k < K; ++k) v[k] = __ldg(&patch_src[(int64_t)(ua + lane) * K + k]);
@@ -1435,7 +1442,8 @@ __device__ __forceinline__ void dense_tma_body(const vm_ctx& c, double* catpart,
     }
   };
 #pragma unroll
-  for (int d = 0; d < PD; ++d) fetch(warp + d * NW, pq_col[d], pq_v[d], pq_rn[d]);
+  for (int d = 0; d < PD; ++d)
+    if (SC || STORE) fetch(warp + d * NW, pq_col[d], pq_v[d], pq_rn[d]);
   float prev[K];
   int64_t prev_idx = -1;
 #pragma unroll
@@ -1446,7 +1454,7 @@ __device__ __forceinline__ void dense_tma_body(const vm_ctx& c, double* catpart,
     // ---- request the patch entry of the row PD rows ahead
     int pn_col;
     float pn_v[NV], pn_rn;
-    fetch(r + PD * NW, pn_col, pn_v, pn_rn);
+    if (SC || STORE) fetch(r + PD * NW, pn_col, pn_v, pn_rn);
     float p[K];
 #pragma unroll
     for (int k = 1; k < K; ++k) p[k] = S.ps[k - 1][r];
@@ -1454,9 +1462,11 @@ __device__ __forceinline__ void dense_tma_body(const vm_ctx& c, double* catpart,
 #pragma unroll
     for (int k = 1; k < K; ++k) rowacc[k] = 0.f;
     float* sb = S.rowbuf[warp][buf];
-    // the bulk store that last read this stage has finished reading it
-    if (lane == 0) vm_bulk_wait_read<VM_TMA_NBUF - 1>();
-    __syncwarp();
+    if (STORE) {
+      // the bulk store that last read this stage has finished reading it
+      if (lane == 0) vm_bulk_wait_read<VM_TMA_NBUF - 1>();
+      __syncwarp();
+    }
 #pragma unroll
     for (int ch = 0; ch < NCH; ++ch) {
       float qv[K][4];
@@ -1483,7 +1493,7 @@ __device__ __forceinline__ void dense_tma_body(const vm_ctx& c, double* catpart,
         }
         if (ELBO) cat += (double)vm_formula_cat<K>(&o[t * K], s, false, lp0, lpk, epsf);
       }
-      vm_stage_chunk<K>(sb + ch * 128 * K, lane, o);
+      if (STORE) vm_stage_chunk<K>(sb + ch * 128 * K, lane, o);
       if (ch < 5) {  // step `ch` of the previous row's reduction (same order as warp_sum: 16, 8, 4, 2, 1)
 #pragma unroll
         for (int k = 1; k < K; ++k) prev[k] += __shfl_down_sync(0xffffffffu, prev[k], 16 >> ch);
@@ -1531,8 +1541,17 @@ __device__ __forceinline__ void dense_tma_body(const vm_ctx& c, double* catpart,
             float* d = sb + cj * K;
             float cf[K], rho[K];
             long long fq[K];
+            if (STORE) {
 #pragma unroll
-            for (int k = 1; k < K; ++k) cf[k] = d[k];  // the closed form the dense partials count for this tie
+              for (int k = 1; k < K; ++k) cf[k] = d[k];  // the closed form the dense partials count for this tie
+            } else {
+              float a[K], epsr;
+              bool dead;
+              a[0] = 0.f;
+#pragma unroll
+              for (int k = 1; k < K; ++k) a[k] = __fadd_rn(p[k], S.qs[k - 1][cj]);
+              vm_formula_rho<K>(a, false, cf, epsr, dead);
+            }
             vm_shortcut_tie<K>(rec, ni, nj, S.lam, cf, rho, fq, nu, p0);
             const bool act_j = nj[K + 1] != 0.f;
 #pragma unroll
@@ -1540,8 +1559,10 @@ __device__ __forceinline__ void dense_tma_body(const vm_ctx& c, double* catpart,
               if (act_j && fq[k] != 0) vm_smem_add_split(S.colfix[cj][k - 1], fq[k]);
               frow[k] += fq[k];
             }
+            if (STORE) {
 #pragma unroll
-            for (int k = 0; k < K; ++k) d[k] = rho[k];
+              for (int k = 0; k < K; ++k) d[k] = rho[k];
+            }
             float* ru = c.rho_u32 + (int64_t)(ua + e) * K;
             if (K == 2) {
               *reinterpret_cast<float2*>(ru) = make_float2(rho[0], rho[1]);
@@ -1563,7 +1584,7 @@ __device__ __forceinline__ void dense_tma_body(const vm_ctx& c, double* catpart,
           }
         }
       }
-    } else {
+    } else if (STORE) {
       if (lane < n) {
         float* d = sb + (pq_col[0] - jt) * K;
 #pragma unroll
@@ -1576,10 +1597,12 @@ __device__ __forceinline__ void dense_tma_body(const vm_ctx& c, double* catpart,
         for (int k = 0; k < K; ++k) d[k] = __ldg(&patch_src[(int64_t)(ua + e) * K + k]);
       }
     }
-    vm_fence_async_smem();
-    __syncwarp();
-    if (lane == 0) vm_bulk_store(c.rho + (lrow * N + jt) * K, sb, (uint32_t)(TW * K * sizeof(float)));
-    buf = (buf + 1 == VM_TMA_NBUF) ? 0 : buf + 1;
+    if (STORE) {
+      vm_fence_async_smem();
+      __syncwarp();
+      if (lane == 0) vm_bulk_store(c.rho + (lrow * N + jt) * K, sb, (uint32_t)(TW * K * sizeof(float)));
+      buf = (buf + 1 == VM_TMA_NBUF) ? 0 : buf + 1;
+    }
 #pragma unroll
     for (int d = 0; d + 1 < PD; ++d) {
       pq_col[d] = pq_col[d + 1];
@@ -1653,21 +1676,21 @@ __device__ __forceinline__ void dense_tma_body(const vm_ctx& c, double* catpart,
                   (unsigned long long)__double2ll_rn(v * VM_FIXP_SCALE));
     }
   }
-  if (lane == 0) vm_bulk_wait_all();  // the stages must outlive the engine's reads
+  if (STORE && lane == 0) vm_bulk_wait_all();  // the stages must outlive the engine's reads
 }
 
-template <int K, bool ELBO, int PD = VM_TMA_PD>
+template <int K, bool ELBO, int PD = VM_TMA_PD, bool STORE = true>
 __global__ void __launch_bounds__(VM_DENSE_THREADS, (K == 2 || K == 4) ? 3 : 2) k_dense_tma(const __grid_constant__ vm_ctx c, double* catpart, int rt0, int rtn) {
   extern __shared__ __align__(128) unsigned char vm_tma_smem[];
-  dense_tma_body<K, ELBO, false, PD>(c, catpart, rt0, rtn, vm_tma_smem);
+  dense_tma_body<K, ELBO, false, PD, STORE>(c, catpart, rt0, rtn, vm_tma_smem);
 }
 // the TMA dense kernel that also evaluates the shortcut ties (iterations without ELBO, vm_ctx.simple_mode).  Prefetch
 // distance 1 row: at K = 2 the records of a second row do not fit in the 80 registers of 3 CTAs per SM.  At K = 4 its
 // column-correction table leaves room for 2 CTAs per SM only.
-template <int K, int PD = 1>
+template <int K, int PD = 1, bool STORE = true>
 __global__ void __launch_bounds__(VM_DENSE_THREADS, (K == 2) ? 3 : 2) k_dense_sc(const __grid_constant__ vm_ctx c, int rt0, int rtn) {
   extern __shared__ __align__(128) unsigned char vm_tma_smem[];
-  dense_tma_body<K, false, true, PD>(c, nullptr, rt0, rtn, vm_tma_smem);
+  dense_tma_body<K, false, true, PD, STORE>(c, nullptr, rt0, rtn, vm_tma_smem);
 }
 
 // Special ties k_dense_sc left at their closed form, copied from rho_u32 into the slab: the list ties of the layers
@@ -2328,6 +2351,39 @@ __global__ void k_infer(const float* rho, int64_t T, int K, int mode, float thr,
     }
   }
 }
+// The posterior the last rho update left, for the local rows [lrow0, lrow0+nrows) (lrow = l*nloc + i), into `out` in the
+// slab's layout -- bit for bit what a storing iteration writes: the closed form from the row/column tables with the
+// layer's dead-row switch (the dense kernels' arithmetic), then the special ties of each row segment overwritten from
+// rho_u32.  One CTA per (row, column tile), rows strided over gridDim.y; store-bound.
+template <int K>
+__global__ void __launch_bounds__(256) k_materialize_rows(const __grid_constant__ vm_ctx c, int64_t lrow0, int64_t nrows,
+                                                          float* out) {
+  const int ct = blockIdx.x, N = (int)c.N;
+  const int j0 = ct * (int)c.tile_w, j1 = min(j0 + (int)c.tile_w, N);
+  for (int64_t r = blockIdx.y; r < nrows; r += gridDim.y) {
+    const int64_t lrow = lrow0 + r;
+    const int l = (int)(lrow / c.nloc);
+    const bool may_dead = vm_may_dead<K>(c, l);
+    float* dst = out + r * N * K;
+    for (int j = j0 + (int)threadIdx.x; j < j1; j += blockDim.x) {
+      float a[K], o[K], epsr;
+      bool dead;
+      vm_tie_logodds<K>(c, l, lrow, j, a);
+      vm_formula_rho<K>(a, may_dead, o, epsr, dead);
+#pragma unroll
+      for (int k = 0; k < K; ++k) dst[(int64_t)j * K + k] = o[k];
+    }
+    __syncthreads();
+    const int64_t seg = lrow * c.nct + ct;
+    for (int64_t u = c.utile_ptr[seg] + threadIdx.x; u < c.utile_ptr[seg + 1]; u += blockDim.x) {
+      const int col = c.u_col[u];
+#pragma unroll
+      for (int k = 0; k < K; ++k) dst[(int64_t)col * K + k] = c.rho_u32[u * K + k];
+    }
+    __syncthreads();
+  }
+}
+
 // =====================================================================================================
 // host-side launchers
 // =====================================================================================================
@@ -2343,6 +2399,13 @@ static inline double* region_b(const vm_ctx* c) { return region_cat(c) + n_catpa
 #define VM_B_BLOCKS 128
 static inline double* region_ep(const vm_ctx* c) { return region_b(c) + VM_B_BLOCKS; }
 static inline double* region_s1(const vm_ctx* c) { return region_ep(c) + 2 * VM_EP_BLOCKS; }  // L*VM_S1_BLOCKS*(3+K)
+
+// an entry point that writes or reads the dense slab needs one: only VM_F_NO_SLAB iterations run without (vm_ctx.rho =
+// NULL), and not under the general mask, whose statistics gather the slab
+static int slab_check(const vm_ctx* c, int flags) {
+  if (!(flags & VM_F_NO_SLAB)) return c->rho != nullptr ? 0 : VM_EINVAL;
+  return c->r_mode == VM_R_CSR ? VM_ENOTSUP : 0;
+}
 
 static int check_ctx(const vm_ctx* c) {
   if (!c) return VM_EINVAL;
@@ -2417,7 +2480,8 @@ static int launch_dense(const vm_ctx* c, int flags, cudaStream_t st, int rt0, in
   if (sums_done) *sums_done = false;
   if (rtn <= 0) return 0;
   const dim3 grid((unsigned)c->nct, (unsigned)(c->L * rtn));
-  const bool elbo = flags & VM_F_ELBO, store = !(flags & VM_F_NO_STORE), csr = c->r_mode == VM_R_CSR;
+  const bool elbo = flags & VM_F_ELBO, store = !(flags & (VM_F_NO_STORE | VM_F_NO_SLAB)), csr = c->r_mode == VM_R_CSR;
+  const bool noslab = flags & VM_F_NO_SLAB;
   double* cp = region_cat(c);
   const bool fast = dense_fast_eligible<K>(c, flags);
   if (fast) {
@@ -2459,7 +2523,13 @@ static int launch_dense(const vm_ctx* c, int flags, cudaStream_t st, int rt0, in
 #define LF()                                                                                                             \
   do {                                                                                                                   \
     if constexpr (K <= 4) {                                                                                              \
-      if (sc) k_dense_sc<K><<<grid, VM_DENSE_THREADS, sizeof(TmaSmem<K, true>), st>>>(*c, rt0, rtn);                      \
+      static_assert(sizeof(TmaSmem<K, true, false>) <= 48 * 1024, "no opt-in for the statistics-only kernels");          \
+      if (noslab && sc) k_dense_sc<K, 1, false><<<grid, VM_DENSE_THREADS, sizeof(TmaSmem<K, true, false>), st>>>(*c, rt0, rtn); \
+      else if (noslab && elbo)                                                                                           \
+        k_dense_tma<K, true, VM_TMA_PD, false><<<grid, VM_DENSE_THREADS, sizeof(TmaSmem<K, false, false>), st>>>(*c, cp, rt0, rtn); \
+      else if (noslab)                                                                                                   \
+        k_dense_tma<K, false, VM_TMA_PD, false><<<grid, VM_DENSE_THREADS, sizeof(TmaSmem<K, false, false>), st>>>(*c, cp, rt0, rtn); \
+      else if (sc) k_dense_sc<K><<<grid, VM_DENSE_THREADS, sizeof(TmaSmem<K, true>), st>>>(*c, rt0, rtn);                 \
       else if (elbo) k_dense_tma<K, true><<<grid, VM_DENSE_THREADS, sizeof(TmaSmem<K>), st>>>(*c, cp, rt0, rtn);          \
       else k_dense_tma<K, false><<<grid, VM_DENSE_THREADS, sizeof(TmaSmem<K>), st>>>(*c, cp, rt0, rtn);                   \
     }                                                                                                                    \
@@ -2487,7 +2557,7 @@ static int launch_dense(const vm_ctx* c, int flags, cudaStream_t st, int rt0, in
   }
 #undef LF
   if constexpr (K <= 4) {
-    if (sc && c->n_ublk > 0) {
+    if (sc && !noslab && c->n_ublk > 0) {
       const dim3 gridp((unsigned)imin64(c->n_ublk * (VM_SPECIAL_TIES_PER_BLOCK / 256), 148 * 8), (unsigned)c->L);
       k_patch_rest<K><<<gridp, 256, 0, st>>>(*c);
     }
@@ -2549,6 +2619,7 @@ static int launch_stats(const vm_ctx* c, int init, cudaStream_t st) {
 static int tu_materialize_prior(const vm_ctx* c, void* stream) {
   int rc = check_ctx(c);
   if (rc) return rc;
+  if ((rc = slab_check(c, 0))) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   const int64_t T = c->L * c->nloc * c->N;
   k_fill_onehot<<<(unsigned)imin64(cdiv(T * c->K, 256), 148 * 16), 256, 0, st>>>(c->rho, T, (int)c->K);
@@ -2644,6 +2715,7 @@ static int tu_phase_phi(const vm_ctx* c, void* stream) {
 static int tu_phase_rho(const vm_ctx* c, int flags, void* stream) {
   int rc = check_ctx(c);
   if (rc) return rc;
+  if ((rc = slab_check(c, flags))) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   DISPATCH_K(c->K, (k_phi_finish<K><<<(unsigned)c->L, 256, 0, st>>>(*c)));
   VM_CHECK_LAUNCH();
@@ -2677,6 +2749,7 @@ static int tu_phase_rho(const vm_ctx* c, int flags, void* stream) {
 static int tu_dense_only(const vm_ctx* c, int flags, void* stream) {
   int rc = check_ctx(c);
   if (rc) return rc;
+  if ((rc = slab_check(c, flags))) return rc;
   DISPATCH_K(c->K, rc = launch_dense<K>(c, flags, (cudaStream_t)stream, 0, (int)c->nrt));
   if (rc) return rc;
   VM_CHECK_LAUNCH();
@@ -2703,6 +2776,7 @@ static int tu_phase_finish(const vm_ctx* c, int flags, void* stream) {
 
 static int tu_iteration(const vm_ctx* c, int flags, void* stream) {
   int rc;
+  if (c && (rc = slab_check(c, flags))) return rc;  // before any phase has changed the state
   if ((rc = tu_phase_gamma(c, stream))) return rc;
   if ((rc = tu_phase_phi(c, stream))) return rc;
   if ((rc = tu_phase_rho(c, flags, stream))) return rc;
@@ -2710,8 +2784,10 @@ static int tu_iteration(const vm_ctx* c, int flags, void* stream) {
 }
 
 static int tu_run(const vm_ctx* c, int n_iter, int flags, int last_flags, void* stream) {
+  int rc;
+  if (c && n_iter > 0 && ((rc = slab_check(c, last_flags)) || (n_iter > 1 && (rc = slab_check(c, flags))))) return rc;
   for (int it = 0; it < n_iter; ++it) {
-    int rc = tu_iteration(c, it == n_iter - 1 ? last_flags : flags, stream);
+    rc = tu_iteration(c, it == n_iter - 1 ? last_flags : flags, stream);
     if (rc) return rc;
   }
   return 0;
@@ -2721,6 +2797,7 @@ static int tu_infer(const vm_ctx* c, int mode, double threshold, uint8_t* out, v
   int rc = check_ctx(c);
   if (rc) return rc;
   if (mode == 1 && c->K < 2) return VM_EINVAL;
+  if ((rc = slab_check(c, 0))) return rc;
   const int64_t T = c->L * c->nloc * c->N;
   k_infer<<<(unsigned)imin64(cdiv(T, 256), 148 * 16), 256, 0, (cudaStream_t)stream>>>(c->rho, T, (int)c->K, mode,
                                                                                           (float)threshold, out);
@@ -2729,11 +2806,24 @@ static int tu_infer(const vm_ctx* c, int mode, double threshold, uint8_t* out, v
 }
 
 
+static int tu_materialize_rows(const vm_ctx* c, int64_t lrow0, int64_t nrows, float* out, void* stream) {
+  int rc = check_ctx(c);
+  if (rc) return rc;
+  if (!out || lrow0 < 0 || nrows < 0 || lrow0 + nrows > c->L * c->nloc) return VM_EINVAL;
+  if (c->r_mode == VM_R_CSR) return VM_ENOTSUP;  // no row/column tables: the general mask's posterior lives in the slab
+  if (nrows == 0) return 0;
+  const dim3 grid((unsigned)c->nct, (unsigned)imin64(nrows, 65535));
+  DISPATCH_K(c->K, (k_materialize_rows<K><<<grid, 256, 0, (cudaStream_t)stream>>>(*c, lrow0, nrows, out)));
+  VM_CHECK_LAUNCH();
+  return 0;
+}
+
 }  // namespace
 
 extern "C" const vm_tu_api* VM_PASTE(vm_tu_api_, VM_TU_ID)(void) {
   using namespace VM_PASTE(vmtu, VM_TU_ID);
   static const vm_tu_api api = {tu_materialize_prior, tu_refresh_cache, tu_init_stats, tu_phase_gamma, tu_phase_phi,
-                                tu_phase_rho,         tu_dense_only,    tu_phase_finish, tu_iteration, tu_run, tu_infer};
+                                tu_phase_rho,         tu_dense_only,    tu_phase_finish, tu_iteration, tu_run, tu_infer,
+                                tu_materialize_rows};
   return &api;
 }

@@ -26,7 +26,14 @@ Extra, optional `fit` keywords (a superset of the reference's):
     concurrent_realisations: "auto" | True | False -- run the `num_realisations` restarts (model.py:386-437) side by
                  side, one CUDA stream + one state per restart over the shared packed data, instead of one after the
                  other.  Same seeds, same trace, same best restart; "auto" = when an iteration is launch-bound
-                 (L*N*N*K <= 2e7) and the restarts' posterior slabs fit together.
+                 (L*N*N*K <= 2e7) and the restarts' posterior slabs fit together;
+    store_rho  : True (default) -- keep the dense posterior slab rho (float32, 4*L*N*N*K bytes) on the device;
+                 False -- write it at the ELBO iterations only (the other iterations run statistics-only kernels);
+                 "never" -- never allocate it: the posterior stays implicit in O(N) row/column tables and the special
+                 ties' posteriors, and `rho`, `rho_f`, `get_inferred_model`, `get_posterior_estimates` and
+                 `sample_inferred_model` evaluate it block by block on demand.  Parameters, trace and every output are
+                 bit-identical to the default; it lets a sparse network whose slab exceeds the GPU's memory be fitted.
+                 Needs an ego or all-reporter mask (ValueError otherwise: the general mask's statistics gather the slab).
 """
 import os
 import time
@@ -225,7 +232,14 @@ class VimureModel(TransformerMixin, BaseEstimator):
         if not torch.cuda.is_available():
             raise RuntimeError("vimure_b200.VimureModel.fit needs a CUDA device (B200); there is no CPU fallback")
         dev = torch.device("cuda", torch.cuda.current_device()) if dev is None else torch.device(dev)
-        self._store_rho = bool(extra_params.get("store_rho", True))
+        store_rho = extra_params.get("store_rho", True)
+        if isinstance(store_rho, str) and store_rho != "never":
+            raise ValueError('store_rho must be True, False or "never"')
+        self._slab = not isinstance(store_rho, str)
+        self._store_rho = bool(store_rho) if self._slab else True
+        if not self._slab and self.R.kind not in ("ego", "all"):
+            raise ValueError('store_rho="never" needs an ego or all-reporter mask: the statistics of a general reporter '
+                             'mask gather the dense posterior slab')
 
         # ---- sharding (row blocks over ranks, SURVEY.md section 8e)
         dist_opt = extra_params.get("distributed", "auto")
@@ -282,7 +296,8 @@ class VimureModel(TransformerMixin, BaseEstimator):
                 self.timings["pack"] = time.time() - t0
             priors = dict(alpha_theta=self.alpha_theta, beta_theta=self.beta_theta, alpha_lambda=self.alpha_lambda,
                           beta_lambda=self.beta_lambda, alpha_eta=self.alpha_mutuality, beta_eta=self.beta_mutuality)
-            self._engine = eng = CaviEngine(P, priors, mutuality=self.mutuality, eps=self.EPS, group=group)
+            self._engine = eng = CaviEngine(P, priors, mutuality=self.mutuality, eps=self.EPS, group=group,
+                                            slab=self._slab)
             if extra_params.get("graphs", True):
                 # one graph replay per iteration instead of ~17 launches: decisive for launch-bound sizes, and still 1.6 %
                 # at config 3 (1.377 -> 1.355 ms per iteration, B200); sharded fits capture their all-reduces too
@@ -391,7 +406,8 @@ class VimureModel(TransformerMixin, BaseEstimator):
         self.timings["draw_init"] = time.time() - t1
 
         t1 = time.time()
-        engines = [self._engine] + [CaviEngine(P, priors, mutuality=self.mutuality, eps=self.EPS) for _ in range(R - 1)]
+        engines = [self._engine] + [CaviEngine(P, priors, mutuality=self.mutuality, eps=self.EPS, slab=self._slab)
+                                    for _ in range(R - 1)]
         streams = [torch.cuda.Stream(device=dev) for _ in range(R)]
         torch.cuda.synchronize(dev)  # the engines' buffers were zero-filled on the current stream
         for eng, st, s in zip(engines, states, streams):
@@ -455,7 +471,8 @@ class VimureModel(TransformerMixin, BaseEstimator):
         self._engine = engines[R - 1]  # `rho`, `gamma_shp`, ... without _f are the LAST restart's (model.py:925-942)
         self._fetch_params()
         self._engine_f = engines[best] if best is not None else None
-        self._rho_f_dev = engines[best].rho_slab() if (best is not None and best != R - 1) else None
+        # (without a slab the best engine's own tables are rho_f: nothing to materialise)
+        self._rho_f_dev = engines[best].rho_slab() if (best is not None and best != R - 1 and self._slab) else None
         self._rho_f_cache = None
         return maxL, trace
 
@@ -623,9 +640,10 @@ class VimureModel(TransformerMixin, BaseEstimator):
         self.G_exp_theta_f = np.exp(sp.psi(self.gamma_shp_f) - np.log(self.gamma_rte_f))
         self.G_exp_lambda_f = np.exp(sp.psi(self.phi_shp_f) - np.log(self.phi_rte_f))
         self.G_exp_nu_f = np.exp(sp.psi(self.nu_shp_f) - np.log(self.nu_rte_f))
-        # rho_f stays on the device; a copy is needed only when further realisations will overwrite the slab
+        # rho_f stays on the device; a copy is needed only when further realisations will overwrite the slab (without a
+        # slab: the tables and special-tie posteriors it is evaluated from)
         if self.num_realisations > 1 and clone_rho:
-            self._rho_f_dev = self._engine.rho_slab().clone()
+            self._rho_f_dev = self._engine.rho_slab().clone() if self._engine.slab else self._engine.snapshot()
         else:
             self._rho_f_dev = None
         self._rho_f_cache = None
@@ -647,14 +665,18 @@ class VimureModel(TransformerMixin, BaseEstimator):
     def rho_f(self):
         """Posterior of the best realisation (reference model.py:937)."""
         if getattr(self, "_rho_f_cache", None) is None:
-            if self._rho_f_dev is None:
+            eng_f = self._engine_of_rho_f()
+            if self._rho_f_dev is None and eng_f is self._engine:
                 self._rho_f_cache = self.rho
             else:
-                self._rho_f_cache = self._gather_rho(self._rho_f_dev)
+                self._rho_f_cache = self._gather_rho(self._rho_f_slab())
         return self._rho_f_cache
 
     def _rho_f_slab(self):
-        return self._engine.rho_slab() if self._rho_f_dev is None else self._rho_f_dev
+        eng_f = self._engine_of_rho_f()
+        if self._rho_f_dev is None:
+            return eng_f.rho_slab()
+        return eng_f.rho_slab(self._rho_f_dev) if isinstance(self._rho_f_dev, dict) else self._rho_f_dev
 
     @property
     def pr_rho(self):
