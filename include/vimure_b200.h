@@ -330,6 +330,40 @@ int vm_infer_mean(const vm_ctx* c, float* out, void* stream);
  * not numpy's (the reference draws with numpy.random.default_rng(seed)). */
 int vm_sample(const vm_ctx* c, int64_t n_trials, uint64_t seed, uint8_t* out, void* stream);
 
+/* ---- sparse consumers: the ties of the inferred network whose label is nonzero, as an edge list ------------------------
+ * The labels of vm_infer (VM_EDGES_ARGMAX: mode 0; VM_EDGES_THRESHOLD: mode 1) and vm_sample (VM_EDGES_SAMPLE), bit for bit,
+ * without any (L, nloc, N)-sized buffer.  Two passes over the local rows lrow = l*nloc + (i-row0), no host synchronisation
+ * inside either:
+ *   vm_edges_count: row_count[lrow] = number of ties of the row whose label is nonzero;
+ *   vm_edges_emit:  with row_off = the caller's exclusive prefix sum of row_count, o_key[row_off[lrow] + r] = (l*N+i)*N+j
+ *                   (the global flat id) and o_val[...] = label (>= 1) of the r-th such tie of the row, ascending in j: the
+ *                   output is sorted by key, and equals np.nonzero of the dense consumer's output.
+ * `source` says where the posterior is read: VM_EDGES_SLAB = ctx->rho (any mask); VM_EDGES_IMPLICIT = what
+ * vm_materialize_rows evaluates (tab_p, tab_q, layer_consts, utile_ptr, u_col, rho_u32; VM_ENOTSUP under VM_R_CSR).  With
+ * the implicit source, vm_edges_count first writes the per-layer column maxima of tab_q into `workspace`, which
+ * vm_edges_emit reads: rows whose closed form provably has label 0 at every column then only visit their special ties.
+ * VM_EINVAL before any launch for a NULL required pointer, an unknown `what` / `source`, n_trials < 1 (SAMPLE), or the slab
+ * source without a slab. */
+#define VM_EDGES_ARGMAX 0
+#define VM_EDGES_THRESHOLD 1
+#define VM_EDGES_SAMPLE 2
+#define VM_EDGES_SLAB 0
+#define VM_EDGES_IMPLICIT 1
+typedef struct vm_edges_args {
+  int64_t what, source;      /* VM_EDGES_ARGMAX / _THRESHOLD / _SAMPLE;  VM_EDGES_SLAB / _IMPLICIT */
+  double threshold;          /* VM_EDGES_THRESHOLD: label = rho_1 >= (float)threshold */
+  int64_t n_trials;          /* VM_EDGES_SAMPLE, >= 1 */
+  uint64_t seed;             /* VM_EDGES_SAMPLE: the Philox key of vm_sample */
+  int64_t* row_count;        /* [L*nloc], written by vm_edges_count */
+  const int64_t* row_off;    /* [L*nloc], exclusive prefix sum of row_count, read by vm_edges_emit */
+  int64_t* o_key;            /* [sum of row_count], written by vm_edges_emit */
+  uint8_t* o_val;            /* [sum of row_count], written by vm_edges_emit */
+  float* workspace;          /* [L*K], written by vm_edges_count, read by vm_edges_emit (implicit source) */
+} vm_edges_args;
+int64_t vm_edges_size(void);
+int vm_edges_count(const vm_ctx* c, const vm_edges_args* a, void* stream);
+int vm_edges_emit(const vm_ctx* c, const vm_edges_args* a, void* stream);
+
 /* ---- data packing (replaces the data preparation of `__check_fit_params`, model.py:147-176, and utils.py:73-84) --------
  * From the COO list of reports (device arrays) to every packed array `vm_ctx` points to, for one node-row block and a
  * structured reporter mask (VM_R_EGO / VM_R_ALL; a general COO mask is packed by the host-side packer): entries outside

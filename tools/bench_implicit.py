@@ -117,18 +117,12 @@ def profiled(sh, slab, iters, prof_dir, tag):
     return per
 
 
-def sparse_run(N, iters):
-    import torch
-
-    import vimure_b200 as vm
-    from bench import PRIORS
-    from vimure_b200 import _packing
+def sparse_reports(N):
+    """The sparse ego network of `sparse_run`: L = 1, K = 2, two true ties per node, report law lam = (1e-4, 1).
+    Returns (L, K, subs, vals) on the device."""
     from vimure_b200 import synthetic as syn
-    from vimure_b200._engine import CaviEngine
 
     L, K = 1, 2
-    torch.cuda.empty_cache()
-    torch.cuda.reset_peak_memory_stats()
     rng = np.random.RandomState(7)
     ys = np.stack([np.zeros(2 * N, np.int64), rng.randint(0, N, 2 * N), rng.randint(0, N, 2 * N)])
     ys = ys[:, ys[1] != ys[2]]
@@ -136,6 +130,20 @@ def sparse_run(N, iters):
     theta = 0.5 + rng.random_sample((L, N))
     subs, vals = syn.device_reports(L, N, N, K, ys, np.ones(ys.shape[1], np.int32), theta, 0.5, seed=11,
                                     lam=np.array([[1e-4, 1.0]]))
+    return L, K, subs, vals
+
+
+def sparse_run(N, iters):
+    import torch
+
+    import vimure_b200 as vm
+    from bench import PRIORS
+    from vimure_b200 import _packing
+    from vimure_b200._engine import CaviEngine
+
+    torch.cuda.empty_cache()
+    torch.cuda.reset_peak_memory_stats()
+    L, K, subs, vals = sparse_reports(N)
     P = _packing.pack(subs, vals, L, N, N, K, vm.masks.EgoMask(L, N, N), torch.device("cuda"), tile_h=128)
     eng = CaviEngine(P, PRIORS, mutuality=True, eps=1e-12, slab=False)
     eng.enable_graphs()

@@ -53,6 +53,7 @@ def _parse_header():
 
 _synth_cls = None
 _pack_cls = None
+_edges_cls = None
 
 
 def pack_class():
@@ -79,6 +80,19 @@ def synth_class():
 
         _synth_cls = VmSynth
     return _synth_cls
+
+
+def edges_class():
+    """ctypes mirror of `vm_edges_args` (sparse consumers), generated from the header."""
+    global _edges_cls
+    if _edges_cls is None:
+        fields = _parse_struct(open(HEADER).read(), "vm_edges_args")
+
+        class VmEdgesArgs(ctypes.Structure):
+            _fields_ = fields
+
+        _edges_cls = VmEdgesArgs
+    return _edges_cls
 
 
 def header_symbols():
@@ -142,6 +156,9 @@ def open_library(path):
         "vm_infer": (i, [P, i, d, vp, vp]),
         "vm_sample": (i, [P, i64, ctypes.c_uint64, vp, vp]),
         "vm_infer_mean": (i, [P, vp, vp]),
+        "vm_edges_size": (i64, []),
+        "vm_edges_count": (i, [P, ctypes.POINTER(edges_class()), vp]),
+        "vm_edges_emit": (i, [P, ctypes.POINTER(edges_class()), vp]),
         "vm_test_special": (i, [vp, vp, vp, i64, vp]),
         "vm_pack_size": (i64, []),
         "vm_pack_workspace_bytes": (i64, [ctypes.POINTER(pack_class())]),
@@ -160,6 +177,8 @@ def open_library(path):
         raise RuntimeError("vm_pack_args layout mismatch between header and library (stale build?)")
     if lib.vm_synth_size() != ctypes.sizeof(synth_class()):
         raise RuntimeError("vm_synth layout mismatch between header and library (stale build?)")
+    if lib.vm_edges_size() != ctypes.sizeof(edges_class()):
+        raise RuntimeError("vm_edges_args layout mismatch between header and library (stale build?)")
     if lib.vm_abi_version() != consts()["VM_ABI_VERSION"]:
         raise RuntimeError("vimure_b200: ABI version mismatch between header and library (stale build?)")
     return lib

@@ -478,6 +478,46 @@ class CaviEngine:
         finally:
             self._restore(old)
 
+    def infer_edges(self, mode=0, threshold=0.5, slab=None):
+        """The ties of `infer(mode, threshold, slab)` whose label is nonzero, as an edge list of this rank's rows: (keys
+        int64 (l*N+i)*N+j ascending, labels uint8) on the device, without any (L, nloc, N) buffer (`vm_edges_*`)."""
+        return self._edges(self.C["VM_EDGES_THRESHOLD"] if mode == 1 else self.C["VM_EDGES_ARGMAX"], slab,
+                           threshold=float(threshold))
+
+    def sample_edges(self, n_trials=1, seed=0, slab=None):
+        """The ties of `sample(n_trials, seed, slab)` whose label is nonzero: (keys int64 ascending, labels uint8) on the
+        device, this rank's rows."""
+        return self._edges(self.C["VM_EDGES_SAMPLE"], slab, n_trials=int(n_trials), seed=int(seed) & (2**64 - 1))
+
+    def _edges(self, what, slab, **kw):
+        """One vm_edges_count, the row offsets (one cumsum), one D2H read of the total, one vm_edges_emit.  The posterior is
+        read where it is cheapest to evaluate: from the tables (implicit source) whenever they describe the posterior being
+        consumed -- this engine's own after an iteration, slab or not, or a `snapshot()` -- and from a slab for a cloned
+        slab of an earlier restart, the prior, and the general mask (which has no tables)."""
+        C, P = self.C, self.P
+        old = self._use_slab(slab)  # the dense consumers' preconditions (and the prior's slab, when that is the posterior)
+        try:
+            implicit = not self.slab or (slab is None and not getattr(self, "rho_is_prior", False) and P.r_mode != 2)
+            rows = P.L * P.nloc
+            i64 = dict(dtype=torch.int64, device=self.dev)
+            off = torch.zeros(rows + 1, **i64)
+            cnt = torch.empty(rows, **i64)
+            ws = torch.empty(P.L * P.K, dtype=torch.float32, device=self.dev)
+            a = _capi.edges_class()(what=what, source=C["VM_EDGES_IMPLICIT"] if implicit else C["VM_EDGES_SLAB"],
+                                    row_count=cnt.data_ptr(), workspace=ws.data_ptr(), **kw)
+            st = self._stream()
+            _capi.check(self.lib.vm_edges_count(self._cref, ctypes.byref(a), st), "vm_edges_count")
+            torch.cumsum(cnt, 0, out=off[1:])
+            total = int(off[-1])
+            keys = torch.empty(max(total, 1), **i64)
+            vals = torch.empty(max(total, 1), dtype=torch.uint8, device=self.dev)
+            a.row_off, a.o_key, a.o_val = off.data_ptr(), keys.data_ptr(), vals.data_ptr()
+            _capi.check(self.lib.vm_edges_emit(self._cref, ctypes.byref(a), st), "vm_edges_emit")
+            self.n_launch += 2 + int(implicit)
+            return keys[:total], vals[:total]
+        finally:
+            self._restore(old)
+
     def sample(self, n_trials=1, seed=0, slab=None):
         """argmax of the counts of `n_trials` categorical draws per tie (reference `sample_inferred_model`,
         model.py:1086-1088) on the device: uint8 (L, nloc, N).  Philox stream keyed by (seed, global tie id)."""

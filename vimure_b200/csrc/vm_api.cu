@@ -58,24 +58,7 @@ extern "C" int vm_infer_mean(const vm_ctx* c, float* out, void* stream) {
   return e == cudaSuccess ? 0 : (int)e;
 }
 
-// ---- posterior sampling on the slab (model.py:1062-1096) ------------------------------------------------------
-// Philox4x32-10 (Salmon et al. 2011), counter = (global tie id, block of 4 draws), key = seed: the stream of a tie does
-// not depend on the launch geometry nor on how the ties are sharded over ranks.
-__device__ __forceinline__ uint4 vm_philox4x32(uint4 ctr, uint2 key) {
-#pragma unroll
-  for (int r = 0; r < 10; ++r) {
-    const uint32_t hi0 = __umulhi(0xD2511F53u, ctr.x), lo0 = 0xD2511F53u * ctr.x;
-    const uint32_t hi1 = __umulhi(0xCD9E8D57u, ctr.z), lo1 = 0xCD9E8D57u * ctr.z;
-    ctr = make_uint4(hi1 ^ ctr.y ^ key.x, lo1, hi0 ^ ctr.w ^ key.y, lo0);
-    key.x += 0x9E3779B9u;
-    key.y += 0xBB67AE85u;
-  }
-  return ctr;
-}
-
-// One thread per owned tie: n_trials draws from Categorical(rho[t,:]) -> the category drawn most often (first one on a
-// draw), i.e. `multinomial(n, rho).argmax(-1)` of model.py:1086-1088.  A draw that exceeds the cumulative sum (rounding,
-// or an all-zero row) falls into the LAST category, as numpy's multinomial assigns the remainder.
+// ---- posterior sampling on the slab (model.py:1062-1096): one thread per owned tie, vm_sample_label -------------
 __global__ void __launch_bounds__(256) k_sample(const float* __restrict__ rho, int64_t nloc, int64_t N, int64_t row0,
                                                 int64_t T, int K, int64_t n_trials, uint64_t seed,
                                                 uint8_t* __restrict__ out) {
@@ -83,37 +66,7 @@ __global__ void __launch_bounds__(256) k_sample(const float* __restrict__ rho, i
   for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < T; t += (int64_t)gridDim.x * blockDim.x) {
     const int64_t lrow = t / N, j = t - lrow * N, l = lrow / nloc, i = lrow - l * nloc + row0;
     const uint64_t gt = (uint64_t)((l * N + i) * N + j);
-    const float* r = rho + t * K;
-    float p[VM_MAX_K];
-    int cnt[VM_MAX_K];
-    float sum = 0.f;
-    for (int k = 0; k < K; ++k) {
-      p[k] = r[k];
-      sum += p[k];
-      cnt[k] = 0;
-    }
-    for (int64_t d0 = 0; d0 < n_trials; d0 += 4) {
-      const uint64_t blk = (uint64_t)(d0 >> 2);
-      const uint4 x = vm_philox4x32(make_uint4((uint32_t)gt, (uint32_t)(gt >> 32), (uint32_t)blk, (uint32_t)(blk >> 32)), key);
-      const uint32_t xs[4] = {x.x, x.y, x.z, x.w};
-#pragma unroll
-      for (int q = 0; q < 4; ++q) {
-        if (d0 + q >= n_trials) break;
-        // uniform strictly inside (0, sum): 23 random bits + 1/2 is exact in fp32 (24 bits would round up to 1.0)
-        const float u = ((float)(xs[q] >> 9) + 0.5f) * (1.0f / 8388608.0f) * sum;
-        float cum = 0.f;
-        int k = 0;
-        for (; k < K - 1; ++k) {
-          cum += p[k];
-          if (u < cum) break;
-        }
-        cnt[k] += 1;
-      }
-    }
-    int best = 0;
-    for (int k = 1; k < K; ++k)
-      if (cnt[k] > cnt[best]) best = k;
-    out[t] = (uint8_t)best;
+    out[t] = (uint8_t)vm_sample_label(rho + t * K, K, n_trials, gt, key);
   }
 }
 extern "C" int vm_sample(const vm_ctx* c, int64_t n_trials, uint64_t seed, uint8_t* out, void* stream) {
@@ -126,6 +79,10 @@ extern "C" int vm_sample(const vm_ctx* c, int64_t n_trials, uint64_t seed, uint8
   cudaError_t e = cudaGetLastError();
   return e == cudaSuccess ? 0 : (int)e;
 }
+
+extern "C" int64_t vm_edges_size(void) { return (int64_t)sizeof(vm_edges_args); }
+extern "C" int vm_edges_count(const vm_ctx* c, const vm_edges_args* a, void* stream) { VM_ROUTE(edges(c, a, 0, stream)); }
+extern "C" int vm_edges_emit(const vm_ctx* c, const vm_edges_args* a, void* stream) { VM_ROUTE(edges(c, a, 1, stream)); }
 
 __global__ void k_test_special(const double* x, double* dg, double* lg, int64_t n) {
   const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;

@@ -29,6 +29,7 @@ struct vm_tu_api {
   int (*run)(const vm_ctx*, int, int, int, void*);
   int (*infer)(const vm_ctx*, int, double, uint8_t*, void*);
   int (*materialize_rows)(const vm_ctx*, int64_t, int64_t, float*, void*);
+  int (*edges)(const vm_ctx*, const vm_edges_args*, int, void*);  // int: 0 = vm_edges_count, 1 = vm_edges_emit
 };
 
 // Column tile of the dense kernels: TW = 128*NCH columns; NCH is K-dependent so that the per-lane column accumulators
@@ -168,6 +169,64 @@ __device__ __forceinline__ void vm_formula_rho(const float* a, bool may_dead, fl
       for (int k = 0; k < K; ++k) out[k] = 0.f;
     }
   }
+}
+
+// ------------------------------------------------------------------ posterior sampling (model.py:1062-1096)
+// Philox4x32-10 (Salmon et al. 2011), counter = (global tie id, block of 4 draws), key = seed: the stream of a tie does
+// not depend on the launch geometry nor on how the ties are sharded over ranks.
+__device__ __forceinline__ uint4 vm_philox4x32(uint4 ctr, uint2 key) {
+#pragma unroll
+  for (int r = 0; r < 10; ++r) {
+    const uint32_t hi0 = __umulhi(0xD2511F53u, ctr.x), lo0 = 0xD2511F53u * ctr.x;
+    const uint32_t hi1 = __umulhi(0xCD9E8D57u, ctr.z), lo1 = 0xCD9E8D57u * ctr.z;
+    ctr = make_uint4(hi1 ^ ctr.y ^ key.x, lo1, hi0 ^ ctr.w ^ key.y, lo0);
+    key.x += 0x9E3779B9u;
+    key.y += 0xBB67AE85u;
+  }
+  return ctr;
+}
+
+// The label vm_sample gives the tie `gt` (global flat id) of posterior r[0..K): n_trials draws from Categorical(r) -> the
+// category drawn most often (first one on a draw), i.e. `multinomial(n, rho).argmax(-1)` of model.py:1086-1088.  A draw
+// that exceeds the cumulative sum (rounding, or an all-zero row) falls into the LAST category, as numpy's multinomial
+// assigns the remainder.  Shared by the dense (k_sample) and the sparse (k_edges) consumers.
+__device__ __forceinline__ int vm_sample_label(const float* r, int K, int64_t n_trials, uint64_t gt, uint2 key) {
+  float p[VM_MAX_K];
+  int cnt[VM_MAX_K];
+  float sum = 0.f;
+  for (int k = 0; k < K; ++k) {
+    p[k] = r[k];
+    sum += p[k];
+    cnt[k] = 0;
+  }
+  // Every draw lands in category 0 when the fp32 sum equals p[0] > 0: the first cumulative sum is p[0] = sum, and the
+  // uniform below is v*sum with v = ((x>>9)+0.5)*2^-23 <= 1-2^-24 (exact), so v*sum <= sum - sum*2^-24.  For sum in
+  // [2^e, 2^(e+1)) that is at least ulp(sum)/2 below sum, strictly unless sum = 2^e, where sum - 2^(e-24) is itself
+  // representable: fl(v*sum) < sum = cum in every case, and the draw stops at k = 0.  (sum = 0, a dead tie, goes to the
+  // last category below; a NaN fails the test.)  Most ties of a sparse network: no Philox evaluation needed.
+  if (sum == p[0] && sum > 0.f) return 0;
+  for (int64_t d0 = 0; d0 < n_trials; d0 += 4) {
+    const uint64_t blk = (uint64_t)(d0 >> 2);
+    const uint4 x = vm_philox4x32(make_uint4((uint32_t)gt, (uint32_t)(gt >> 32), (uint32_t)blk, (uint32_t)(blk >> 32)), key);
+    const uint32_t xs[4] = {x.x, x.y, x.z, x.w};
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+      if (d0 + q >= n_trials) break;
+      // uniform strictly inside (0, sum): 23 random bits + 1/2 is exact in fp32 (24 bits would round up to 1.0)
+      const float u = ((float)(xs[q] >> 9) + 0.5f) * (1.0f / 8388608.0f) * sum;
+      float cum = 0.f;
+      int k = 0;
+      for (; k < K - 1; ++k) {
+        cum += p[k];
+        if (u < cum) break;
+      }
+      cnt[k] += 1;
+    }
+  }
+  int best = 0;
+  for (int k = 1; k < K; ++k)
+    if (cnt[k] > cnt[best]) best = k;
+  return best;
 }
 
 // log1p for fp32: series below 0.05 (exact to ~1e-10 relative), MUFU-based above

@@ -2333,22 +2333,177 @@ __global__ void k_patch_special(const __grid_constant__ vm_ctx c) {
   float* dst = c.rho + ((int64_t)c.u_lrow[u] * c.N + c.u_col[u]) * c.K;
   for (int k = 0; k < (int)c.K; ++k) dst[k] = (float)c.rho_u[u * c.K + k];
 }
-// rho_max (model.py:1148-1149) / fixed threshold on rho[...,1] (model.py:1155-1166, utils.py:207-217)
+// rho_max (model.py:1148-1149): argmax_k r[k], the first maximum wins (mode 0) / fixed threshold on rho[...,1]
+// (model.py:1155-1166, utils.py:207-217, mode 1).  Shared by the dense (k_infer) and the sparse (k_edges) consumers.
+__device__ __forceinline__ int vm_infer_label(const float* r, int K, int mode, float thr) {
+  if (mode == 0) {
+    int best = 0;
+    float bv = r[0];
+    for (int k = 1; k < K; ++k)
+      if (r[k] > bv) {
+        bv = r[k];
+        best = k;
+      }
+    return best;
+  }
+  return r[1] >= thr ? 1 : 0;
+}
 __global__ void k_infer(const float* rho, int64_t T, int K, int mode, float thr, uint8_t* out) {
-  for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < T; t += (int64_t)gridDim.x * blockDim.x) {
-    const float* r = rho + t * K;
-    if (mode == 0) {
-      int best = 0;
-      float bv = r[0];
-      for (int k = 1; k < K; ++k)
-        if (r[k] > bv) {
-          bv = r[k];
-          best = k;
-        }
-      out[t] = (uint8_t)best;
-    } else {
-      out[t] = r[1] >= thr ? 1 : 0;
+  for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < T; t += (int64_t)gridDim.x * blockDim.x)
+    out[t] = (uint8_t)vm_infer_label(rho + t * K, K, mode, thr);
+}
+
+// ---- sparse consumers (vm_edges_count / vm_edges_emit) ----------------------------------------------------------------
+// qmax[l*K+k] = max_j tab_q[l,j,k], one CTA per (k, l); NaN when the layer has a NaN entry (then no row of it is skipped:
+// every comparison with NaN is false).
+__global__ void __launch_bounds__(256) k_edges_qmax(const float* __restrict__ tab_q, int64_t N, int K, float* qmax) {
+  __shared__ float sm[8];
+  const int k = blockIdx.x, l = blockIdx.y;
+  float m = -INFINITY;
+  bool nan = false;
+  for (int64_t j = threadIdx.x; j < N; j += blockDim.x) {
+    const float v = tab_q[((int64_t)l * N + j) * K + k];
+    m = fmaxf(m, v);
+    nan |= v != v;
+  }
+  nan = __syncthreads_or(nan);
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_down_sync(0xffffffffu, m, o));
+  if ((threadIdx.x & 31) == 0) sm[threadIdx.x >> 5] = m;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    for (int w = 1; w < 8; ++w) m = fmaxf(m, sm[w]);
+    qmax[l * K + k] = nan ? __int_as_float(0x7fc00000) : m;
+  }
+}
+
+// Can no tie of this row's closed form have a nonzero label?  With a_k = fl(p_k + q_k) for the tie's column and the layer's
+// column maximum qmax_k >= q_k, rounding is monotone: a_k <= fl(p_k + qmax_k) =: b_k.  Then (vm_formula_rho: r_k =
+// ex2(a_k), s = sum r_k, inv = rcp(1+s), out = (inv, r_k*inv); ex2/rcp.approx are within 2 ulp, far inside the margins):
+//  ARGMAX:    b_k < -1 for every k >= 1 gives r_k < 1/2 (1+2^-21) < 1, so out_k = fl(r_k*inv) <= fl(inv) = out_0: never
+//             strictly greater, the label stays 0.  A dead tie (all zeros) is label 0 too.
+//  THRESHOLD: thr > 0 and b_1 < log2(thr) - 1 gives r_1 < thr/2 (1+2^-21) and inv <= 1 (1+2^-23), so out_1 < thr.  A dead
+//             tie is 0 < thr.
+//  SAMPLE:    b_k < -30 for every k >= 1 gives r_k < 2^-30 (1+2^-21), out_k < 2^-29.9 inv: K-1 <= 31 such terms are each
+//             below half an ulp of inv (inv >= 1/2 since s < 2^-25), so the fp32 sum of vm_sample_label equals p[0] = inv > 0
+//             and every draw lands in category 0 (see there).  Only when the layer cannot be dead: a dead tie sums to 0 and
+//             goes to the LAST category, an edge.
+template <int K>
+__device__ __forceinline__ bool vm_edges_row_skip(const float* p, const float* qmax, int what, float thr, float thr_bound,
+                                                  bool may_dead) {
+  if (what == VM_EDGES_THRESHOLD) return thr > 0.f && __fadd_rn(p[1], qmax[1]) < thr_bound;
+  if (what == VM_EDGES_SAMPLE && may_dead) return false;
+  const float bound = what == VM_EDGES_ARGMAX ? -1.f : -30.f;
+  bool s = true;
+#pragma unroll
+  for (int k = 1; k < K; ++k) s = s && __fadd_rn(p[k], qmax[k]) < bound;
+  return s;
+}
+
+template <int K>
+__device__ __forceinline__ int vm_edge_label(const float* o, int what, float thr, int64_t n_trials, uint64_t gt, uint2 key) {
+  if (what == VM_EDGES_SAMPLE) return vm_sample_label(o, K, n_trials, gt, key);
+  return vm_infer_label(o, K, what, thr);  // VM_EDGES_ARGMAX / _THRESHOLD = vm_infer's modes 0 / 1
+}
+
+// One step of 256 ties (one per thread, in order): the block-wide exclusive prefix of (label != 0) places this thread's
+// edge; returns the row's running count.  Every thread of the block calls it.
+__device__ __forceinline__ int64_t vm_edges_put(int lab, int64_t key, int64_t pos, bool emit, const vm_edges_args& a,
+                                                int* s_warp) {
+  const bool pred = lab != 0;
+  const unsigned b = __ballot_sync(0xffffffffu, pred);
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  if (lane == 0) s_warp[w] = __popc(b);
+  __syncthreads();
+  int off = __popc(b & ((1u << lane) - 1u)), tot = 0;
+#pragma unroll
+  for (int q = 0; q < 8; ++q) {
+    const int v = s_warp[q];
+    off += q < w ? v : 0;
+    tot += v;
+  }
+  __syncthreads();
+  if (emit && pred) {
+    a.o_key[pos + off] = key;
+    a.o_val[pos + off] = (uint8_t)lab;
+  }
+  return pos + tot;
+}
+
+// Count (emit = 0) or write (emit = 1) the edges of the local rows, one CTA of 256 threads per row (rows strided over the
+// grid), columns in chunks of 256.  Implicit source: the closed form of vm_materialize_rows, and the row's special ties
+// (utile_ptr[lrow*nct] .. utile_ptr[(lrow+1)*nct], ascending in column) from rho_u32, found chunk by chunk by a moving
+// pointer -- at most 256 of them fall into a chunk of 256 columns; a row that vm_edges_row_skip rules out only walks its
+// special ties.  Slab source: ctx->rho.
+template <int K>
+__global__ void __launch_bounds__(256) k_edges(const __grid_constant__ vm_ctx c, const __grid_constant__ vm_edges_args a,
+                                               int emit, float thr, float thr_bound) {
+  __shared__ int s_u[256];
+  __shared__ int s_warp[8];
+  const int N = (int)c.N, tid = threadIdx.x, what = (int)a.what;
+  const bool implicit = a.source == VM_EDGES_IMPLICIT;
+  const uint2 key = make_uint2((uint32_t)a.seed, (uint32_t)(a.seed >> 32));
+  const int64_t rows = c.L * c.nloc;
+  for (int64_t lrow = blockIdx.x; lrow < rows; lrow += gridDim.x) {
+    const int l = (int)(lrow / c.nloc);
+    const int64_t g0 = ((int64_t)l * N + (lrow - (int64_t)l * c.nloc + c.row0)) * N;  // global id of the row's column 0
+    int64_t pos = emit ? a.row_off[lrow] : 0;
+    int us = 0, ue = 0;
+    bool may_dead = false, skip = false;
+    if (implicit) {
+      us = c.utile_ptr[lrow * c.nct];
+      ue = c.utile_ptr[(lrow + 1) * c.nct];
+      may_dead = vm_may_dead<K>(c, l);
+      skip = vm_edges_row_skip<K>(c.tab_p + lrow * K, a.workspace + (int64_t)l * K, what, thr, thr_bound, may_dead);
     }
+    if (skip) {
+      for (int u0 = us; u0 < ue; u0 += 256) {
+        const int u = u0 + tid;
+        int lab = 0, col = 0;
+        if (u < ue) {
+          float o[K];
+          col = c.u_col[u];
+#pragma unroll
+          for (int k = 0; k < K; ++k) o[k] = c.rho_u32[(int64_t)u * K + k];
+          lab = vm_edge_label<K>(o, what, thr, a.n_trials, (uint64_t)(g0 + col), key);
+        }
+        pos = vm_edges_put(lab, g0 + col, pos, emit, a, s_warp);
+      }
+    } else {
+      int up = us;
+      for (int j0 = 0; j0 < N; j0 += 256) {
+        const int j = j0 + tid;
+        int su = -1;
+        if (implicit) {
+          s_u[tid] = -1;
+          __syncthreads();
+          const int u = up + tid;
+          const bool in = u < ue && c.u_col[u] < j0 + 256;
+          if (in) s_u[c.u_col[u] - j0] = u;
+          up += __syncthreads_count(in);
+          su = s_u[tid];
+        }
+        int lab = 0;
+        if (j < N) {
+          float o[K];
+          if (!implicit) {
+#pragma unroll
+            for (int k = 0; k < K; ++k) o[k] = c.rho[(lrow * N + j) * K + k];
+          } else if (su >= 0) {
+#pragma unroll
+            for (int k = 0; k < K; ++k) o[k] = c.rho_u32[(int64_t)su * K + k];
+          } else {
+            float lo[K], epsr;
+            bool dead;
+            vm_tie_logodds<K>(c, l, lrow, j, lo);
+            vm_formula_rho<K>(lo, may_dead, o, epsr, dead);
+          }
+          lab = vm_edge_label<K>(o, what, thr, a.n_trials, (uint64_t)(g0 + j), key);
+        }
+        pos = vm_edges_put(lab, g0 + j, pos, emit, a, s_warp);
+      }
+    }
+    if (!emit && tid == 0) a.row_count[lrow] = pos;
   }
 }
 // The posterior the last rho update left, for the local rows [lrow0, lrow0+nrows) (lrow = l*nloc + i), into `out` in the
@@ -2818,12 +2973,38 @@ static int tu_materialize_rows(const vm_ctx* c, int64_t lrow0, int64_t nrows, fl
   return 0;
 }
 
+// vm_edges_count (emit = 0) / vm_edges_emit (emit = 1); every argument is checked before anything is launched
+static int tu_edges(const vm_ctx* c, const vm_edges_args* a, int emit, void* stream) {
+  int rc = check_ctx(c);
+  if (rc) return rc;
+  if (!a || a->what < VM_EDGES_ARGMAX || a->what > VM_EDGES_SAMPLE) return VM_EINVAL;
+  if (a->source != VM_EDGES_SLAB && a->source != VM_EDGES_IMPLICIT) return VM_EINVAL;
+  if (a->what == VM_EDGES_SAMPLE && a->n_trials < 1) return VM_EINVAL;
+  if (emit ? (!a->row_off || !a->o_key || !a->o_val) : !a->row_count) return VM_EINVAL;
+  const bool implicit = a->source == VM_EDGES_IMPLICIT;
+  if (implicit ? !a->workspace : !c->rho) return VM_EINVAL;
+  if (implicit && c->r_mode == VM_R_CSR) return VM_ENOTSUP;  // no row/column tables (as vm_materialize_rows)
+  const int64_t rows = c->L * c->nloc;
+  if (rows <= 0) return 0;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (implicit && !emit) {
+    k_edges_qmax<<<dim3((unsigned)c->K, (unsigned)c->L), 256, 0, st>>>(c->tab_q, c->N, (int)c->K, a->workspace);
+    VM_CHECK_LAUNCH();
+  }
+  const float thr = (float)a->threshold;  // as vm_infer
+  const float thr_bound = thr > 0.f ? (float)(log2((double)thr) - 1.0) : 0.f;
+  const unsigned grid = (unsigned)imin64(rows, 148 * 8);
+  DISPATCH_K(c->K, (k_edges<K><<<grid, 256, 0, st>>>(*c, *a, emit, thr, thr_bound)));
+  VM_CHECK_LAUNCH();
+  return 0;
+}
+
 }  // namespace
 
 extern "C" const vm_tu_api* VM_PASTE(vm_tu_api_, VM_TU_ID)(void) {
   using namespace VM_PASTE(vmtu, VM_TU_ID);
   static const vm_tu_api api = {tu_materialize_prior, tu_refresh_cache, tu_init_stats, tu_phase_gamma, tu_phase_phi,
                                 tu_phase_rho,         tu_dense_only,    tu_phase_finish, tu_iteration, tu_run, tu_infer,
-                                tu_materialize_rows};
+                                tu_materialize_rows,  tu_edges};
   return &api;
 }

@@ -722,12 +722,53 @@ class VimureModel(TransformerMixin, BaseEstimator):
         earlier restart won -- and assemble the (L, N, N) result on the host: 1 byte (4 for rho_mean) per tie crosses
         PCIe instead of an fp64 copy of rho.  On a sharded fit every rank consumes its row block and the blocks are
         all-gathered (collective: every rank must call)."""
-        eng = getattr(self, "_engine_f", None) or self._engine
-        slab = None if (getattr(self, "_engine_f", None) is not None or self._rho_f_dev is None) else self._rho_f_dev
+        eng, slab = self._rho_f_source()
         out = getattr(eng, what)(*args, slab=slab)
         if self._world > 1:
             out = self._all_gather_rows(out)
         return out.cpu().numpy()
+
+    def _rho_f_source(self):
+        """(engine, slab argument of its consumers) that read rho_f: see `_consume`."""
+        eng = getattr(self, "_engine_f", None) or self._engine
+        slab = None if (getattr(self, "_engine_f", None) is not None or self._rho_f_dev is None) else self._rho_f_dev
+        return eng, slab
+
+    def _consume_edges(self, what, dtype, *args):
+        """Run a sparse consumer (`infer_edges`, `sample_edges` of the engine) on rho_f, chosen as in `_consume`, and return
+        the ties whose label is nonzero as an sptensor (L, N, N) with subs (l, i, j), sorted, and `dtype` values.  On a
+        sharded fit every rank extracts its own rows and the edge lists are all-gathered (collective: every rank must
+        call); a rank's rows cover every layer, so the gathered lists are merged by key."""
+        eng, slab = self._rho_f_source()
+        keys, vals = getattr(eng, what)(*args, slab=slab)
+        if self._world > 1:
+            keys, vals = self._all_gather_edges(keys, vals)
+        keys, vals = keys.cpu().numpy(), vals.cpu().numpy()
+        l, r = np.divmod(keys, np.int64(self.N) * self.N)
+        i, j = np.divmod(r, np.int64(self.N))
+        return sptensor((l, i, j), vals.astype(dtype), shape=(self.L, self.N, self.N))
+
+    def _all_gather_edges(self, keys, vals):
+        """Every rank's (keys, labels), merged by key on every rank (collective): the counts first, then one padded
+        all_gather of each -- on the device with NCCL, on the host with gloo (as `_all_gather_rows`)."""
+        import torch.distributed as dist
+
+        if dist.get_backend() != "nccl":
+            keys, vals = keys.cpu(), vals.cpu()
+        n = torch.tensor([keys.numel()], dtype=torch.int64, device=keys.device)
+        ns = [torch.empty_like(n) for _ in range(self._world)]
+        dist.all_gather(ns, n)
+        ns = [int(v) for v in torch.cat(ns).cpu()]
+        cap = max(max(ns), 1)
+        parts = []
+        for t in (keys, vals):
+            pad = torch.zeros(cap, dtype=t.dtype, device=t.device)
+            pad[:t.numel()] = t
+            got = [torch.empty_like(pad) for _ in range(self._world)]
+            dist.all_gather(got, pad)
+            parts.append(torch.cat([g[:c] for g, c in zip(got, ns)]))
+        keys, order = torch.sort(parts[0])
+        return keys, parts[1][order]
 
     def _all_gather_rows(self, t):
         """Concatenate the ranks' row blocks (dim 1) of a per-tie tensor; every rank gets the whole (collective).  NCCL
@@ -745,20 +786,28 @@ class VimureModel(TransformerMixin, BaseEstimator):
 
     def _engine_of_rho_f(self):
         """The engine whose consumers read rho_f (see `_consume`; pass `slab=self._rho_f_dev` when that is not None)."""
-        return getattr(self, "_engine_f", None) or self._engine
+        return self._rho_f_source()[0]
 
-    def sample_inferred_model(self, N=1, seed=None, rng="auto"):
+    def sample_inferred_model(self, N=1, seed=None, rng="auto", sparse=False):
         """Sample Y trials from the rho distribution (reference model.py:1062-1096): a list of N arrays (L, N, N), each the
         argmax of the counts of N categorical draws per tie.
 
         rng = "numpy": the reference's generator (`default_rng(seed + i).multinomial`) on the host, which materialises
         rho_f as float64 -- 8 bytes * L*N*N*K; rng = "device": the `vm_sample` kernel on the fp32 slab (Philox stream
         keyed by seed and tie: same law, different stream, 1 byte per tie comes back); "auto": numpy while
-        L*N*N*K <= 5e7, else device."""
+        L*N*N*K <= 5e7, else device.
+
+        sparse=True: a list of `sptensor` (L, N, N) holding the ties whose label is nonzero, equal to `sptensor.fromarray`
+        of the device draws for the same seeds, evaluated tie by tie on the device without any N*N-sized buffer (the
+        device generator only: "auto" means "device", "numpy" raises)."""
         if seed is None:
             seed = self.seed
         if rng not in ("auto", "numpy", "device"):
             raise ValueError("rng must be 'auto', 'numpy' or 'device'")
+        if sparse:
+            if rng == "numpy":
+                raise ValueError('sample_inferred_model(sparse=True) draws on the device: rng="numpy" materialises rho_f')
+            return [self._consume_edges("sample_edges", "int", N, int(seed) + i) for i in range(0, N)]
         if rng == "auto":
             rng = "device" if float(self.L) * self.N * self.N * self.K > AUTO_REFERENCE_INIT_LIMIT else "numpy"
         if rng == "device":
@@ -772,10 +821,9 @@ class VimureModel(TransformerMixin, BaseEstimator):
 
         return [sampleY(seed + i) for i in range(0, N)]
 
-    def get_inferred_model(self, method="rho_max", threshold=None):
-        """Estimate Y from rho_f: rho_max | rho_mean | fixed_threshold | heuristic_threshold (model.py:1099-1188).
-        Every method runs on the device slab (float32 storage: a posterior that sits within ~1e-7 of a threshold, or two
-        categories that tie to that precision, can come out differently from a float64 evaluation)."""
+    def _inferred_method(self, method, threshold):
+        """Resolve `get_inferred_model`'s method (model.py:1099-1188): (the engine's infer arguments (mode, threshold), or
+        None for rho_mean; the dtype of the result)."""
         OPTIONS = ["rho_max", "rho_mean", "fixed_threshold", "heuristic_threshold"]
         try:
             method = match_arg(method, OPTIONS)[0]
@@ -789,15 +837,33 @@ class VimureModel(TransformerMixin, BaseEstimator):
             method = "rho_max"
 
         if method == "rho_max":
-            return self._consume("infer", 0, 0.5).astype("int")
+            return (0, 0.5), "int"
         if method == "rho_mean":  # np.dot(rho_f, range(K)), model.py:1151-1153
-            return self._consume("infer_mean").astype(np.float64)
+            return None, np.float64
         if method == "fixed_threshold":
             if (threshold is None) or (threshold > 1) or (threshold < 0):
                 raise ValueError('For method="fixed_threshold", you must set the threshold to a value in [0,1].')
-            return self._consume("infer", 1, float(threshold)).astype(np.float64)
+            return (1, float(threshold)), np.float64
         # heuristic_threshold: 0.54 * G_exp_nu - 0.01 (utils.py:200-204; reads G_exp_nu, not G_exp_nu_f)
-        return self._consume("infer", 1, float(get_optimal_threshold(self))).astype("int")
+        return (1, float(get_optimal_threshold(self))), "int"
+
+    def get_inferred_model(self, method="rho_max", threshold=None, sparse=False):
+        """Estimate Y from rho_f: rho_max | rho_mean | fixed_threshold | heuristic_threshold (model.py:1099-1188).
+        Every method runs on the device slab (float32 storage: a posterior that sits within ~1e-7 of a threshold, or two
+        categories that tie to that precision, can come out differently from a float64 evaluation).
+
+        sparse=True: an `sptensor` (L, N, N) of the ties whose estimate is nonzero, equal to `sptensor.fromarray` of the
+        dense result (same subs, values and dtype), evaluated tie by tie on the device without any N*N-sized buffer --
+        the form to ask for on large networks.  Not for rho_mean, whose every tie is nonzero (ValueError)."""
+        args, dtype = self._inferred_method(method, threshold)
+        if args is None:
+            if sparse:
+                raise ValueError('get_inferred_model("rho_mean") has no sparse form: the posterior mean of every tie is '
+                                 "nonzero")
+            return self._consume("infer_mean").astype(dtype)
+        if sparse:
+            return self._consume_edges("infer_edges", dtype, *args)
+        return self._consume("infer", *args).astype(dtype)
 
     def get_posterior_estimates(self):
         """Posterior estimates nu, theta, lambda, rho (reference model.py:1191-1214)."""
