@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define VM_ABI_VERSION 16
+#define VM_ABI_VERSION 17
 
 /* reporter-mask structure (how R[l,i,j,m] is represented) */
 #define VM_R_EGO 0 /* reporter m == node m reports row m and column m (vimure synthetic.py:1184-1204, _io.py:229-242) */
@@ -38,13 +38,12 @@ extern "C" {
 
 /* flags for vm_phase_rho / vm_phase_finish / vm_iteration */
 #define VM_F_ELBO 1      /* also produce the ELBO (model.py:948-1019) */
-#define VM_F_NO_STORE 2  /* do not write the dense rho slab this iteration (statistics only) */
+#define VM_F_NO_STORE 2  /* write no dense rho slab this iteration: the dense kernels run statistics-only (no stage,
+                            no store, no patches) and vm_ctx.rho may be NULL.  Every other kernel and every number is
+                            that of a storing iteration; the tables (tab_p, tab_q, layer_consts) and rho_u32 the
+                            iteration leaves behind ARE the posterior (vm_materialize_rows evaluates it).  Not with
+                            VM_R_CSR, whose statistics gather the slab: VM_ENOTSUP before any phase runs. */
 #define VM_F_INIT 4      /* vm_phase_finish only: consume the initial statistics, do not update nu */
-#define VM_F_NO_SLAB 8   /* this rank has no slab (vm_ctx.rho == NULL): the fast dense kernels run statistics-only (no
-                            stage, no store, no patches); the tables (tab_p, tab_q, layer_consts) and rho_u32 the iteration
-                            leaves behind ARE the posterior (vm_materialize_rows evaluates it).  Not with VM_R_CSR, whose
-                            statistics gather the slab (VM_ENOTSUP).  Unlike VM_F_NO_STORE, every kernel and every number
-                            is that of a storing iteration. */
 
 /* error codes (negative) */
 #define VM_EINVAL (-1)    /* bad argument / unsupported K */
@@ -127,9 +126,9 @@ typedef struct vm_ctx {
                   ln rho_k/rho_0 = ln2 lo_k - S (E[lambda_k]-E[lambda_0])
                                    + x [ (f_k-f_0) E[log theta_m] + f_k E[log lambda_k] - f_0 E[log lambda_0] ],
                every term O(1..30).
-     On iterations that store the slab and do not evaluate the ELBO the dense kernel itself (k_dense_sc: in fp32, from
-     one 16/32-byte record per tie (u_rec) and the per-node table, no entry list, no fp64 transcendental) evaluates
-     these ties -- posterior into the slab and rho_u32, (posterior - closed form) into the fixed-point per-reporter corrections, the
+     On iterations that do not evaluate the ELBO the dense kernel itself (k_dense_sc: in fp32, from one 16/32-byte
+     record per tie (u_rec) and the per-node table, no entry list, no fp64 transcendental) evaluates these ties --
+     posterior into rho_u32 (and the slab, if stored), (posterior - closed form) into the fixed-point per-reporter corrections, the
      SINGLE ties' part of the nu statistic (x z2 sum_k rho_k/(z1_k+z2), model.py:822-825) -- and the fp64 special-tie
      kernel only visits the others (`cx_idx`, `cx_*`); every other iteration runs the special-tie kernel over all special
      ties in fp64, as does any layer for which k_phi_finish cannot rule out a completely underflowed tie or an fp32 range
@@ -238,7 +237,7 @@ typedef struct vm_ctx {
   float* rho_u32;           /* [U*K] fp32 posterior of the special ties: patch source of the dense slab and what the gamma /
                                phi passes gather (written by the special-tie kernel and by the shortcut-tie kernel) */
   double* delta_u;          /* [U*K] rho_u - formula value */
-  float* rho;               /* [L*nloc*N*K] dense posterior slab, or NULL: then every iteration must pass VM_F_NO_SLAB,
+  float* rho;               /* [L*nloc*N*K] dense posterior slab, or NULL: then every iteration must pass VM_F_NO_STORE,
                                and the entry points that read or write the slab return VM_EINVAL */
 
   /* ---- workspaces ---- */
@@ -289,8 +288,9 @@ int vm_phase_phi(const vm_ctx* c, void* stream);
 
 /* Phase 3 -- finishes `_update_phi` (model.py:729-761) from red2 and A, then `_update_rho` +
  * `_sp_uttkrp_rho` (model.py:763-818, 889-923) for every owned tie: special ties in fp64, all ties by
- * the per-tie dense kernel (writes the fp32 slab unless VM_F_NO_STORE), and this rank's share of the
- * statistics of the NEW rho into red3: A, the nu sum (model.py:820-830) and, with VM_F_ELBO, the ELBO sums. */
+ * the per-tie dense kernel (writes the fp32 slab unless VM_F_NO_STORE; the statistics are the same bits either way),
+ * and this rank's share of the statistics of the NEW rho into red3: A, the nu sum (model.py:820-830) and, with
+ * VM_F_ELBO, the ELBO sums. */
 int vm_phase_rho(const vm_ctx* c, int flags, void* stream);
 
 /* Measurement hook: launches ONLY the per-tie dense kernel of phase 3 (tables and special ties as left by the last
@@ -311,8 +311,8 @@ int vm_run(const vm_ctx* c, int n_iter, int flags, int last_flags, void* stream)
 /* Writes rho = pr_rho into the dense slab (one-hot + special ties), model.py:602. */
 int vm_materialize_prior(const vm_ctx* c, void* stream);
 
-/* The posterior the last rho update left (the implicit one of a VM_F_NO_SLAB fit, or the slab's own values), for the
- * local rows [lrow0, lrow0+nrows), lrow = l*nloc + (i-row0), into `out` (float32 [nrows][N][K], the slab's layout):
+/* The posterior the last rho update left (the implicit one of a VM_F_NO_STORE iteration, or the slab's own values), for
+ * the local rows [lrow0, lrow0+nrows), lrow = l*nloc + (i-row0), into `out` (float32 [nrows][N][K], the slab's layout):
  * bit-identical to what a storing iteration writes into those rows of the slab.  Reads tab_p, tab_q, layer_consts,
  * utile_ptr, u_col and rho_u32 only; VM_ENOTSUP under the general mask (VM_R_CSR). */
 int vm_materialize_rows(const vm_ctx* c, int64_t lrow0, int64_t nrows, float* out, void* stream);

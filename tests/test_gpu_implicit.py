@@ -17,8 +17,9 @@ pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def _pair(subs, vals, L, N, M, K, mask, mutuality=True, tile_h=64, may_dead=False, seed=3):
-    """Two engines over the same packed data and initial state: one with the slab, one without."""
+def _pair(subs, vals, L, N, M, K, mask, mutuality=True, tile_h=64, may_dead=False, seed=3, slabs=(True, False)):
+    """Engines over the same packed data and initial state, with the slab or without it as `slabs` says (default: one
+    with, one without), then the packed data."""
     torch = _cuda()
     from vimure_b200 import _packing
     from vimure_b200._engine import CaviEngine
@@ -34,13 +35,13 @@ def _pair(subs, vals, L, N, M, K, mask, mutuality=True, tile_h=64, may_dead=Fals
     pr_u[keep] = pr / pr.sum(axis=1)[:, None]
     nu_rte = PRIORS["beta_eta"] + float(np.asarray(vals).sum()) if mutuality else 1.0
     engs = []
-    for slab in (True, False):
+    for slab in slabs:
         e = CaviEngine(P, PRIORS, mutuality=mutuality, eps=1e-12, may_dead=may_dead, slab=slab)
         e.set_state(st["gamma_shp"], st["gamma_rte"], st["phi_shp"], st["phi_rte"], st["nu_shp"] if mutuality else 1e-6,
                     nu_rte, pr_u, 1e-12)
         engs.append(e)
     torch.cuda.synchronize()
-    return engs[0], engs[1], P
+    return (*engs, P)
 
 
 def _sbm(N, K=2, mutuality=0.5, L=1):
@@ -88,12 +89,16 @@ def _case(name):
 
 CASES = ["ego_k2_partial_tile", "hub_tile_h32", "gm_n640_l2_k3", "all_reporters_k_all32", "may_dead", "no_mutuality"]
 
+# every buffer an iteration leaves behind besides the posterior
+STATE = ("gamma_shp", "gamma_rte", "phi_shp", "phi_rte", "nu", "red3", "elbo_out", "rho_u32", "fixA", "fixP")
+
 
 @pytest.mark.parametrize("name", CASES)
 def test_engine_without_slab_is_bit_identical(name):
+    """Without a slab (imp), and with one that only the last iteration of each step stores (nst)."""
     torch = _cuda()
     kw = _case(name)
-    ref, imp, P = _pair(**kw)
+    ref, imp, nst, P = _pair(**kw, slabs=(True, False, True))
     L, N, K, nloc = P.L, P.N, P.K, P.nloc
     assert ref.rho is not None and imp.rho is None and imp.ctx.rho is None
     if name == "all_reporters_k_all32":
@@ -106,9 +111,11 @@ def test_engine_without_slab_is_bit_identical(name):
     for step, (n, elbo) in enumerate(((1, False), (2, False), (1, True), (3, False), (1, True))):
         for e in (ref, imp):
             e.iterate(n, elbo_last=elbo)
+        nst.iterate(n, elbo_last=elbo, store=False, store_last=True)
         tag = f"{name} step {step}"
-        for k in ("gamma_shp", "gamma_rte", "phi_shp", "phi_rte", "nu", "red3", "elbo_out", "rho_u32", "fixA", "fixP"):
+        for k in STATE:
             assert torch.equal(getattr(ref, k), getattr(imp, k)), f"{k}: {tag}"
+            assert torch.equal(getattr(ref, k), getattr(nst, k)), f"{k}: {tag}, store=False"
         slab = ref.rho_slab().view(L * nloc, N, K)
         for blk in (7, 64, L * nloc):
             for a in range(0, L * nloc, blk):
@@ -120,6 +127,16 @@ def test_engine_without_slab_is_bit_identical(name):
         assert torch.equal(imp.infer(1, 0.3), ref.infer(1, 0.3)), tag
         assert torch.equal(imp.infer_mean(), ref.infer_mean()), tag
         assert torch.equal(imp.sample(5, seed=11 + step), ref.sample(5, seed=11 + step)), tag
+        assert torch.equal(nst.rho_slab(), ref.rho_slab()), tag
+    # an iteration that stores nothing leaves the slab stale and the posterior implicit
+    for e in (ref, imp):
+        e.iterate(1)
+    nst.iterate(1, store=False, store_last=False)
+    for k in STATE:
+        assert torch.equal(getattr(ref, k), getattr(nst, k)), f"{k}: {name}, store_last=False"
+    with pytest.raises(RuntimeError, match="not stored"):
+        nst.rho_slab()
+    assert torch.equal(nst.materialize_rows(0, L * nloc), ref.rho_slab().view(L * nloc, N, K)), name
     # a copy of the implicit posterior (what a fit keeps of an earlier restart) still reads as it did
     snap, before = imp.snapshot(), ref.rho_slab().clone()
     for e in (ref, imp):
@@ -145,7 +162,7 @@ def test_entry_points_that_need_a_slab_refuse_without_one():
     assert lib.vm_materialize_prior(imp._cref, st) == F["VM_EINVAL"]
     assert lib.vm_dense_only(imp._cref, 0, st) == F["VM_EINVAL"]
     assert lib.vm_iteration(imp._cref, 0, st) == F["VM_EINVAL"]
-    assert lib.vm_run(imp._cref, 2, F["VM_F_NO_SLAB"], 0, st) == F["VM_EINVAL"]
+    assert lib.vm_run(imp._cref, 2, F["VM_F_NO_STORE"], 0, st) == F["VM_EINVAL"]
     assert lib.vm_phase_rho(imp._cref, F["VM_F_ELBO"], st) == F["VM_EINVAL"]
     assert lib.vm_materialize_rows(imp._cref, 0, P.L * P.nloc + 1, ctypes.c_void_p(out.data_ptr()), st) == F["VM_EINVAL"]
     torch.cuda.synchronize()
@@ -153,7 +170,7 @@ def test_entry_points_that_need_a_slab_refuse_without_one():
     ref.iterate(1, elbo_last=True)
     imp.iterate(1, elbo_last=True)
     assert torch.equal(ref.gamma_shp, imp.gamma_shp) and torch.equal(ref.red3, imp.red3)
-    assert _capi.consts()["VM_ABI_VERSION"] == 16
+    assert _capi.consts()["VM_ABI_VERSION"] == 17
 
 
 def _fit(g, X, R, **kw):
@@ -211,6 +228,8 @@ def test_fit_without_slab_is_bit_identical():
         if not conc:
             assert isinstance(imp._rho_f_dev, dict)  # the restart's tables, not a slab
         _assert_fits_identical(ref, imp)
+        _assert_fits_identical(ref, _fit(g, X, R, num_realisations=2, max_iter=40, seed=seed,
+                                         concurrent_realisations=conc, store_rho=False))
 
     g = Golden("karnataka_vil1")
     X, R = build_inputs(g)
@@ -218,20 +237,31 @@ def test_fit_without_slab_is_bit_identical():
     b = _fit(g, X, R, init_state=g.init_state(), store_rho="never")
     assert b._engine.rho is None
     _assert_fits_identical(a, b)
+    _assert_fits_identical(a, _fit(g, X, R, init_state=g.init_state(), store_rho=False))
 
 
 def test_general_mask_without_slab_raises():
-    _cuda()
+    torch = _cuda()
     from tests.golden_util import Golden
-    from tests.test_gpu_parity import build_inputs
+    from tests.test_gpu_parity import build_inputs, make_engine
 
     g = Golden("custom_mask")
     assert g.R_spec["kind"] == "coo"
     X, R = build_inputs(g)
-    with pytest.raises(ValueError, match="store_rho"):
-        _fit(g, X, R, store_rho="never", max_iter=3)
-    with pytest.raises(ValueError, match="store_rho"):
-        _fit(g, X, R, store_rho="sometimes", max_iter=3)
+    for store in ("never", False, "sometimes"):
+        with pytest.raises(ValueError, match="store_rho"):
+            _fit(g, X, R, store_rho=store, max_iter=3)
+    # the C ABI refuses an iteration without the slab write before any phase has changed the state
+    csr, _ = make_engine(g, structured=False)
+    assert csr.P.r_mode == 2 and csr.rho is not None
+    csr.iterate(1, elbo_last=True)
+    before = {k: getattr(csr, k).clone() for k in ("gamma_shp", "red3", "rho_u32")}
+    lib, st, F = csr.lib, csr._stream(), csr.C
+    assert lib.vm_iteration(csr._cref, F["VM_F_NO_STORE"], st) == F["VM_ENOTSUP"]
+    assert lib.vm_phase_rho(csr._cref, F["VM_F_NO_STORE"], st) == F["VM_ENOTSUP"]
+    torch.cuda.synchronize()
+    for k, v in before.items():
+        assert torch.equal(getattr(csr, k), v), k
 
 
 def _free_port():
@@ -259,16 +289,18 @@ def _dist_worker(rank, world, port, out):
         g = Golden("sbm_n520")  # N >= 512: the fast dense kernels and a partial column tile on every rank
         X, R = build_inputs(g)
         fits = [_fit(g, X, R, init_state=g.init_state(), max_iter=12, convergence_tol=0.0, **kw)
-                for kw in ({}, {"store_rho": "never"})]
-        a, b = fits
-        res["world"] = b._world
-        res["no_slab"] = b._engine.rho is None
-        res["params"] = all(np.array_equal(getattr(a, k), getattr(b, k)) for k in
-                            ("gamma_shp", "gamma_rte", "phi_shp", "phi_rte", "nu_shp")) and a.maxL == b.maxL
-        res["rho_max"] = bool(np.array_equal(a.get_inferred_model("rho_max"), b.get_inferred_model("rho_max")))
-        res["sample"] = bool(np.array_equal(a.sample_inferred_model(N=2, seed=4, rng="device")[1],
-                                            b.sample_inferred_model(N=2, seed=4, rng="device")[1]))
-        res["rho"] = bool(np.array_equal(a.rho, b.rho))
+                for kw in ({}, {"store_rho": "never"}, {"store_rho": False})]
+        a = fits[0]
+        res["world"] = fits[1]._world
+        res["no_slab"] = fits[1]._engine.rho is None
+        for b, tag in zip(fits[1:], ("never", "no_store")):
+            res[tag] = dict(
+                params=all(np.array_equal(getattr(a, k), getattr(b, k)) for k in
+                           ("gamma_shp", "gamma_rte", "phi_shp", "phi_rte", "nu_shp")) and a.maxL == b.maxL,
+                rho_max=bool(np.array_equal(a.get_inferred_model("rho_max"), b.get_inferred_model("rho_max"))),
+                sample=bool(np.array_equal(a.sample_inferred_model(N=2, seed=4, rng="device")[1],
+                                           b.sample_inferred_model(N=2, seed=4, rng="device")[1])),
+                rho=bool(np.array_equal(a.rho, b.rho)))
         res["ok"] = True
     except Exception:  # noqa: BLE001
         import traceback
@@ -297,7 +329,8 @@ def test_two_rank_fit_without_slab_is_bit_identical():
         res = results[rank]
         assert res["ok"], res.get("error")
         assert res["world"] == world and res["no_slab"], res
-        assert res["params"] and res["rho_max"] and res["sample"] and res["rho"], res
+        for tag in ("never", "no_store"):
+            assert set(res[tag]) == {"params", "rho_max", "sample", "rho"} and all(res[tag].values()), (tag, res)
     del torch
 
 

@@ -1,9 +1,10 @@
 """Host-side driver of the CUDA CAVI kernels: owns the device buffers (PyTorch tensors = plumbing),
 fills the `vm_ctx` of include/vimure_b200.h and calls the extern "C" launchers.
 
-One engine = one rank's shard (node-row block) of one fit.  With `slab=False` it holds no dense posterior slab: every
-iteration runs with VM_F_NO_SLAB, the posterior stays implicit in the row/column tables and the special ties' rho_u32,
-and the consumers evaluate it block by block (`vm_materialize_rows`) -- bit-identical to a fit that stores the slab.  With `group` set, the three statistics vectors
+One engine = one rank's shard (node-row block) of one fit.  An iteration that does not store the slab (VM_F_NO_STORE)
+leaves the posterior implicit in the row/column tables and the special ties' rho_u32, bit-identical to what a storing
+one writes.  With `slab=False` the engine holds no dense posterior slab: every iteration runs so, and the consumers
+evaluate the posterior block by block (`vm_materialize_rows`).  With `group` set, the three statistics vectors
 (red1: gamma-shape sums, red2: phi-shape sums, red3: A + nu + ELBO sums) are all-reduced with
 torch.distributed (NCCL over NVLink on the GPU box) between the phases -- the only exchange the path needs
 (SURVEY.md section 8e).  There is no CPU fallback: without CUDA the constructor raises.
@@ -157,7 +158,6 @@ class CaviEngine:
                      "elbo_out", "u_rec", "nodetab", "fixP", "simple_consts", "cx_logpr", "gfpart", "u_lo"):
             setattr(c, name, ptr(getattr(self, name)))
         c.rho = ptr(self.rho) if self.slab else None
-        self._nsl = 0 if self.slab else self.C["VM_F_NO_SLAB"]  # flag of every rho update
         c.A = self.red3.data_ptr()  # A aliases the (all-reduced) statistics vector
         c.ev_fork, c.ev_join = self._ev_fork.cuda_event, self._ev_join.cuda_event
         self._cref = ctypes.byref(c)
@@ -179,15 +179,14 @@ class CaviEngine:
         [dense_fast], dense, [col_reduce], stats, [elbo_b], sums_reduce | finish: [elbo_partial], finish."""
         P = self.P
         csr, ego = P.r_mode == 2, P.r_mode == 0
-        fast = (P.K <= 4 and (store or not self.slab) and not csr and (P.N * P.K) % 4 == 0 and P.N >= P.tile_w
-                and P.tile_h <= 128)
+        fast = P.K <= 4 and not csr and (P.N * P.K) % 4 == 0 and P.N >= P.tile_w and P.tile_h <= 128
         n = 2 + 3 + 1 + (0 if csr else 1) + 1 + (1 if fast else 0) + 1 + (1 if ego else 0) + 1 + 2 + 1
         if elbo:
             n += 1 + (1 if self.mutuality else 0)
         elif self.simple_mode and fast:
             # the special-tie kernel is launched twice (layers that take the shortcut / that cannot) + k_patch_rest, which
-            # only a slab needs
-            n += 2 if self.slab else 1
+            # only a stored slab needs
+            n += 2 if store else 1
         elif self.all32_mode:
             n += 1  # k_all32 + the fp64 special-tie kernel for the layers whose guard fails
         return n
@@ -249,14 +248,20 @@ class CaviEngine:
         self.rho_is_prior = True
 
     # ------------------------------------------------------------------ iterations
+    def _flags(self, store=True, elbo=False):
+        """vm_* flags of an iteration that stores the slab if `store` (an engine without a slab never does) and
+        evaluates the ELBO if `elbo`."""
+        F = self.C
+        return (0 if store and self.slab else F["VM_F_NO_STORE"]) | (F["VM_F_ELBO"] if elbo else 0)
+
     def iterate(self, n=1, elbo_last=False, store=True, store_last=True):
-        """Run n CAVI iterations; the last one also evaluates the ELBO if `elbo_last`.
+        """Run n CAVI iterations; the last one also evaluates the ELBO if `elbo_last`.  Only the iterations with `store`
+        (the last one: `store or store_last`) write the slab; every statistic is the same either way.
         Returns nothing; read `elbo()` after an ELBO iteration (one D2H scalar)."""
         if n <= 0:
             return
-        F = self.C
-        base = (0 if store else F["VM_F_NO_STORE"]) | self._nsl
-        last = (0 if (store or store_last) else F["VM_F_NO_STORE"]) | (F["VM_F_ELBO"] if elbo_last else 0) | self._nsl
+        nost = self.C["VM_F_NO_STORE"]
+        base, last = self._flags(store), self._flags(store or store_last, elbo_last)
         st = self._stream()
         if self._graphs is not None:
             for it in range(n):
@@ -266,9 +271,9 @@ class CaviEngine:
         else:
             for it in range(n):
                 self._sharded_iteration(last if it == n - 1 else base)
-        self.n_launch += (n - 1) * self.kernels_per_iteration(False, store) + \
-            self.kernels_per_iteration(elbo_last, store or store_last)
-        self.rho_valid = bool(store or store_last) and self.slab
+        self.n_launch += (n - 1) * self.kernels_per_iteration(False, not (base & nost)) + \
+            self.kernels_per_iteration(elbo_last, not (last & nost))
+        self.rho_valid = not (last & nost)
         self.rho_is_prior = False
 
     def _sharded_iteration(self, flags):
@@ -300,8 +305,7 @@ class CaviEngine:
         """Capture the graphs `iterate(..., elbo_last=True, store=store, store_last=True)` replays, up front (a capture
         synchronises the device: do it before several engines start to run side by side on their own streams)."""
         if self._graphs is not None:
-            F = self.C
-            for flags in ((0 if store else F["VM_F_NO_STORE"]) | self._nsl, F["VM_F_ELBO"] | self._nsl):
+            for flags in (self._flags(store), self._flags(elbo=True)):
                 self._graph(flags)
 
     def _graph(self, flags):
@@ -340,17 +344,18 @@ class CaviEngine:
     def phase(self, name, flags=0):
         st = self._stream()
         fn = getattr(self.lib, "vm_phase_" + name)
+        flags = int(flags) | self._flags()
         if name in ("rho", "finish"):
-            _capi.check(fn(self._cref, int(flags) | self._nsl, st), "vm_phase_" + name)
+            _capi.check(fn(self._cref, flags, st), "vm_phase_" + name)
         else:
             _capi.check(fn(self._cref, st), "vm_phase_" + name)
         if name == "rho":
-            self.rho_valid = self.slab and not (flags & self.C["VM_F_NO_STORE"])
+            self.rho_valid = not (flags & self.C["VM_F_NO_STORE"])
             self.rho_is_prior = False
 
     def dense_only(self, flags=0):
         """Launch only the per-tie dense kernel (measurement hook, see vm_dense_only)."""
-        _capi.check(self.lib.vm_dense_only(self._cref, int(flags) | self._nsl, self._stream()), "vm_dense_only")
+        _capi.check(self.lib.vm_dense_only(self._cref, int(flags) | self._flags(), self._stream()), "vm_dense_only")
         self.n_launch += 1
 
     def elbo(self):

@@ -1188,9 +1188,9 @@ __global__ void __launch_bounds__(VM_DENSE_THREADS) k_dense(const __grid_constan
 }
 
 // ---- fast (TMA) dense kernels: tile limit ---------------------------------------------------------------------------
-// Same tiling and warp-autonomous structure as k_dense, for the common case: separable mask (ego / all), slab stored,
-// K <= 4, N*K % 4 == 0, column tile entirely inside the matrix, and no row of the layer can underflow completely
-// (checked on the device; k_dense handles every tile they skip).  ~10 instructions per tie, branch-free chunk loop.
+// Same tiling and warp-autonomous structure as k_dense, for the common case: separable mask (ego / all), K <= 4,
+// N*K % 4 == 0, column tile entirely inside the matrix, and no row of the layer can underflow completely (checked on
+// the device; k_dense handles every tile they skip).  ~10 instructions per tie, branch-free chunk loop.
 #define VM_FAST_MAX_TILE_H 128
 
 // ---- TMA dense kernel ------------------------------------------------------------------------------------------------
@@ -1211,9 +1211,9 @@ __global__ void __launch_bounds__(VM_DENSE_THREADS) k_dense(const __grid_constan
 // keeps its closed form here; k_patch_rest copies their rho_u32 into the slab once the special-tie kernel, which runs
 // next to this one, has written it.  The dense partials only ever count the closed form, so nothing else waits for it.
 //
-// STORE = false (VM_F_NO_SLAB: the rank has no slab): statistics only -- no stage, no bulk store, no patch loads.  The
-// SC variant still evaluates the shortcut ties (rho_u32, fixA, fixP, nu); the closed form their correction subtracts is
-// recomputed with vm_formula_rho, which gives the very bits the chunk loop counted.
+// STORE = false (VM_F_NO_STORE: the iteration writes no slab): statistics only -- no stage, no bulk store, no patch
+// loads.  The SC variant still evaluates the shortcut ties (rho_u32, fixA, fixP, nu); the closed form their correction
+// subtracts is recomputed with vm_formula_rho, which gives the very bits the chunk loop counted.
 __device__ __forceinline__ void vm_bulk_store(void* gdst, const void* ssrc, uint32_t bytes) {
   asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(gdst),
                "r"((uint32_t)__cvta_generic_to_shared(ssrc)), "r"(bytes)
@@ -1244,7 +1244,7 @@ __device__ __forceinline__ unsigned long long vm_smem_split_value(const unsigned
 template <int K, bool SC = false, bool STORE = true>
 struct TmaSmem {
   static constexpr int TW = DenseCfg<K>::TW, NW = VM_DENSE_THREADS / 32, TH = VM_FAST_MAX_TILE_H;
-  // row-segment stages (slab layout), 128-byte aligned (first member); a placeholder without a slab
+  // row-segment stages (slab layout), 128-byte aligned (first member); a placeholder if nothing is stored
   float rowbuf[STORE ? NW : 1][STORE ? VM_TMA_NBUF : 1][STORE ? TW * K : 4];
   float qs[K - 1][TW];                    // column terms of the log2-odds
   union {
@@ -2555,10 +2555,10 @@ static inline double* region_b(const vm_ctx* c) { return region_cat(c) + n_catpa
 static inline double* region_ep(const vm_ctx* c) { return region_b(c) + VM_B_BLOCKS; }
 static inline double* region_s1(const vm_ctx* c) { return region_ep(c) + 2 * VM_EP_BLOCKS; }  // L*VM_S1_BLOCKS*(3+K)
 
-// an entry point that writes or reads the dense slab needs one: only VM_F_NO_SLAB iterations run without (vm_ctx.rho =
+// an entry point that writes or reads the dense slab needs one: only VM_F_NO_STORE iterations run without (vm_ctx.rho =
 // NULL), and not under the general mask, whose statistics gather the slab
 static int slab_check(const vm_ctx* c, int flags) {
-  if (!(flags & VM_F_NO_SLAB)) return c->rho != nullptr ? 0 : VM_EINVAL;
+  if (!(flags & VM_F_NO_STORE)) return c->rho != nullptr ? 0 : VM_EINVAL;
   return c->r_mode == VM_R_CSR ? VM_ENOTSUP : 0;
 }
 
@@ -2586,14 +2586,14 @@ static int check_ctx(const vm_ctx* c) {
 
 // does this rho update use the fast dense kernel (for the tiles that qualify on the device)?
 template <int K>
-static bool dense_fast_eligible(const vm_ctx* c, int flags) {
-  return K <= 4 && !(flags & VM_F_NO_STORE) && c->r_mode != VM_R_CSR && ((c->N * K) & 3) == 0 && c->N >= c->tile_w &&
+static bool dense_fast_eligible(const vm_ctx* c) {
+  return K <= 4 && c->r_mode != VM_R_CSR && ((c->N * K) & 3) == 0 && c->N >= c->tile_w &&
          c->tile_h <= VM_FAST_MAX_TILE_H;
 }
 // ... and do the fast dense kernel / the list mode of the special-tie kernel handle the simple special ties in it?
 template <int K>
 static bool simple_iteration(const vm_ctx* c, int flags) {
-  return c->simple_mode != 0 && c->r_mode == VM_R_EGO && !(flags & VM_F_ELBO) && dense_fast_eligible<K>(c, flags);
+  return c->simple_mode != 0 && c->r_mode == VM_R_EGO && !(flags & VM_F_ELBO) && dense_fast_eligible<K>(c);
 }
 
 // dynamic shared memory of the TMA dense kernels (opt-in above 48 KB)
@@ -2625,20 +2625,34 @@ static void launch_listed(const vm_ctx* c, cudaStream_t s) {
   }
 }
 
+// the TMA dense kernel of one rho update: k_dense_sc on the iterations whose shortcut ties it evaluates (`sc`), else
+// k_dense_tma.  STORE = false (VM_F_NO_STORE): their statistics-only variants, which need no shared-memory opt-in.
+template <int K, bool STORE>
+static void launch_tma(const vm_ctx* c, bool sc, bool elbo, dim3 grid, cudaStream_t st, int rt0, int rtn) {
+  if constexpr (K <= 4) {
+    static_assert(sizeof(TmaSmem<K, true, false>) <= 48 * 1024, "no opt-in for the statistics-only kernels");
+    constexpr size_t smem = sizeof(TmaSmem<K, false, STORE>), smem_sc = sizeof(TmaSmem<K, true, STORE>);
+    double* cp = region_cat(c);
+    if (sc) k_dense_sc<K, 1, STORE><<<grid, VM_DENSE_THREADS, smem_sc, st>>>(*c, rt0, rtn);
+    else if (elbo) k_dense_tma<K, true, VM_TMA_PD, STORE><<<grid, VM_DENSE_THREADS, smem, st>>>(*c, cp, rt0, rtn);
+    else k_dense_tma<K, false, VM_TMA_PD, STORE><<<grid, VM_DENSE_THREADS, smem, st>>>(*c, cp, rt0, rtn);
+  }
+}
+
 // `sums_flags` >= 0: the scalar-sum kernels that only depend on the special-tie kernels (k_elbo_b, k_sums_stage1) also go
 // to the aux stream, under the dense kernel; *sums_done tells the caller whether they were launched here.
 // `sc` (simple_iteration): the dense kernel is k_dense_sc, and the list-mode special-tie kernels are launched here, on the
-// aux stream ahead of the sums and the partial tiles, so that they run under it; k_patch_rest follows the join.
+// aux stream ahead of the sums and the partial tiles, so that they run under it; k_patch_rest follows the join when the
+// iteration stores the slab.
 template <int K>
 static int launch_dense(const vm_ctx* c, int flags, cudaStream_t st, int rt0, int rtn, int sums_flags = -1,
                         bool* sums_done = nullptr, bool sc = false) {
   if (sums_done) *sums_done = false;
   if (rtn <= 0) return 0;
   const dim3 grid((unsigned)c->nct, (unsigned)(c->L * rtn));
-  const bool elbo = flags & VM_F_ELBO, store = !(flags & (VM_F_NO_STORE | VM_F_NO_SLAB)), csr = c->r_mode == VM_R_CSR;
-  const bool noslab = flags & VM_F_NO_SLAB;
+  const bool elbo = flags & VM_F_ELBO, store = !(flags & VM_F_NO_STORE), csr = c->r_mode == VM_R_CSR;
   double* cp = region_cat(c);
-  const bool fast = dense_fast_eligible<K>(c, flags);
+  const bool fast = dense_fast_eligible<K>(c);
   if (fast) {
     const cudaError_t e = fast_setup_all<K>();
     if (e != cudaSuccess) return (int)e;
@@ -2675,26 +2689,14 @@ static int launch_dense(const vm_ctx* c, int flags, cudaStream_t st, int rt0, in
   } else if (sc) {
     launch_listed<K>(c, st);
   }
-#define LF()                                                                                                             \
-  do {                                                                                                                   \
-    if constexpr (K <= 4) {                                                                                              \
-      static_assert(sizeof(TmaSmem<K, true, false>) <= 48 * 1024, "no opt-in for the statistics-only kernels");          \
-      if (noslab && sc) k_dense_sc<K, 1, false><<<grid, VM_DENSE_THREADS, sizeof(TmaSmem<K, true, false>), st>>>(*c, rt0, rtn); \
-      else if (noslab && elbo)                                                                                           \
-        k_dense_tma<K, true, VM_TMA_PD, false><<<grid, VM_DENSE_THREADS, sizeof(TmaSmem<K, false, false>), st>>>(*c, cp, rt0, rtn); \
-      else if (noslab)                                                                                                   \
-        k_dense_tma<K, false, VM_TMA_PD, false><<<grid, VM_DENSE_THREADS, sizeof(TmaSmem<K, false, false>), st>>>(*c, cp, rt0, rtn); \
-      else if (sc) k_dense_sc<K><<<grid, VM_DENSE_THREADS, sizeof(TmaSmem<K, true>), st>>>(*c, rt0, rtn);                 \
-      else if (elbo) k_dense_tma<K, true><<<grid, VM_DENSE_THREADS, sizeof(TmaSmem<K>), st>>>(*c, cp, rt0, rtn);          \
-      else k_dense_tma<K, false><<<grid, VM_DENSE_THREADS, sizeof(TmaSmem<K>), st>>>(*c, cp, rt0, rtn);                   \
-    }                                                                                                                    \
-  } while (0)
-  if (fast && !side) LF();
-  int rc = 0;
+  const auto launch_fast = [&] {
+    if (store) launch_tma<K, true>(c, sc, elbo, grid, st, rt0, rtn);
+    else launch_tma<K, false>(c, sc, elbo, grid, st, rt0, rtn);
+  };
+  if (fast && !side) launch_fast();
 #define LD(E, S, C) k_dense<K, E, S, C><<<grid, VM_DENSE_THREADS, 0, sg>>>(*c, cp, fast ? 1 : 0, rt0, rtn)
-  if (csr) {
-    if (!store) rc = VM_ENOTSUP;  // the general-mask statistics gather the slab
-    else if (elbo) LD(true, true, true); else LD(false, true, true);
+  if (csr) {  // always stores (slab_check)
+    if (elbo) LD(true, true, true); else LD(false, true, true);
   } else if (elbo) {
     if (store) LD(true, true, false); else LD(true, false, false);
   } else {
@@ -2702,7 +2704,7 @@ static int launch_dense(const vm_ctx* c, int flags, cudaStream_t st, int rt0, in
   }
 #undef LD
   if (side) {
-    LF();
+    launch_fast();
     cudaEventRecord(ev_join, aux);
     cudaStreamWaitEvent(st, ev_join, 0);
     if (own_events) {
@@ -2710,14 +2712,13 @@ static int launch_dense(const vm_ctx* c, int flags, cudaStream_t st, int rt0, in
       cudaEventDestroy(ev_join);
     }
   }
-#undef LF
   if constexpr (K <= 4) {
-    if (sc && !noslab && c->n_ublk > 0) {
+    if (sc && store && c->n_ublk > 0) {
       const dim3 gridp((unsigned)imin64(c->n_ublk * (VM_SPECIAL_TIES_PER_BLOCK / 256), 148 * 8), (unsigned)c->L);
       k_patch_rest<K><<<gridp, 256, 0, st>>>(*c);
     }
   }
-  return rc;
+  return 0;
 }
 
 template <int K>

@@ -31,9 +31,10 @@ Extra, optional `fit` keywords (a superset of the reference's):
                  False -- write it at the ELBO iterations only (the other iterations run statistics-only kernels);
                  "never" -- never allocate it: the posterior stays implicit in O(N) row/column tables and the special
                  ties' posteriors, and `rho`, `rho_f`, `get_inferred_model`, `get_posterior_estimates` and
-                 `sample_inferred_model` evaluate it block by block on demand.  Parameters, trace and every output are
-                 bit-identical to the default; it lets a sparse network whose slab exceeds the GPU's memory be fitted.
-                 Needs an ego or all-reporter mask (ValueError otherwise: the general mask's statistics gather the slab).
+                 `sample_inferred_model` evaluate it block by block on demand; it lets a sparse network whose slab
+                 exceeds the GPU's memory be fitted.  With False and "never", parameters, trace and every output are
+                 bit-identical to the default.  Both need an ego or all-reporter mask (ValueError otherwise: the general
+                 mask's statistics gather the slab).
 """
 import os
 import time
@@ -236,10 +237,10 @@ class VimureModel(TransformerMixin, BaseEstimator):
         if isinstance(store_rho, str) and store_rho != "never":
             raise ValueError('store_rho must be True, False or "never"')
         self._slab = not isinstance(store_rho, str)
-        self._store_rho = bool(store_rho) if self._slab else True
-        if not self._slab and self.R.kind not in ("ego", "all"):
-            raise ValueError('store_rho="never" needs an ego or all-reporter mask: the statistics of a general reporter '
-                             'mask gather the dense posterior slab')
+        self._store_rho = self._slab and bool(store_rho)
+        if not self._store_rho and self.R.kind not in ("ego", "all"):
+            raise ValueError('store_rho=%r needs an ego or all-reporter mask: the statistics of a general reporter '
+                             'mask gather the dense posterior slab' % (store_rho,))
 
         # ---- sharding (row blocks over ranks, SURVEY.md section 8e)
         dist_opt = extra_params.get("distributed", "auto")
