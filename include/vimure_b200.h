@@ -364,6 +364,17 @@ int64_t vm_edges_size(void);
 int vm_edges_count(const vm_ctx* c, const vm_edges_args* a, void* stream);
 int vm_edges_emit(const vm_ctx* c, const vm_edges_args* a, void* stream);
 
+/* rho at given ties: out[q*K + k] = posterior of the tie key[q] = (l*N+i)*N+j, for every key of this rank's rows;
+ * the outputs of other keys are not written.  source = VM_EDGES_SLAB (ctx->rho, any mask) or VM_EDGES_IMPLICIT
+ * (what vm_materialize_rows evaluates; VM_ENOTSUP under VM_R_CSR).  Bit for bit the value the slab / vm_materialize_rows
+ * holds for that tie.  n = 0 launches nothing.
+ * One thread per query, in any order, duplicates allowed; a key outside [0, L*N*N) or outside the rows [row0, row0+nloc)
+ * is skipped, so that on a sharded fit every rank answers the keys of its own rows into a zero-filled buffer and one
+ * sum over the ranks combines them exactly.  The implicit source finds a special tie by a binary search of u_col within
+ * its (row, column tile) segment of utile_ptr.  VM_EINVAL before any launch for n < 0, a NULL key / out with n > 0, an
+ * unknown source, or the slab source without a slab. */
+int vm_rho_at(const vm_ctx* c, int64_t source, int64_t n, const int64_t* key, float* out, void* stream);
+
 /* ---- data packing (replaces the data preparation of `__check_fit_params`, model.py:147-176, and utils.py:73-84) --------
  * From the COO list of reports (device arrays) to every packed array `vm_ctx` points to, for one node-row block and a
  * structured reporter mask (VM_R_EGO / VM_R_ALL; a general COO mask is packed by the host-side packer): entries outside

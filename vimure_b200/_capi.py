@@ -159,6 +159,7 @@ def open_library(path):
         "vm_edges_size": (i64, []),
         "vm_edges_count": (i, [P, ctypes.POINTER(edges_class()), vp]),
         "vm_edges_emit": (i, [P, ctypes.POINTER(edges_class()), vp]),
+        "vm_rho_at": (i, [P, i64, i64, vp, vp, vp]),
         "vm_test_special": (i, [vp, vp, vp, i64, vp]),
         "vm_pack_size": (i64, []),
         "vm_pack_workspace_bytes": (i64, [ctypes.POINTER(pack_class())]),

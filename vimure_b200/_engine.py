@@ -494,15 +494,19 @@ class CaviEngine:
         device, this rank's rows."""
         return self._edges(self.C["VM_EDGES_SAMPLE"], slab, n_trials=int(n_trials), seed=int(seed) & (2**64 - 1))
 
+    def _implicit_source(self, slab):
+        """Where the per-tie consumers (`_edges`, `rho_at`) read the posterior: from the tables (implicit source) whenever
+        they describe the posterior being consumed -- this engine's own after an iteration, slab or not, or a `snapshot()`
+        -- and from a slab for a cloned slab of an earlier restart, the prior, and the general mask (which has no tables)."""
+        return not self.slab or (slab is None and not getattr(self, "rho_is_prior", False) and self.P.r_mode != 2)
+
     def _edges(self, what, slab, **kw):
         """One vm_edges_count, the row offsets (one cumsum), one D2H read of the total, one vm_edges_emit.  The posterior is
-        read where it is cheapest to evaluate: from the tables (implicit source) whenever they describe the posterior being
-        consumed -- this engine's own after an iteration, slab or not, or a `snapshot()` -- and from a slab for a cloned
-        slab of an earlier restart, the prior, and the general mask (which has no tables)."""
+        read where it is cheapest to evaluate (`_implicit_source`)."""
         C, P = self.C, self.P
         old = self._use_slab(slab)  # the dense consumers' preconditions (and the prior's slab, when that is the posterior)
         try:
-            implicit = not self.slab or (slab is None and not getattr(self, "rho_is_prior", False) and P.r_mode != 2)
+            implicit = self._implicit_source(slab)
             rows = P.L * P.nloc
             i64 = dict(dtype=torch.int64, device=self.dev)
             off = torch.zeros(rows + 1, **i64)
@@ -520,6 +524,25 @@ class CaviEngine:
             _capi.check(self.lib.vm_edges_emit(self._cref, ctypes.byref(a), st), "vm_edges_emit")
             self.n_launch += 2 + int(implicit)
             return keys[:total], vals[:total]
+        finally:
+            self._restore(old)
+
+    def rho_at(self, keys, slab=None):
+        """The posterior at the ties `keys` (int64 device tensor of global ids (l*N+i)*N+j, any order, duplicates allowed)
+        as the slab holds it: float32 (n, K) on the device (`vm_rho_at`), read from the source `_edges` reads.  Only the
+        keys of this rank's rows are answered; the rows of the others are zero."""
+        if not torch.is_tensor(keys) or keys.dtype != torch.int64 or keys.device != self.dev:
+            raise ValueError("rho_at takes an int64 tensor of tie keys on the engine's device (%s)" % self.dev)
+        keys = keys.reshape(-1).contiguous()
+        old = self._use_slab(slab)
+        try:
+            C, n = self.C, keys.numel()
+            out = torch.zeros(n, self.P.K, dtype=torch.float32, device=self.dev)
+            source = C["VM_EDGES_IMPLICIT"] if self._implicit_source(slab) else C["VM_EDGES_SLAB"]
+            _capi.check(self.lib.vm_rho_at(self._cref, source, n, ctypes.c_void_p(keys.data_ptr()),
+                                           ctypes.c_void_p(out.data_ptr()), self._stream()), "vm_rho_at")
+            self.n_launch += int(n > 0)
+            return out
         finally:
             self._restore(old)
 

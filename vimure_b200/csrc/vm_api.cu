@@ -83,6 +83,9 @@ extern "C" int vm_sample(const vm_ctx* c, int64_t n_trials, uint64_t seed, uint8
 extern "C" int64_t vm_edges_size(void) { return (int64_t)sizeof(vm_edges_args); }
 extern "C" int vm_edges_count(const vm_ctx* c, const vm_edges_args* a, void* stream) { VM_ROUTE(edges(c, a, 0, stream)); }
 extern "C" int vm_edges_emit(const vm_ctx* c, const vm_edges_args* a, void* stream) { VM_ROUTE(edges(c, a, 1, stream)); }
+extern "C" int vm_rho_at(const vm_ctx* c, int64_t source, int64_t n, const int64_t* key, float* out, void* stream) {
+  VM_ROUTE(rho_at(c, source, n, key, out, stream));
+}
 
 __global__ void k_test_special(const double* x, double* dg, double* lg, int64_t n) {
   const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;

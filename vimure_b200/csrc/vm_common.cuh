@@ -30,6 +30,7 @@ struct vm_tu_api {
   int (*infer)(const vm_ctx*, int, double, uint8_t*, void*);
   int (*materialize_rows)(const vm_ctx*, int64_t, int64_t, float*, void*);
   int (*edges)(const vm_ctx*, const vm_edges_args*, int, void*);  // int: 0 = vm_edges_count, 1 = vm_edges_emit
+  int (*rho_at)(const vm_ctx*, int64_t, int64_t, const int64_t*, float*, void*);
 };
 
 // Column tile of the dense kernels: TW = 128*NCH columns; NCH is K-dependent so that the per-lane column accumulators

@@ -2539,6 +2539,49 @@ __global__ void __launch_bounds__(256) k_materialize_rows(const __grid_constant_
   }
 }
 
+// The posterior at given ties (vm_rho_at): one thread per query, grid-stride.  key[q] = (l*N+i)*N+j; a key outside
+// [0, L*N*N) or outside this rank's rows [row0, row0+nloc) is skipped and out[q*K..] is not written.  Implicit source: the
+// special ties of the tie's (row, column tile) segment are sorted by column (at most tile_w of them): a binary search
+// finds the tie there (rho_u32), else the closed form of k_materialize_rows -- the same bits.  Slab source: ctx->rho.
+template <int K>
+__global__ void __launch_bounds__(256) k_rho_at(const __grid_constant__ vm_ctx c, int implicit, int64_t n,
+                                                const int64_t* __restrict__ key, float* __restrict__ out) {
+  const int64_t N = c.N, T = c.L * N * N;
+  for (int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; q < n; q += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t g = key[q];
+    if (g < 0 || g >= T) continue;
+    const int64_t li = g / N, j = g - li * N, l = li / N, i = li - l * N;
+    if (i < c.row0 || i >= c.row0 + c.nloc) continue;
+    const int64_t lrow = l * c.nloc + i - c.row0;
+    float o[K];
+    if (!implicit) {
+#pragma unroll
+      for (int k = 0; k < K; ++k) o[k] = c.rho[(lrow * N + j) * K + k];
+    } else {
+      const int64_t seg = lrow * c.nct + j / c.tile_w;
+      // 64-bit: the indices reach U < 2^31, where lo + hi would overflow an int
+      const int64_t end = c.utile_ptr[seg + 1];
+      int64_t lo = c.utile_ptr[seg], hi = end;
+      while (lo < hi) {
+        const int64_t mid = (lo + hi) >> 1;
+        if (c.u_col[mid] < j) lo = mid + 1;
+        else hi = mid;
+      }
+      if (lo < end && c.u_col[lo] == j) {
+#pragma unroll
+        for (int k = 0; k < K; ++k) o[k] = c.rho_u32[lo * K + k];
+      } else {
+        float a[K], epsr;
+        bool dead;
+        vm_tie_logodds<K>(c, (int)l, lrow, (int)j, a);
+        vm_formula_rho<K>(a, vm_may_dead<K>(c, (int)l), o, epsr, dead);
+      }
+    }
+#pragma unroll
+    for (int k = 0; k < K; ++k) out[q * K + k] = o[k];
+  }
+}
+
 // =====================================================================================================
 // host-side launchers
 // =====================================================================================================
@@ -3000,12 +3043,28 @@ static int tu_edges(const vm_ctx* c, const vm_edges_args* a, int emit, void* str
   return 0;
 }
 
+// vm_rho_at; every argument is checked before anything is launched
+static int tu_rho_at(const vm_ctx* c, int64_t source, int64_t n, const int64_t* key, float* out, void* stream) {
+  int rc = check_ctx(c);
+  if (rc) return rc;
+  if (n < 0 || (n > 0 && (!key || !out))) return VM_EINVAL;
+  if (source != VM_EDGES_SLAB && source != VM_EDGES_IMPLICIT) return VM_EINVAL;
+  const bool implicit = source == VM_EDGES_IMPLICIT;
+  if (!implicit && !c->rho) return VM_EINVAL;
+  if (implicit && c->r_mode == VM_R_CSR) return VM_ENOTSUP;  // no row/column tables (as vm_materialize_rows)
+  if (n == 0) return 0;
+  const unsigned grid = (unsigned)imin64(cdiv(n, 256), 148 * 16);
+  DISPATCH_K(c->K, (k_rho_at<K><<<grid, 256, 0, (cudaStream_t)stream>>>(*c, (int)implicit, n, key, out)));
+  VM_CHECK_LAUNCH();
+  return 0;
+}
+
 }  // namespace
 
 extern "C" const vm_tu_api* VM_PASTE(vm_tu_api_, VM_TU_ID)(void) {
   using namespace VM_PASTE(vmtu, VM_TU_ID);
   static const vm_tu_api api = {tu_materialize_prior, tu_refresh_cache, tu_init_stats, tu_phase_gamma, tu_phase_phi,
                                 tu_phase_rho,         tu_dense_only,    tu_phase_finish, tu_iteration, tu_run, tu_infer,
-                                tu_materialize_rows,  tu_edges};
+                                tu_materialize_rows,  tu_edges,         tu_rho_at};
   return &api;
 }

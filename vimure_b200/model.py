@@ -866,6 +866,38 @@ class VimureModel(TransformerMixin, BaseEstimator):
             return self._consume_edges("infer_edges", dtype, *args)
         return self._consume("infer", *args).astype(dtype)
 
+    def rho_f_at(self, subs):
+        """The posterior rho_f at given ties: subs = (l, i, j), three 1-D integer arrays of equal length (the first three
+        subscripts of an `sptensor`, such as the edges `get_inferred_model(..., sparse=True)` returns) -> float64 (n, K),
+        equal to `rho_f[l, i, j]`.  Evaluated tie by tie on the device (`vm_rho_at`) wherever rho_f lives -- the best
+        restart's engine, a snapshot or a cloned slab (see `_consume`) -- without any N*N-sized buffer: only the keys go to
+        the device and n*K floats come back; the form to ask for on networks whose rho_f does not fit.  On a sharded fit
+        every rank answers the ties of its own rows and one all-reduce combines them (collective: every rank must call with
+        the same subs).  ValueError, before any device work, for anything but three integer arrays of equal length within
+        the shape (L, N, N); empty integer arrays give (0, K)."""
+        if not isinstance(subs, (tuple, list)) or len(subs) != 3:
+            raise ValueError("rho_f_at takes subs = (l, i, j): three 1-D integer arrays")
+        subs = [np.asarray(s) for s in subs]
+        if any(s.ndim != 1 for s in subs) or len({s.size for s in subs}) != 1:
+            raise ValueError("rho_f_at: l, i, j must be 1-D arrays of equal length")
+        if any(not np.issubdtype(s.dtype, np.integer) for s in subs):
+            raise ValueError("rho_f_at: the subscripts must be integer arrays")
+        if subs[0].size == 0:
+            return np.zeros((0, self.K))
+        l, i, j = (s.astype(np.int64) for s in subs)
+        for s, hi, name in ((l, self.L, "l"), (i, self.N, "i"), (j, self.N, "j")):
+            if s.min() < 0 or s.max() >= hi:
+                raise ValueError("rho_f_at: %s out of range [0, %d)" % (name, hi))
+        eng, slab = self._rho_f_source()
+        keys = torch.as_tensor((l * self.N + i) * self.N + j, device=eng.dev)
+        out = eng.rho_at(keys, slab=slab)  # this rank's rows, zeros elsewhere
+        if self._world > 1:
+            # every key belongs to exactly one rank and x + 0 = x: the sum is exact.  NCCL on the device, gloo on the host
+            if torch.distributed.get_backend() != "nccl":
+                out = out.cpu()
+            torch.distributed.all_reduce(out)
+        return out.cpu().numpy().astype(np.float64)
+
     def get_posterior_estimates(self):
         """Posterior estimates nu, theta, lambda, rho (reference model.py:1191-1214)."""
         return {"nu": self.G_exp_nu_f, "theta": self.G_exp_theta_f, "lambda": self.G_exp_lambda_f, "rho": self.rho_f}
