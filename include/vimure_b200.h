@@ -447,6 +447,27 @@ typedef struct vm_synth {
 int64_t vm_synth_size(void);
 int vm_synth_ego(const vm_synth* s, void* stream);
 
+/* The same generator under the other reporter masks.  Every kernel draws reporter m's two counts on the pair {a, b} with
+ * one function of (seed, layer, m, {a, b}), so every mask gives the same count for the same (seed, layer, reporter, pair):
+ * a reporter on the pair (m in {a, b}) draws exactly as vm_synth_ego does, a reporter off the pair draws from a disjoint
+ * part of the counter space.  Self-tie convention: X[l,a,a,m] is drawn for every reporter m the mask allows, with the
+ * self-tie law of vm_synth_ego's (m,m) entries and m's theta -- the reference's report loop visits i == j, and the second
+ * of its two assignments overwrites the first: x ~ Poisson(theta lam_0 + eta Poisson(theta lam_0 / (1-eta))).
+ * Both follow vm_synth_ego's protocol: the node-row block [row0, row0+nloc), emit_transposed, *counter = the number of
+ * entries (only the first `cap` stored), VM_EINVAL before `counter` is touched or anything is launched.
+ *
+ * vm_synth_all: the all-reporter mask (flag_self_reporter=False, R == 1): every reporter m < M reports every ordered pair,
+ * self ties included.  Reporters are not nodes here, so M <= N is not required.
+ * vm_synth_masked: an explicit mask, one entry (l, i, j, m) per position; emits X[l,i,j,m] when positive.  A duplicated
+ * entry is emitted once per occurrence (pass distinct entries); an entry outside (L, N, N, M) is skipped. */
+typedef struct vm_synth_mask {
+  const int32_t *l, *i, *j, *m;  /* [n] device */
+  int64_t n;
+} vm_synth_mask;
+int64_t vm_synth_mask_size(void);
+int vm_synth_all(const vm_synth* s, void* stream);
+int vm_synth_masked(const vm_synth* s, const vm_synth_mask* mask, void* stream);
+
 /* Special functions exposed for testing the device implementations against scipy. */
 int vm_test_special(const double* x, double* out_digamma, double* out_lgamma, int64_t n, void* stream);
 

@@ -52,6 +52,7 @@ def _parse_header():
 
 
 _synth_cls = None
+_synth_mask_cls = None
 _pack_cls = None
 _edges_cls = None
 
@@ -80,6 +81,19 @@ def synth_class():
 
         _synth_cls = VmSynth
     return _synth_cls
+
+
+def synth_mask_class():
+    """ctypes mirror of `vm_synth_mask` (explicit mask of `vm_synth_masked`), generated from the header."""
+    global _synth_mask_cls
+    if _synth_mask_cls is None:
+        fields = _parse_struct(open(HEADER).read(), "vm_synth_mask")
+
+        class VmSynthMask(ctypes.Structure):
+            _fields_ = fields
+
+        _synth_mask_cls = VmSynthMask
+    return _synth_mask_cls
 
 
 def edges_class():
@@ -166,6 +180,9 @@ def open_library(path):
         "vm_pack": (i, [ctypes.POINTER(pack_class()), vp]),
         "vm_synth_size": (i64, []),
         "vm_synth_ego": (i, [ctypes.POINTER(synth_class()), vp]),
+        "vm_synth_all": (i, [ctypes.POINTER(synth_class()), vp]),
+        "vm_synth_mask_size": (i64, []),
+        "vm_synth_masked": (i, [ctypes.POINTER(synth_class()), ctypes.POINTER(synth_mask_class()), vp]),
     }
     for name, (res, args) in protos.items():
         fn = getattr(lib, name)
@@ -178,6 +195,8 @@ def open_library(path):
         raise RuntimeError("vm_pack_args layout mismatch between header and library (stale build?)")
     if lib.vm_synth_size() != ctypes.sizeof(synth_class()):
         raise RuntimeError("vm_synth layout mismatch between header and library (stale build?)")
+    if lib.vm_synth_mask_size() != ctypes.sizeof(synth_mask_class()):
+        raise RuntimeError("vm_synth_mask layout mismatch between header and library (stale build?)")
     if lib.vm_edges_size() != ctypes.sizeof(edges_class()):
         raise RuntimeError("vm_edges_args layout mismatch between header and library (stale build?)")
     if lib.vm_abi_version() != consts()["VM_ABI_VERSION"]:

@@ -15,10 +15,13 @@ Laws
   X (`_build_X` with the self-reporter mask, synthetic.py:138-209): theta_lm ~ Gamma(sh, sc);
       lambda_lij = Y_lij if Y_lij > 0 else 0.01; for reporter m and every pair {m,n} a fair coin picks the first
       direction, first ~ Poisson((th*lam_ab + eta*th*lam_ba)/(1-eta^2)), second ~ Poisson(th*lam_ba + eta*first).
+      The device generators (`device_reports`) draw the same law for any reporter and pair, under the self-reporter,
+      the all-reporter or an explicit mask.
 """
 import numpy as np
 
-from .masks import EgoMask
+from . import masks
+from .masks import AllMask, EgoMask
 from .sptensor import sptensor
 
 LAMBDA_0 = 0.01
@@ -213,33 +216,112 @@ class SparseSyntheticNetwork:
 
     # ------------------------------------------------------------------ X on the device
     def build_X_device(self, mutuality=0.5, sh_theta=2.0, sc_theta=0.5, seed=None, theta=None, device="cuda", row0=0,
-                       nloc=None, emit_transposed=False):
-        """Device-side `build_X` (the `vm_synth_ego` kernels of include/vimure_b200.h): the same law, sampled with a
-        counter-based RNG keyed by (seed, layer, reporter, partner), for the node-row block [row0, row0+nloc) only.
+                       nloc=None, emit_transposed=False, flag_self_reporter=True, Rinput=None):
+        """Device-side `build_X` (the `vm_synth_*` kernels of include/vimure_b200.h): the same law, sampled with a
+        counter-based RNG keyed by (seed, layer, reporter, pair), for the node-row block [row0, row0+nloc) only.
+
+        The mask follows the reference's arguments: `Rinput` (anything `masks.from_input` accepts, or a ReporterMask) when
+        given, else the self-reporter mask (`flag_self_reporter=True`) or the all-reporter mask (False); see
+        `device_reports` for how each is generated.
 
         Returns (subs, vals): int32 tensors (4, n) and (n,) ON THE DEVICE -- the entries X[l,i,j,m] with i in the block and,
         with `emit_transposed`, the reciprocal entries X[l,j,i,m] whose row the block does not own (so that the shard can
         be paired without an exchange).  Every rank that evaluates an entry gets the same value, whatever its block.
-        Also sets self.theta, self.R, self.mutuality (not self.X: use `sptensor(tuple(subs.cpu()), vals.cpu(), ...)`)."""
+        Also sets self.theta, self.R (the EgoMask, AllMask or CooMask used), self.mutuality (not self.X: use
+        `sptensor(tuple(subs.cpu()), vals.cpu(), ...)`)."""
         sd = self.seed if seed is None else seed
         eta = float(mutuality)
         if eta < 0 or eta >= 1:
             raise ValueError("The mutuality parameter has to be in [0, 1)!")
+        R = _report_mask(Rinput, flag_self_reporter, self.L, self.N, self.M)
         if theta is None:
             theta = np.random.RandomState(sd).gamma(shape=sh_theta, scale=sc_theta, size=(self.L, self.M))
         self.theta = theta
         subs, vals = device_reports(self.L, self.N, self.M, self.K, self.Y_subs, self.Y_vals, theta, eta, sd, device=device,
-                                    row0=row0, nloc=nloc, emit_transposed=emit_transposed)
-        self.R = EgoMask(self.L, self.N, self.M, diag=True)
+                                    row0=row0, nloc=nloc, emit_transposed=emit_transposed, mask=R)
+        self.R = R
         self.mutuality = eta
         return subs, vals
 
 
+def _report_mask(Rinput, flag_self_reporter, L, N, M):
+    """The reporter mask of the reference's `build_X(Rinput=..., flag_self_reporter=...)`, as a ReporterMask."""
+    if Rinput is not None:
+        return masks.from_input(Rinput, L, N, M)
+    return EgoMask(L, N, M, diag=True) if flag_self_reporter else AllMask(L, N, M)
+
+
+def _full_ego(R):
+    return isinstance(R, EgoMask) and R.diag and bool(np.all(R.rep))
+
+
 def device_reports(L, N, M, K, Y_subs, Y_vals, theta, eta, seed, lam=None, device="cuda", row0=0, nloc=None,
+                   emit_transposed=False, mask=None):
+    """Reports X for a given ground truth Y (COO), reliabilities theta (L, M), mutuality eta and, optionally, a table lam
+    (L, K) of average interactions per ground-truth category (default: 0.01, 1, 2, ..), sampled on the device
+    (include/vimure_b200.h).  Returns int32 device tensors (subs (4, n), vals (n,)).
+
+    mask: None or a full EgoMask(diag=True) -> `vm_synth_ego`; any other EgoMask -> `vm_synth_ego`, filtered on the
+    device by rep[l, m] and diag; AllMask -> `vm_synth_all`; anything else `masks.from_input` accepts -> `vm_synth_masked`
+    over its distinct entries (`masked_reports`).  Every mask gives the same count for the same (seed, layer, reporter,
+    pair), so a mask's reports are those of a larger mask restricted to its entries."""
+    R = None if mask is None else masks.from_input(mask, L, N, M)
+    args = (L, N, M, K, Y_subs, Y_vals, theta, eta, seed, lam, device, row0, nloc, emit_transposed)
+    if R is None or isinstance(R, EgoMask):
+        subs, vals = _generate("vm_synth_ego", *args)
+        if R is None or _full_ego(R):
+            return subs, vals
+        import torch
+
+        keep = torch.as_tensor(R.rep.astype(bool), device=subs.device)[subs[0].long(), subs[3].long()]
+        if not R.diag:
+            keep &= subs[1] != subs[2]
+        return subs[:, keep], vals[keep]
+    if isinstance(R, AllMask):
+        return _generate("vm_synth_all", *args)
+    sel = R.vals != 0
+    return masked_reports(L, N, M, K, Y_subs, Y_vals, theta, eta, seed, R.subs[:, sel], lam=lam, device=device, row0=row0,
+                          nloc=nloc, emit_transposed=emit_transposed)
+
+
+def masked_reports(L, N, M, K, Y_subs, Y_vals, theta, eta, seed, entries, lam=None, device="cuda", row0=0, nloc=None,
                    emit_transposed=False):
-    """Reports X under the self-reporter mask for a given ground truth Y (COO), reliabilities theta (L, M), mutuality eta
-    and, optionally, a table lam (L, K) of average interactions per ground-truth category (default: 0.01, 1, 2, ..) --
-    sampled on the device by `vm_synth_ego` (include/vimure_b200.h).  Returns int32 device tensors (subs (4, n), vals (n,))."""
+    """Reports X under an explicit mask `entries` (4, n) = (l, i, j, m), duplicates allowed: `vm_synth_masked` over the
+    distinct entries, X[l,i,j,m] = reporter m's i->j count on the pair {i, j} (as every other generator draws it).
+    ValueError, before any device work, for an entry outside (L, N, N, M).  Returns int32 device tensors as
+    `device_reports`."""
+    import torch
+
+    e = np.asarray(entries)
+    if e.ndim != 2 or e.shape[0] != 4:
+        raise ValueError("entries must be (4, n): l, i, j, m")
+    e = e.astype(np.int64)
+    if e.shape[1]:
+        lo, hi = e.min(axis=1), e.max(axis=1)
+        if np.any(lo < 0) or np.any(hi >= np.array([L, N, N, M])):
+            raise ValueError("mask entries outside the shape (L, N, N, M) = (%d, %d, %d, %d)" % (L, N, N, M))
+    if L * N * N * M >= 2 ** 63:
+        raise ValueError("L*N*N*M must stay below 2^63")
+    dev = torch.device(device)
+    if dev.type != "cuda":
+        raise RuntimeError("masked_reports needs a CUDA device")
+    t = torch.from_numpy(np.ascontiguousarray(e)).to(dev)
+    key = torch.unique(((t[0] * N + t[1]) * N + t[2]) * M + t[3])
+    del t
+    rest = torch.div(key, M, rounding_mode="floor")
+    m = (key - rest * M).to(torch.int32)
+    lij = torch.div(rest, N, rounding_mode="floor")
+    j = (rest - lij * N).to(torch.int32)
+    l = torch.div(lij, N, rounding_mode="floor")
+    i = (lij - l * N).to(torch.int32)
+    l = l.to(torch.int32)
+    del key, rest, lij
+    return _generate("vm_synth_masked", L, N, M, K, Y_subs, Y_vals, theta, eta, seed, lam, device, row0, nloc,
+                     emit_transposed, mask=(l, i, j, m))
+
+
+def _generate(entry, L, N, M, K, Y_subs, Y_vals, theta, eta, seed, lam, device, row0, nloc, emit_transposed, mask=None):
+    """One `vm_synth_*` entry point, counted then filled: returns int32 device tensors (subs (4, n), vals (n,))."""
     import ctypes
 
     import torch
@@ -268,31 +350,39 @@ def device_reports(L, N, M, K, Y_subs, Y_vals, theta, eta, seed, lam=None, devic
     S.lam = None if lam_t is None else lam_t.data_ptr()
     S.counter = counter.data_ptr()
     stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+    fn = getattr(lib, entry)
+    extra = ()
+    if mask is not None:
+        Mk = _capi.synth_mask_class()()
+        Mk.l, Mk.i, Mk.j, Mk.m = (int(t.data_ptr()) for t in mask)
+        Mk.n = int(mask[0].numel())
+        extra = (ctypes.byref(Mk),)
     # pass 1 counts (cap = 0: nothing is stored), pass 2 fills arrays of exactly that size
     S.cap = 0
-    _capi.check(lib.vm_synth_ego(ctypes.byref(S), stream), "vm_synth_ego (count)")
+    _capi.check(fn(ctypes.byref(S), *extra, stream), entry + " (count)")
     n = int(counter.item())
     out = torch.empty((5, max(n, 1)), dtype=torch.int32, device=dev)
     S.cap = n
     S.o_l, S.o_i, S.o_j, S.o_m, S.o_x = (out[d].data_ptr() for d in range(5))
-    _capi.check(lib.vm_synth_ego(ctypes.byref(S), stream), "vm_synth_ego (fill)")
+    _capi.check(fn(ctypes.byref(S), *extra, stream), entry + " (fill)")
     if int(counter.item()) != n:
-        raise RuntimeError("vm_synth_ego: the two passes disagree (%d vs %d entries)" % (int(counter.item()), n))
+        raise RuntimeError("%s: the two passes disagree (%d vs %d entries)" % (entry, int(counter.item()), n))
     return out[:4, :n], out[4, :n]
 
 
 class PosteriorSyntheticNetwork:
     """Generates data (Y, X) from the posterior estimates of a fitted model: the counterpart of the reference's
-    `vimure.synthetic.PosteriorSyntheticNetwork` (synthetic.py:964-1177) for the self-reporter mask, without an fp64 host
-    copy of rho and without dense (L,N,N,M) arrays.
+    `vimure.synthetic.PosteriorSyntheticNetwork` (synthetic.py:964-1177) under the ego, all-reporter or an explicit
+    reporter mask, without an fp64 host copy of rho and without dense (L,N,N) or (L,N,N,M) arrays.
 
     build_Y : Y_lij ~ Categorical(rho_f[l,i,j,:]) (one draw; `model.sample_inferred_model(N=1, seed=seed_Y)`: numpy's
-              stream like the reference for small problems, the device kernel for large ones).
+              stream like the reference for small problems, the device kernel for large ones -- as an edge list
+              evaluated on the device, so it works without the posterior slab at any N).
     build_X : theta ~ Gamma(gamma_shp_f, 1/gamma_rte_f), lambda ~ Gamma(phi_shp_f, 1/phi_rte_f), eta ~ Gamma(nu_shp_f,
               1/nu_rte_f) drawn with RandomState(seed_X) in the reference's order (synthetic.py:1040-1042); a tie of
               category k >= 1 gets lambda[l,k], every other tie lambda[0,0] (synthetic.py:1044-1048); the reports follow
-              `_build_X`'s law (synthetic.py:1063-1098), sampled by the device generator.  Also the union / intersection
-              baselines (synthetic.py:1139-1172)."""
+              `_build_X`'s law (synthetic.py:1063-1098) under the mask of `Rinput` / `flag_self_reporter`, sampled by the
+              device generator (`device_reports`).  Also the union / intersection baselines (synthetic.py:1139-1172)."""
 
     def __init__(self, model, seed_Y):
         self.model, self.seed_Y = model, seed_Y
@@ -303,17 +393,29 @@ class PosteriorSyntheticNetwork:
         self.M = self.theta_shp.shape[1]
 
     def build_Y(self, rng="auto"):
-        Y = np.asarray(self.model.sample_inferred_model(N=1, seed=self.seed_Y, rng=rng)[0])
-        Y = np.minimum(Y, self.K - 1)
-        subs = np.nonzero(Y)
-        self.Y_subs = np.stack(subs).astype(np.int64)
-        self.Y_vals = Y[subs].astype(np.int64)
+        from .model import AUTO_REFERENCE_INIT_LIMIT
+
+        device = rng == "device" or (rng == "auto" and float(self.L) * self.N * self.N * self.K > AUTO_REFERENCE_INIT_LIMIT)
+        if device:  # the device sampler's draws as an edge list: no (L, N, N) array
+            Ys = self.model.sample_inferred_model(N=1, seed=self.seed_Y, sparse=True)[0]
+            self.Y_subs = np.stack(Ys.subs).astype(np.int64)
+            self.Y_vals = np.minimum(Ys.vals, self.K - 1).astype(np.int64)
+        else:
+            Y = np.asarray(self.model.sample_inferred_model(N=1, seed=self.seed_Y, rng=rng)[0])
+            Y = np.minimum(Y, self.K - 1)
+            subs = np.nonzero(Y)
+            self.Y_subs = np.stack(subs).astype(np.int64)
+            self.Y_vals = Y[subs].astype(np.int64)
         self.Y = sptensor(tuple(self.Y_subs), self.Y_vals, shape=(self.L, self.N, self.N))
         return self
 
     def build_X(self, Rinput=None, flag_self_reporter=True, cutoff_X=False, Q=None, seed_X=None, device="cuda"):
-        if Rinput is not None or not flag_self_reporter:
-            raise NotImplementedError("vimure_b200.PosteriorSyntheticNetwork samples under the self-reporter mask only")
+        """Reports under `Rinput` (anything `masks.from_input` accepts) when given, else under the self-reporter mask
+        (`flag_self_reporter=True`) or the all-reporter mask (False).  Sets X, R (the EgoMask, AllMask or CooMask sampled,
+        so that `VimureModel().fit(X, R=R, ...)` takes them as they are), theta, lambda_k, mutuality and the baselines."""
+        import torch
+
+        R = _report_mask(Rinput, flag_self_reporter, self.L, self.N, self.M)
         for nm in ("theta_rte", "lambda_rte", "mutuality_rte"):
             if np.any(np.asarray(getattr(self, nm)) == 0):
                 raise ValueError(nm + " has some zero entries!")
@@ -328,20 +430,26 @@ class PosteriorSyntheticNetwork:
             raise ValueError("the drawn mutuality (%g) is outside [0, 1)" % mutuality)
         lam = np.array(lambda_k, dtype=np.float64)
         lam[:, 0] = lambda_k[0, 0]  # every tie without a positive category gets lambda_k[0, 0] (synthetic.py:1044)
-        subs, vals = device_reports(self.L, self.N, self.M, self.K, self.Y_subs, self.Y_vals, theta, mutuality, seed_X, lam=lam,
-                                    device=device)
-        subs, vals = subs.cpu().numpy().astype(np.int64), vals.cpu().numpy().astype(np.int64)
+        subs_d, vals_d = device_reports(self.L, self.N, self.M, self.K, self.Y_subs, self.Y_vals, theta, mutuality, seed_X,
+                                        lam=lam, device=device, mask=R)
+        # baselines (synthetic.py:1139-1172): ties reported by anybody / by exactly two reports, from int64 tie keys
+        s64 = subs_d[:3].long()
+        ties, cnt = torch.unique((s64[0] * self.N + s64[1]) * self.N + s64[2], return_counts=True)
+        inter = ties[cnt == 2]
+        del s64
+        subs, vals = subs_d.cpu().numpy().astype(np.int64), vals_d.cpu().numpy().astype(np.int64)
+        del subs_d, vals_d
         if cutoff_X:
             vals = np.minimum(vals, (self.K if Q is None else Q) - 1)
         self.X = sptensor(tuple(subs), vals, shape=(self.L, self.N, self.N, self.M))
-        self.R = EgoMask(self.L, self.N, self.M, diag=True)
+        self.R = R
         self.theta, self.lambda_k, self.mutuality = theta, lambda_k, mutuality
-        # baselines (synthetic.py:1139-1172): ties reported by anybody / by exactly two reports
-        ties, cnt = np.unique(subs[:3].T, axis=0, return_counts=True)
         shape3 = (self.L, self.N, self.N)
-        self.X_union = sptensor(tuple(ties.T), np.ones(len(ties), dtype=np.int8), shape=shape3)
-        inter = ties[cnt == 2]
-        self.X_intersection = sptensor(tuple(inter.T), np.ones(len(inter), dtype=np.int8), shape=shape3)
+        for name, k in (("X_union", ties), ("X_intersection", inter)):
+            k = k.cpu().numpy()
+            l, r = np.divmod(k, np.int64(self.N) * self.N)
+            i, j = np.divmod(r, np.int64(self.N))
+            setattr(self, name, sptensor((l, i, j), np.ones(len(k), dtype=np.int8), shape=shape3))
         return self
 
 
