@@ -253,3 +253,7 @@ def test_simple_special_tie_classification(mutuality):
     small = syn.StandardSBM(N=300, L=1, K=2, C=2, avg_degree=4, seed=1).build_X(mutuality=0.3, seed=2)
     Ps = _packing.pack(small.X.subs, small.X.vals, 1, 300, 300, 2, small.R, "cpu", mutuality=mutuality)
     assert not Ps.simple_ok and Ps.n_cx == Ps.U
+    # the packer itself records whether the E0 / E1 split holds (what the engine's fp32 paths require)
+    Pt = _packing.pack_torch(small.X.subs, small.X.vals, 1, 300, 300, 2, small.R, "cpu", mutuality=mutuality,
+                             split_e0=False)
+    assert Pt.split_e0 == (not mutuality)

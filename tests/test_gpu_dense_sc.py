@@ -1,9 +1,7 @@
 """The dense kernel that evaluates the shortcut ties itself (k_dense_sc) on row segments with many of them: a hub whose
 segments of one column tile carry more than 32 and more than 64 shortcut ties (the kernel's per-lane loop over a
-segment's ties), next to segments without special ties.  Against the CPU oracle and the fp64 path (VM_NO_SIMPLE=1);
+segment's ties), next to segments without special ties.  Against the CPU oracle and the fp64 path (simple=False);
 the slab must equal rho_u32 at every special tie."""
-import os
-
 import numpy as np
 import pytest
 
@@ -35,7 +33,7 @@ def _hub_network(N=1100, K=2):
     return net
 
 
-def test_crowded_row_segments_in_the_fused_dense_kernel(monkeypatch):
+def test_crowded_row_segments_in_the_fused_dense_kernel():
     torch = _cuda()
     N, K = 1100, 2
     net = _hub_network(N, K)
@@ -50,9 +48,7 @@ def test_crowded_row_segments_in_the_fused_dense_kernel(monkeypatch):
     assert per_seg[5 * 3 + 0] > 64 and 32 < per_seg[9 * 3 + 1] <= 64
     quiet = np.isin(row, [13, 17])
     assert (P.t["u_col"].cpu().numpy()[quiet] == row[quiet]).all()  # their only special tie is the diagonal
-    monkeypatch.setenv("VM_NO_SIMPLE", "1")
-    ref, _, _ = _engine_and_oracle(net, net.R, None, K, tile_h=32)
-    monkeypatch.delenv("VM_NO_SIMPLE")
+    ref, _, _ = _engine_and_oracle(net, net.R, None, K, tile_h=32, simple=False)
     assert not ref.simple_mode
 
     u_row, u_col = P.t["u_lrow"].long(), P.t["u_col"].long()

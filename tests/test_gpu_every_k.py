@@ -145,9 +145,9 @@ def _problem(K):
                 tile_h=tile_h)
 
 
-def _engines(subs, vals, L, N, M, K, mask, spec=None, mutuality=True, tile_h=64, slabs=(True,), seed=3):
-    """Engines over the same packed data and initial state (`slabs`: with or without a slab), the packed data, and the
-    fp64 oracle from that state if `spec` is given."""
+def _engines(subs, vals, L, N, M, K, mask, spec=None, mutuality=True, tile_h=64, slabs=(True,), seed=3, gamma_ts=True):
+    """Engines over the same packed data and initial state (`slabs`: with or without a slab; `gamma_ts` permits the
+    tie-sorted gamma pass), the packed data, and the fp64 oracle from that state if `spec` is given."""
     torch = _cuda()
     from oracle.cavi_numpy import OracleCAVI
     from vimure_b200 import _packing
@@ -165,7 +165,7 @@ def _engines(subs, vals, L, N, M, K, mask, spec=None, mutuality=True, tile_h=64,
     nu_rte = PRIORS["beta_eta"] + float(np.sum(vals)) if mutuality else 1.0
     engs = []
     for slab in slabs:
-        e = CaviEngine(P, PRIORS, mutuality=mutuality, eps=1e-12, slab=slab)
+        e = CaviEngine(P, PRIORS, mutuality=mutuality, eps=1e-12, slab=slab, gamma_ts=gamma_ts)
         e.set_state(st["gamma_shp"], st["gamma_rte"], st["phi_shp"], st["phi_rte"], st["nu_shp"] if mutuality else 1e-6,
                     nu_rte, pr_u, 1e-12)
         engs.append(e)
@@ -495,11 +495,11 @@ def test_general_mask_boundary_k(K):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("xmax", [2 ** 19 - 1, 2 ** 19])
-def test_gamma_ts_count_guard(xmax, monkeypatch):
+def test_gamma_ts_count_guard(xmax):
     """The tie-sorted gamma pass accumulates x * rho in fixed point (2^-30, three 20-bit limbs) and runs only while every
     count is below 2^19; at 2^19 the reporter-sorted pass takes over.  At such a count the fp64 oracle itself overflows
     (its exp of the tie's log-posterior is not shifted by the maximum), so the reference here is the same engine with the
-    tie-sorted pass switched off (VM_NO_GAMMA_TS=1).  Only at 2^19 - 1 does that compare two different kernels: there the
+    tie-sorted pass switched off (gamma_ts=False).  Only at 2^19 - 1 does that compare two different kernels: there the
     passes must agree at the part-2 tolerances over the cadence.  At 2^19 both engines run the reporter-sorted pass, so
     that case pins the guard itself (which pass runs) and that the fit stays finite.  The count is put on every entry of
     one reporter that has a reciprocal report, so that a warp's shared limbs sum many terms of ~2^19 (the 512-term
@@ -520,8 +520,7 @@ def test_gamma_ts_count_guard(xmax, monkeypatch):
     vals[recip] = xmax
     mask = vm.masks.AllMask(L, N, M)
     (eng,), P, _ = _engines(subs, vals, L, N, M, K, mask)
-    monkeypatch.setenv("VM_NO_GAMMA_TS", "1")
-    (ref,), _, _ = _engines(subs, vals, L, N, M, K, mask)
+    (ref,), _, _ = _engines(subs, vals, L, N, M, K, mask, gamma_ts=False)
     assert float(P.t["f_x"].max()) == xmax
     assert eng.gamma_ts == (xmax < 2 ** 19) and not ref.gamma_ts
     for step, (n, elbo) in enumerate(CADENCE):

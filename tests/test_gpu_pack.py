@@ -80,7 +80,7 @@ def test_vm_pack_matches_the_torch_packer(case):
     a = _packing.pack_device(subs, vals, L, N, M, K, mask, "cuda", row0=row0, nloc=nloc, tile_h=32, **kw)
     b = _packing.pack_torch(subs, vals, L, N, M, K, mask, "cuda", row0=row0, nloc=nloc, tile_h=32, **kw)
     for f in ("L", "N", "M", "K", "row0", "nloc", "tile_w", "tile_h", "nct", "nrt", "U", "I", "I1", "IT", "n_cx", "n_gchunk",
-              "n_ublk", "phi_chunk", "n_phichunk", "n_cxblk", "r_mode", "ego_diag", "simple_ok"):
+              "n_ublk", "phi_chunk", "n_phichunk", "n_cxblk", "r_mode", "ego_diag", "simple_ok", "split_e0"):
         assert getattr(a, f) == getattr(b, f), f
     assert a.b_all == b.b_all
     assert a.sumX_owned == (b.sumX_owned if b.sumX_owned is not None else b.sumX)

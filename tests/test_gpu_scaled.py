@@ -16,7 +16,7 @@ def _cuda():
     return torch
 
 
-def _engine_and_oracle(net, mask, spec, K, mutuality=True, seed=3, tile_h=64, row0=0, nloc=None):
+def _engine_and_oracle(net, mask, spec, K, mutuality=True, seed=3, tile_h=64, row0=0, nloc=None, simple=True, all32=True):
     _cuda()
     from oracle.cavi_numpy import OracleCAVI
     from vimure_b200 import _packing
@@ -25,8 +25,8 @@ def _engine_and_oracle(net, mask, spec, K, mutuality=True, seed=3, tile_h=64, ro
     L, N, M = net.X.shape[0], net.X.shape[1], net.X.shape[3]
     subs = np.stack(net.X.subs)
     P = _packing.pack(subs, net.X.vals, L, N, M, K, mask, "cuda", row0=row0, nloc=nloc, tile_h=tile_h,
-                      mutuality=mutuality)
-    eng = CaviEngine(P, PRIORS, mutuality=mutuality, eps=1e-12)
+                      mutuality=mutuality, simple=simple)
+    eng = CaviEngine(P, PRIORS, mutuality=mutuality, eps=1e-12, all32=all32)
     prng = np.random.RandomState(seed)
     rs = prng.random_sample
     st = dict(gamma_shp=0.1 * rs((L, M)) + 0.1, phi_shp=10.0 * rs((L, K)) + 10.0, gamma_rte=0.1 * rs((L, M)) + 0.1,
@@ -93,10 +93,10 @@ def test_config4_scaled_dense_reporting():
 
 
 @pytest.mark.parametrize("case", ["k2_m16", "k3_m40_nomut_layer"])
-def test_all_reporter_mask_fp32_special_ties(case, monkeypatch):
+def test_all_reporter_mask_fp32_special_ties(case):
     """All-reporter mask: on iterations without ELBO every special tie is evaluated in fp32, entry-parallel (k_all32,
     include/vimure_b200.h: vm_ctx.all32_mode).  Against the oracle (usual tolerances, after runs of such iterations, slab
-    included) and against the same engine on the fp64 special-tie kernel (VM_NO_ALL32=1)."""
+    included) and against the same engine on the fp64 special-tie kernel (all32=False)."""
     torch = _cuda()
     import vimure_b200 as vm
     import vimure_b200.synthetic as syn
@@ -116,8 +116,7 @@ def test_all_reporter_mask_fp32_special_ties(case, monkeypatch):
     mask = vm.masks.AllMask(L, N, M)
     eng, o, P = _engine_and_oracle(net, mask, {"kind": "all", "dense_input": True}, K)
     assert eng.all32_mode
-    monkeypatch.setenv("VM_NO_ALL32", "1")
-    ref, _, _ = _engine_and_oracle(net, mask, None, K)
+    ref, _, _ = _engine_and_oracle(net, mask, None, K, all32=False)
     assert not ref.all32_mode
 
     def check(tag):
@@ -210,7 +209,7 @@ def test_full_size_properties_config3():
 
 
 @pytest.mark.parametrize("case", ["sbm_k2", "gm_l2_k3", "nomut_k2", "subset_k4"])
-def test_simple_special_ties_in_the_dense_kernel(case, monkeypatch):
+def test_simple_special_ties_in_the_dense_kernel(case):
     """On iterations without ELBO the shortcut kernel (k_shortcut) evaluates the special ties that have no reciprocal report
     (fp32, include/vimure_b200.h: vm_ctx.simple_mode) and the special-tie kernel only walks the others.  Against the
     oracle (the usual tolerances, after runs of such iterations) and against the same engine with the shortcut off."""
@@ -244,8 +243,7 @@ def test_simple_special_ties_in_the_dense_kernel(case, monkeypatch):
     eng, o, P = _engine_and_oracle(net, mask, spec, K, mutuality=mutuality, tile_h=32)
     assert eng.simple_mode and int(P.t["u_simple"].sum()) > 0 and P.n_cx < P.U
     assert bool(P.t["u_single"].any()) == mutuality
-    monkeypatch.setenv("VM_NO_SIMPLE", "1")
-    ref, _, P2 = _engine_and_oracle(net, mask, None, K, mutuality=mutuality, tile_h=32)
+    ref, _, P2 = _engine_and_oracle(net, mask, None, K, mutuality=mutuality, tile_h=32, simple=False)
     assert not ref.simple_mode and P2.n_cx == P2.U
 
     def check(tag, slab):
@@ -285,23 +283,16 @@ def test_simple_special_ties_in_the_dense_kernel(case, monkeypatch):
 
 def test_shortcut_ties_vs_fp64_path_at_config3_size():
     """N = 20 000 (config 3): 10 iterations in which the shortcut kernel evaluates the SIMPLE and SINGLE special ties in
-    fp32 against the same 10 iterations with every special tie in fp64 (VM_NO_SIMPLE=1).  The fp32 table rounding is common
+    fp32 against the same 10 iterations with every special tie in fp64 (simple=False).  The fp32 table rounding is common
     to all ties of a node, so its effect does not average down with N: this is the size at which it has to be checked."""
     torch = _cuda()
-    import os
-
     import vimure_b200.synthetic as syn
 
     N, K = 20000, 2
     net = syn.StandardSBM(N=N, L=1, K=K, C=2, avg_degree=10, seed=10).build_X(mutuality=0.5, seed=20)
     res = {}
     for mode in ("shortcut", "fp64"):
-        if mode == "fp64":
-            os.environ["VM_NO_SIMPLE"] = "1"
-        try:
-            eng, _, P = _engine_and_oracle(net, net.R, None, K, tile_h=128)
-        finally:
-            os.environ.pop("VM_NO_SIMPLE", None)
+        eng, _, P = _engine_and_oracle(net, net.R, None, K, tile_h=128, simple=(mode == "shortcut"))
         assert eng.simple_mode == (mode == "shortcut")
         if mode == "shortcut":
             frac = 1.0 - P.n_cx / P.U

@@ -15,6 +15,7 @@ import numpy as np
 import torch
 
 from . import _capi
+from ._pack_native import dense_fast_eligible
 
 
 def _packing_const():
@@ -32,7 +33,11 @@ IMPLICIT_STATE = ("tab_p", "tab_q", "layer_consts", "rho_u32")
 
 
 class CaviEngine:
-    def __init__(self, packed, priors, mutuality=True, eps=1e-12, group=None, may_dead=False, slab=True):
+    def __init__(self, packed, priors, mutuality=True, eps=1e-12, group=None, may_dead=False, slab=True, all32=True,
+                 gamma_ts=True):
+        """`all32` and `gamma_ts` permit the fp32 special-tie kernel and the tie-sorted gamma pass of an all-reporter
+        mask where the problem allows them; `False` keeps the fp64 special-tie kernel / the reporter-sorted gamma pass,
+        the references the tests compare them against."""
         P = self.P = packed
         if not torch.cuda.is_available():
             raise RuntimeError("vimure_b200 needs a CUDA device: the CAVI kernels have no CPU fallback")
@@ -50,7 +55,7 @@ class CaviEngine:
         if not self.slab and P.r_mode == 2:
             raise ValueError("a fit without the dense slab needs an ego or all-reporter mask (the general mask's "
                              "statistics gather the slab)")
-        if self.mutuality and not getattr(P, "mutuality", True):
+        if self.mutuality and not P.mutuality:
             raise ValueError("the data were packed for mutuality=False (no entry visits the gamma/phi passes)")
         f64 = dict(dtype=torch.float64, device=dev)
         f32 = dict(dtype=torch.float32, device=dev)
@@ -92,27 +97,24 @@ class CaviEngine:
         self.fixG = torch.zeros(L * M, dtype=torch.int64, device=dev)
         self.phi0 = z(L * K)
         # simple special ties (see include/vimure_b200.h): patch source of the fast dense kernel, their phi0 part
-        self.simple_mode = bool(getattr(P, "simple_ok", False))
+        self.simple_mode = bool(P.simple_ok)
         self.u_rec = torch.zeros(max(U, 1) if self.simple_mode else 1, 4 if K == 2 else 8, **f32)
         stride = 4 if K == 2 else (8 if K <= 6 else K + 2)
         self.nodetab = torch.zeros(L * N * stride if self.simple_mode else 4, **f32)
         self.fixP = torch.zeros(L * K, dtype=torch.int64, device=dev)
         self.simple_consts = z(3 + K)
         # all-reporter mask: every special tie in fp32 on iterations without ELBO (k_all32, see the header)
-        import os
-
-        self.all32_mode = bool(P.r_mode == 1 and K <= 4 and M <= 4096 and U > 0 and getattr(P, "split_e0", False)
-                               and os.environ.get("VM_NO_ALL32") != "1")
+        self.all32_mode = bool(all32 and P.r_mode == 1 and K <= 4 and M <= 4096 and U > 0 and P.split_e0)
         self.u_lo = torch.zeros(max(U, 1) * K if self.all32_mode else 1, **f32)
         self.gfpart = z(L * ((M + 255) // 256) * (K + 4))
         # fork/join events of the aux stream, created once (vm_ctx.ev_fork / ev_join)
         self._ev_fork, self._ev_join = torch.cuda.Event(), torch.cuda.Event()
         self._ev_fork.record()
         self._ev_join.record()
-        self.cx_logpr = z(max(int(getattr(P, "n_cx", 0)), 1) if self.simple_mode else 1, K)
+        self.cx_logpr = z(max(P.n_cx, 1) if self.simple_mode else 1, K)
         assert _packing_const() == self.C["VM_SPECIAL_TIES_PER_BLOCK"]
         # tie-sorted gamma pass (vm_ctx.gamma_ts): few reporters, counts small enough for its 2^-30 fixed point
-        self.gamma_ts = bool(P.r_mode == 1 and K <= 8 and M <= 256 and P.I1 > 0 and os.environ.get("VM_NO_GAMMA_TS") != "1"
+        self.gamma_ts = bool(gamma_ts and P.r_mode == 1 and K <= 8 and M <= 256 and P.I1 > 0
                              and float(P.t["f_x"].max()) < 2.0 ** 19)
         n_blk = max(P.n_gchunk, L * P.n_phichunk * K, (L * P.n_phichunk * M) if self.gamma_ts else 0,
                     L * P.n_ublk * 8 * (3 + 2 * K) + P.nct * L * P.nrt + 128 + 2 * 64 + L * 64 * (3 + K)) + 64
@@ -125,7 +127,7 @@ class CaviEngine:
         Ctx = _capi.ctx_class()
         c = self.ctx = Ctx()
         for name in ("L", "N", "M", "K", "row0", "nloc", "U", "I", "I1", "IT", "tile_w", "tile_h", "nct", "nrt", "n_gchunk",
-                     "phi_chunk", "n_phichunk", "n_ublk", "r_mode", "ego_diag"):
+                     "phi_chunk", "n_phichunk", "n_ublk", "n_cx", "n_cxblk", "r_mode", "ego_diag"):
             setattr(c, name, int(getattr(P, name)))
         c.mutuality = int(self.mutuality)
         c.may_dead = int(bool(may_dead))
@@ -135,8 +137,6 @@ class CaviEngine:
         c.simple_mode = int(self.simple_mode)
         c.all32_mode = int(self.all32_mode)
         c.gamma_ts = int(self.gamma_ts)
-        c.n_cx = int(getattr(P, "n_cx", U))
-        c.n_cxblk = int(getattr(P, "n_cxblk", P.n_ublk))
         # the aux stream carries the general dense kernel (partial column tiles) under the fast one (see launch_dense)
         self.aux_stream = torch.cuda.Stream(device=dev)
         c.aux_stream = self.aux_stream.cuda_stream
@@ -179,7 +179,7 @@ class CaviEngine:
         [dense_fast], dense, [col_reduce], stats, [elbo_b], sums_reduce | finish: [elbo_partial], finish."""
         P = self.P
         csr, ego = P.r_mode == 2, P.r_mode == 0
-        fast = P.K <= 4 and not csr and (P.N * P.K) % 4 == 0 and P.N >= P.tile_w and P.tile_h <= 128
+        fast = dense_fast_eligible(P.K, P.r_mode, P.N, P.tile_w, P.tile_h)
         n = 2 + 3 + 1 + (0 if csr else 1) + 1 + (1 if fast else 0) + 1 + (1 if ego else 0) + 1 + 2 + 1
         if elbo:
             n += 1 + (1 if self.mutuality else 0)
@@ -290,13 +290,11 @@ class CaviEngine:
     def enable_graphs(self):
         """Replay one captured CUDA graph per iteration instead of ~17 launches.  On a sharded fit the graph holds the
         whole iteration INCLUDING the three NCCL all-reduces (every rank captures the same sequence), so that nothing
-        waits for the host between the phases; VM_DIST_GRAPHS=0 keeps the sharded path on eager launches."""
-        import os
-
-        if self.group is not None:
-            # only NCCL collectives are stream operations that a graph can hold (gloo reduces on the host)
-            if os.environ.get("VM_DIST_GRAPHS", "1") == "0" or torch.distributed.get_backend() != "nccl":
-                return False
+        waits for the host between the phases.  Returns False, and leaves the engine on eager launches, for a sharded fit
+        whose backend is not NCCL.  An engine on which this is never called runs eagerly (`fit(graphs=False)`)."""
+        # only NCCL collectives are stream operations that a graph can hold (gloo reduces on the host)
+        if self.group is not None and torch.distributed.get_backend() != "nccl":
+            return False
         if self._graphs is None:
             self._graphs = {}
         return self._graphs is not None

@@ -22,6 +22,21 @@ PHI_CHUNK = 4096
 SPECIAL_TIES_PER_BLOCK = 1024  # == VM_SPECIAL_TIES_PER_BLOCK of include/vimure_b200.h
 
 
+def dense_fast_eligible(K, r_mode, N, tile_w, tile_h):
+    """Does a rho update run the fast (TMA) dense kernel?  A copy of `dense_fast_eligible` in csrc/vm_kernels.cu, which
+    decides it: an ego or all-reporter mask (not the general COO mask, r_mode 2), K <= 4, N*K % 4 == 0, at least one
+    full column tile, and row tiles of at most 128 = VM_FAST_MAX_TILE_H rows."""
+    return K <= 4 and r_mode != 2 and (N * K) % 4 == 0 and N >= tile_w and tile_h <= 128
+
+
+def shortcut_ties_eligible(K, r_mode, N, tile_w, tile_h, split_e0, U):
+    """Can the fast dense kernel evaluate special ties itself (shortcut ties, include/vimure_b200.h: vm_ctx.simple_mode)?
+    An ego mask (r_mode 0) on the fast dense kernel, the E0 / E1 split of the packed layout (`Packed.split_e0`), some
+    special ties, and column ids exact in fp32 (N < 2^24: the per-tie record stores them as floats)."""
+    return (r_mode == 0 and dense_fast_eligible(K, r_mode, N, tile_w, tile_h) and split_e0 and U > 0
+            and N < (1 << 24))
+
+
 def _i32(t):
     return t.to(torch.int32).contiguous()
 
@@ -65,19 +80,15 @@ class Packed:
 
 
 def pack_device(X_subs, X_vals, L, N, M, K, mask, device, row0=0, nloc=None, tile_h=64, mutuality=True, split_e0=True,
-                simple=None, single=None):
-    """The packed layout through `vm_pack` (include/vimure_b200.h): one call, one host synchronisation (to read the
-    counts).  Same contract as `pack_torch`; within a tie the entries are ordered by reporter (the sort key is
-    (l,i,j,m)) instead of by their position in the caller's list."""
+                simple=True, single=True):
+    """The packed layout through `vm_pack` (include/vimure_b200.h) for an ego or all-reporter mask on a CUDA device: one
+    call, one host synchronisation (to read the counts).  Same contract as `pack_torch`, `simple` and `single` included;
+    within a tie the entries are ordered by reporter (the sort key is (l,i,j,m)) instead of by their position in the
+    caller's list."""
     import ctypes
-    import os
 
     from . import _capi
 
-    if simple is None:
-        simple = os.environ.get("VM_NO_SIMPLE") != "1"
-    if single is None:
-        single = os.environ.get("VM_NO_SINGLE") != "1"
     dev = torch.device(device)
     nloc = N - row0 if nloc is None else int(nloc)
     _mark = _Trace(dev)
@@ -90,6 +101,8 @@ def pack_device(X_subs, X_vals, L, N, M, K, mask, device, row0=0, nloc=None, til
     P.nrt = (nloc + P.tile_h - 1) // P.tile_h
     P.mask = mask
     P.mutuality = bool(mutuality)
+    # (the fp32 paths need the E0 / E1 split's precondition: no prior so small that exp(E[log theta/lambda]) can be 0)
+    P.split_e0 = bool(split_e0 or not mutuality)
 
     def up32(a):
         if torch.is_tensor(a):
@@ -141,13 +154,15 @@ def pack_device(X_subs, X_vals, L, N, M, K, mask, device, row0=0, nloc=None, til
     counts = torch.zeros(16, **i64)
     rep = torch.as_tensor(mask.rep, device=dev).to(torch.uint8).flatten().contiguous() if ego else None
 
-    simple_ok = bool(simple and ego and K <= 4 and (N * K) % 4 == 0 and N >= TILE_W and P.tile_h <= 128
-                     and (split_e0 or not mutuality) and N < (1 << 24))
+    # vm_pack classifies the shortcut ties, so the rule is decided before U is known: only an ego mask can have them,
+    # and it makes every owned diagonal tie special, so there U > 0 exactly when L * nloc > 0
+    P.r_mode = 0 if ego else 1
+    P.simple_ok = bool(simple) and shortcut_ties_eligible(P.K, P.r_mode, P.N, TILE_W, P.tile_h, P.split_e0, L * nloc)
     A = _capi.pack_class()()
     A.L, A.N, A.M, A.K, A.row0, A.nloc, A.tile_h = P.L, P.N, P.M, P.K, P.row0, nloc, P.tile_h
-    A.r_mode, A.ego_diag = (0 if ego else 1), int(getattr(mask, "diag", False))
+    A.r_mode, A.ego_diag = P.r_mode, int(getattr(mask, "diag", False))
     A.mutuality, A.split_e0 = int(bool(mutuality)), int(bool(split_e0))
-    A.simple, A.single = int(simple_ok), int(bool(single))
+    A.simple, A.single = int(P.simple_ok), int(bool(single))
     A.n_in = n_in
     A.x_l, A.x_i, A.x_j, A.x_m = (t.data_ptr() for t in xs)
     A.x_v = xv.data_ptr()
@@ -181,7 +196,6 @@ def pack_device(X_subs, X_vals, L, N, M, K, mask, device, row0=0, nloc=None, til
     P.sumX_owned = float(cn[11])
     P.sumX = float(cn[11])
     P.b_all = float(cn[12])
-    P.simple_ok = simple_ok and U > 0
     size = dict(e_u=I, e_m=I, e_src=I, e_x=I, e_xT=I, e_flags=I, f_u=I1, f_m=I1, f_x=I1, f_xT=I1, g_u=I1, g_x=I1, g_xT=I1,
                 t_u=IT, t_lrow=IT, t_col=IT, t_x=IT, u_lrow=U, u_col=U, u_cnt=U, u_m0=U, u_x0=U, u_xT0=U, u_x0sum=U, u_px=U,
                 u_pxt=U, u_ptr=U + 1, u_gflat=U, u_has_x=U, u_reported=U, cx_idx=n_cx, cx_lrow=n_cx, cx_col=n_cx, cx_cnt=n_cx,
@@ -193,7 +207,6 @@ def pack_device(X_subs, X_vals, L, N, M, K, mask, device, row0=0, nloc=None, til
     P.t["u_single"] = P.t["u_pxt"] != 0
     P.t["u_simple"] = (P.t["u_px"] > 0) & ~P.t["u_single"]
     P.entry_src = P.t["e_src"].to(torch.int64)
-    P.r_mode = 0 if ego else 1
     P.ego_diag = int(getattr(mask, "diag", False))
     if ego:
         P.t["rep"] = rep

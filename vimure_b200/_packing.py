@@ -16,47 +16,33 @@ import torch
 
 
 from ._pack_native import (GAMMA_CHUNK, PHI_CHUNK, SPECIAL_TIES_PER_BLOCK, Packed, _Trace, _i32,  # noqa: F401
-                           dense_tile_w, pack_device)
+                           dense_tile_w, pack_device, shortcut_ties_eligible)
 
 
 def pack(X_subs, X_vals, L, N, M, K, mask, device, row0=0, nloc=None, tile_h=64, mutuality=True, split_e0=True,
-         simple=None, single=None):
-    """Build the packed layout: on a CUDA device and for a structured mask through the library's own packer (`vm_pack`
-    behind the C ABI, csrc/vm_pack.cu); otherwise (CPU tests, general COO masks, VM_PY_PACKER=1) with the torch index
-    ops of `pack_torch`, which doubles as the executable specification of the layout."""
-    import os
-
-    dev = torch.device(device)
-    if dev.type == "cuda" and mask.kind in ("ego", "all") and os.environ.get("VM_PY_PACKER") != "1":
-        P = pack_device(X_subs, X_vals, L, N, M, K, mask, dev, row0=row0, nloc=nloc, tile_h=tile_h, mutuality=mutuality,
-                        split_e0=split_e0, simple=simple, single=single)
-    else:
-        P = pack_torch(X_subs, X_vals, L, N, M, K, mask, device, row0=row0, nloc=nloc, tile_h=tile_h, mutuality=mutuality,
-                       split_e0=split_e0, simple=simple, single=single)
-    # (the fp32 paths need the E0 / E1 split's precondition: no prior so small that exp(E[log theta/lambda]) can be 0)
-    P.split_e0 = bool(split_e0 or not mutuality)
-    return P
+         simple=True, single=True):
+    """Build the packed layout: on a CUDA device and for an ego or all-reporter mask through the library's own packer
+    (`pack_device`: `vm_pack` behind the C ABI, csrc/vm_pack.cu); otherwise (CPU, general COO masks) with the torch index
+    ops of `pack_torch`, which doubles as the executable specification of the layout (call it directly to run it on a
+    CUDA device).  The arguments are those of `pack_torch`."""
+    packer = pack_device if torch.device(device).type == "cuda" and mask.kind in ("ego", "all") else pack_torch
+    return packer(X_subs, X_vals, L, N, M, K, mask, device, row0=row0, nloc=nloc, tile_h=tile_h, mutuality=mutuality,
+                  split_e0=split_e0, simple=simple, single=single)
 
 
 def pack_torch(X_subs, X_vals, L, N, M, K, mask, device, row0=0, nloc=None, tile_h=64, mutuality=True, split_e0=True,
-               simple=None, single=None):
+               simple=True, single=True):
     """Build the packed layout with torch index ops (any device).
 
     X_subs : (4, I) integer array-like (l, i, j, m);  X_vals : (I,) counts;  mask : masks.ReporterMask.
     mutuality / split_e0 : the gamma and phi passes only visit the entries with a reciprocal report (x^T > 0); for the
         others dz1_k = x, a constant (reference model.py:679-681, 693 with z2 = 0).  `split_e0=False` makes every entry
         visited (needed when a prior is so small that exp(E[log theta]) can underflow to 0, where model.py:692 gives 0).
-    simple : classify the special ties whose posterior the fast dense kernel can evaluate itself (default: yes, unless the
-        environment says VM_NO_SIMPLE=1 -- the A/B switch of the tests and tools).
-    single : ... including the ties with exactly one report that has a reciprocal report (default: yes, unless
-        VM_NO_SINGLE=1).
+    simple : classify the special ties whose posterior the fast dense kernel can evaluate itself, where
+        `shortcut_ties_eligible` allows it.  `False` leaves every special tie to the fp64 special-tie kernel: the
+        reference the tests compare the shortcut against.
+    single : ... including the ties with exactly one report that has a reciprocal report.
     """
-    import os
-
-    if simple is None:
-        simple = os.environ.get("VM_NO_SIMPLE") != "1"
-    if single is None:
-        single = os.environ.get("VM_NO_SINGLE") != "1"
     dev = torch.device(device)
     nloc = N - row0 if nloc is None else int(nloc)
     _mark = _Trace(dev)
@@ -67,7 +53,10 @@ def pack_torch(X_subs, X_vals, L, N, M, K, mask, device, row0=0, nloc=None, tile
     P.nct = (N + TILE_W - 1) // TILE_W
     P.nrt = (nloc + P.tile_h - 1) // P.tile_h
     P.mask = mask
+    P.r_mode = {"ego": 0, "all": 1, "coo": 2}[mask.kind]
     P.mutuality = bool(mutuality)
+    # (the fp32 paths need the E0 / E1 split's precondition: no prior so small that exp(E[log theta/lambda]) can be 0)
+    P.split_e0 = bool(split_e0 or not mutuality)
 
     def _up(a, small):
         """host array -> device int64/float64 tensor, moving as few bytes as possible over PCIe"""
@@ -230,8 +219,7 @@ def pack_torch(X_subs, X_vals, L, N, M, K, mask, device, row0=0, nloc=None, tile
     # SIMPLE (no entry with a reciprocal report) or SINGLE (exactly one entry, with a reciprocal report, reported by the row
     # or the column node).  On iterations without ELBO the dense kernel (k_dense_sc) evaluates them and the special-tie kernel walks
     # `cx_idx`, the others, through compacted copies of their per-tie arrays.
-    P.simple_ok = bool(simple and mask.kind == "ego" and K <= 4 and (N * K) % 4 == 0 and N >= TILE_W and P.tile_h <= 128
-                       and (split_e0 or not mutuality) and U > 0 and N < (1 << 24))
+    P.simple_ok = bool(simple) and shortcut_ties_eligible(P.K, P.r_mode, P.N, TILE_W, P.tile_h, P.split_e0, U)
     u_simple = torch.zeros(U, dtype=torch.bool, device=dev)
     u_single = torch.zeros(U, dtype=torch.bool, device=dev)
     if P.simple_ok:
@@ -307,7 +295,6 @@ def pack_torch(X_subs, X_vals, L, N, M, K, mask, device, row0=0, nloc=None, tile
 
     _mark("transposed list")
     # ---- reporter mask
-    P.r_mode = {"ego": 0, "all": 1, "coo": 2}[mask.kind]
     P.ego_diag = int(getattr(mask, "diag", False))
     if mask.kind == "ego":
         P.t["rep"] = torch.as_tensor(mask.rep, device=dev).to(torch.uint8).flatten().contiguous()
