@@ -102,7 +102,8 @@ def test_ego_detection_rejects_duplicates_and_near_misses():
     assert not vm.masks._ego_entries_distinct(*dup, L=L, N=10**6, M=M)
 
 
-@pytest.mark.parametrize("name,world", [("f1_over", 1), ("karnataka_vil1", 1), ("gm_l2_k3", 3), ("custom_mask", 2), ("nomut", 2)])
+@pytest.mark.parametrize("name,world", [("f1_over", 1), ("karnataka_vil1", 1), ("gm_l2_k3", 3), ("custom_mask", 2), ("nomut", 2),
+                                        ("dense_reporting", 3), ("f1_over", 8)])
 def test_packing_invariants(name, world):
     import vimure_b200 as vm
     from vimure_b200 import _packing

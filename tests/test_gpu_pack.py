@@ -27,7 +27,8 @@ def _sorted_coo(X):
     return s[:, o], np.asarray(X.vals)[o]
 
 
-CASES = ["ego_k2", "ego_l2_k3_shard", "ego_nomut", "ego_subset_nodiag", "all_mask", "ego_no_shortcut"]
+CASES = ["ego_k2", "ego_l2_k3_shard", "ego_nomut", "ego_subset_nodiag", "all_mask", "ego_no_shortcut", "all_mask_shard",
+         "ego_subset_nodiag_k4_shard", "ego_empty_shard"]
 
 
 @pytest.mark.parametrize("case", CASES)
@@ -54,13 +55,24 @@ def test_vm_pack_matches_the_torch_packer(case):
         net = syn.StandardSBM(N=N, L=L, K=K, C=2, avg_degree=6, seed=5).build_X(mutuality=0.3, seed=6)
         mask, M = net.R, N
         kw = dict(mutuality=False, split_e0=True)
-    elif case == "ego_subset_nodiag":
+    elif case in ("ego_subset_nodiag", "ego_subset_nodiag_k4_shard"):
         L, N, K, M = 2, 520, 4, 60
         net = syn.StandardSBM(N=N, M=M, L=L, K=K, C=2, avg_degree=6, seed=7).build_X(mutuality=0.4, seed=8)
         rep = np.zeros((L, M), dtype=np.uint8)
         rep[:, ::2] = 1
         mask = vm.masks.EgoMask(L, N, M, rep=rep, diag=False)  # X keeps entries of inactive reporters: outside R
-    elif case == "all_mask":
+        if case == "ego_subset_nodiag_k4_shard":  # rows >= M: no row node of the shard reports
+            row0, nloc = shard_rows(N, 3, 2)
+    elif case == "ego_empty_shard":  # every report that touches the shard's rows dropped: only its diagonal ties remain
+        L, N, K = 1, 1100, 2
+        net = syn.StandardSBM(N=N, L=L, K=K, C=2, avg_degree=10, seed=10).build_X(mutuality=0.5, seed=20)
+        mask, M = net.R, N
+        row0, nloc = shard_rows(N, 3, 1)
+        s = np.stack(net.X.subs)
+        inside = lambda a: (a >= row0) & (a < row0 + nloc)  # noqa: E731
+        keep = ~(inside(s[1]) | inside(s[2]))
+        net.X = vm.sptensor.sptensor(tuple(s[:, keep]), np.asarray(net.X.vals)[keep], shape=net.X.shape)
+    elif case in ("all_mask", "all_mask_shard"):
         L, N, K, M = 2, 300, 2, 16
         y = syn.StandardSBM(N=N, M=M, L=L, K=K, C=2, avg_degree=8, seed=5)
         X, _ = syn.dense_reporting_X(y, M=M, mutuality=0.4, seed=6)
@@ -71,6 +83,8 @@ def test_vm_pack_matches_the_torch_packer(case):
         net = Net()
         net.X = X
         mask = vm.masks.AllMask(L, N, M)
+        if case == "all_mask_shard":
+            row0, nloc = shard_rows(N, 3, 1)
     else:  # no fast dense kernel (N below a column tile): no shortcut ties; every entry visited (split_e0 off)
         L, N, K = 1, 300, 2
         net = syn.StandardSBM(N=N, L=L, K=K, C=2, avg_degree=4, seed=1).build_X(mutuality=0.3, seed=2)
@@ -91,7 +105,77 @@ def test_vm_pack_matches_the_torch_packer(case):
         assert x.shape == y.shape, (name, x.shape, y.shape)
         assert np.array_equal(x, y), name
     assert np.array_equal(a.entry_src.cpu().numpy(), b.entry_src.cpu().numpy())
-    assert int(a.t["u_single"].sum()) > 0 or case in ("ego_nomut", "all_mask", "ego_no_shortcut")
+    assert int(a.t["u_single"].sum()) > 0 or case in ("ego_nomut", "all_mask", "ego_no_shortcut", "all_mask_shard",
+                                                      "ego_empty_shard")
+    if case == "ego_empty_shard":
+        assert a.I == 0 and a.U == nloc and a.n_cx == a.U
+    if case == "ego_subset_nodiag_k4_shard":
+        assert a.row0 >= M and a.I > 0
+
+
+def _assert_same_packing(a, b, src_a, src_b, tag):
+    """Two packings of one shard from different inputs: every array equal; the packed entries come from the same entries
+    of the whole list (`src_*` maps a position in each input to the whole list)."""
+    for f in ("U", "I", "I1", "IT", "n_cx", "n_gchunk", "n_ublk", "n_phichunk", "n_cxblk", "simple_ok"):
+        assert getattr(a, f) == getattr(b, f), (f, tag)
+    assert a.b_all == b.b_all and a.sumX_owned == b.sumX_owned, tag
+    assert set(a.t) == set(b.t), tag
+    for name in sorted(set(a.t) - {"e_src"}):
+        x, y = a.t[name].cpu().numpy(), b.t[name].cpu().numpy()
+        assert x.shape == y.shape and np.array_equal(x, y), (name, tag)
+    assert np.array_equal(src_a[a.entry_src.cpu().numpy()], src_b[b.entry_src.cpu().numpy()]), tag
+
+
+@pytest.mark.parametrize("kind", ["ego", "all"])
+def test_vm_pack_of_a_shard_from_its_own_rows_and_reciprocals(kind):
+    """A shard packed from the entries of its own rows plus the reciprocal entries of other rows (in the order
+    `_exchange_reciprocals` delivers them: own entries, then the received ones by sending rank; and as
+    `device_reports(..., emit_transposed=True)` generates them) is the shard packed from the whole list."""
+    torch = _cuda()
+    import vimure_b200 as vm
+    import vimure_b200.synthetic as syn
+    from vimure_b200._pack_native import pack_device
+    from vimure_b200.model import shard_rows
+
+    W, r = 3, 1
+    if kind == "ego":
+        L, N, M, K = 2, 1100, 1100, 3
+        net = syn.Multitensor(N=N, L=L, K=K, C=2, avg_degree=8, eta=0.5, seed=3).build_X(mutuality=0.5, seed=4)
+        mask = net.R
+    else:
+        L, N, M, K = 2, 600, 16, 2
+        net = syn.StandardSBM(N=N, M=M, L=L, K=K, C=2, avg_degree=8, seed=5)
+        net.X, _ = syn.dense_reporting_X(net, M=M, mutuality=0.4, seed=6)
+        mask = vm.masks.AllMask(L, N, M)
+    row0, nloc = shard_rows(N, W, r)
+    kw = dict(row0=row0, nloc=nloc, tile_h=128)
+    # 1. a host list: the whole of it, and the shard's own entries followed by the reciprocals it receives
+    s, v = np.stack(net.X.subs).astype(np.int64), np.asarray(net.X.vals).astype(np.int64)
+    owner = np.searchsorted(np.array([shard_rows(N, W, q)[0] for q in range(1, W)]), s[1], side="right")
+    col_owner = np.searchsorted(np.array([shard_rows(N, W, q)[0] for q in range(1, W)]), s[2], side="right")
+    own = np.nonzero(owner == r)[0]
+    recv = np.nonzero((col_owner == r) & (owner != r))[0]
+    recv = recv[np.argsort(owner[recv], kind="stable")]
+    sel = np.concatenate([own, recv])
+    assert len(recv) and len(own)
+    a = pack_device(s, v, L, N, M, K, mask, "cuda", **kw)
+    b = pack_device(s[:, sel], v[sel], L, N, M, K, mask, "cuda", **kw)
+    _assert_same_packing(a, b, np.arange(len(v)), sel, f"{kind}: own rows + received reciprocals")
+    # 2. the device generator: the shard's rows with their transposed entries, against the whole generated list
+    theta = np.random.RandomState(7).gamma(2.0, 0.5, size=(L, M))
+    gen = dict(mask=mask) if kind == "all" else {}
+    fs, fv = syn.device_reports(L, N, M, K, net.Y_subs, net.Y_vals, theta, 0.4, 17, **gen)
+    ps, pv = syn.device_reports(L, N, M, K, net.Y_subs, net.Y_vals, theta, 0.4, 17, row0=row0, nloc=nloc,
+                                emit_transposed=True, **gen)
+    fk = (((fs[0].long() * N + fs[1]) * N + fs[2]) * M + fs[3]).cpu().numpy()
+    pk = (((ps[0].long() * N + ps[1]) * N + ps[2]) * M + ps[3]).cpu().numpy()
+    o = np.argsort(fk)
+    pos = o[np.searchsorted(fk[o], pk)]
+    assert np.array_equal(fk[pos], pk) and np.array_equal(fv.cpu().numpy()[pos], pv.cpu().numpy())
+    a = pack_device(fs, fv, L, N, M, K, mask, "cuda", **kw)
+    b = pack_device(ps, pv, L, N, M, K, mask, "cuda", **kw)
+    _assert_same_packing(a, b, np.arange(fk.size), pos, f"{kind}: device_reports(emit_transposed=True)")
+    torch.cuda.synchronize()
 
 
 def test_vm_pack_reports_bad_input():
